@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- GausPcgc encode+decode throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--points P] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--points P] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one scene: device-resident voxel anchors -> pyramid ->
@@ -26,6 +26,11 @@ roofline = the dominant kernel family of the step (the sparse conv of the big de
 --impl reference: the reference algorithm on the host cores (CPU oracle port; the reference's own
            dependencies torchsparse/torchac are not installable offline) on the SAME workload when the
            run fits the time budget, else on the largest sample that does (config.sample_points says which).
+--dump-outputs DIR: after the timed steps, what the last of them computed, as DIR/<name>.npy (float32, or float64 where
+           float32 cannot hold an integer exactly): base_xyz, base_occ, occupancy (every coded level, coarse -> fine),
+           cdf_bounds_stage<i> (c_low, c_high of the range coder's interval per row of stage i, coarse -> fine) and points
+           (the decoded cloud).  The scene and weights are seeded, so two builds run with the same arguments can be compared
+           array for array.  Above DUMP_BYTES every array keeps the same fraction of its rows, picked with a fixed seed.
 """
 from __future__ import annotations
 
@@ -49,6 +54,7 @@ UNIT = "Mpoints/s"
 DTYPE = "bf16x3-split/f32-acc"        # every product is hi.hi + hi.lo + lo.hi of bf16 halves (16 mantissa bits), fp32 accumulation
 REF_BUDGET_S = 330.0                  # the reference arm's whole run (warm-up + steps) stays within a few minutes
 CPU_BASELINE_S = 15.0                 # the cpu_baseline leg of the repo arm: one bounded sample
+DUMP_BYTES = 60_000_000               # --dump-outputs: array bytes at most (with the .npy headers, under 64 MB)
 
 
 def _peaks():
@@ -175,6 +181,32 @@ def run_reference(args):
 
 
 # ----------------------------------------------------------------------------- the repo arm
+def _exact_float(a: np.ndarray) -> np.ndarray:
+    if a.dtype.kind == "f":
+        return a.astype(np.float32 if a.dtype.itemsize <= 4 else np.float64)
+    return a.astype(np.float32 if a.size == 0 or int(np.abs(a.astype(np.int64)).max()) < (1 << 24) else np.float64)
+
+
+def dump_outputs(path: str, out: dict):
+    """Write what one step computed (step(keep=...)) as path/<name>.npy; see --dump-outputs in the module docstring."""
+    import torch
+    lohi = [t.cpu().numpy().view(np.uint32) for t in out["lohi"]]      # [4 * level + stage], levels coarse -> fine
+    arrays = {"base_xyz": out["base_xyz"], "base_occ": out["base_occ"],
+              "occupancy": torch.cat(out["occupancy"]).cpu().numpy() if out["occupancy"] else np.zeros(0, np.uint8)}
+    for i in range(4):
+        w = np.concatenate(lohi[i::4]) if lohi else np.zeros(0, np.uint32)
+        arrays[f"cdf_bounds_stage{i}"] = np.stack([w & 0xFFFF, w >> 16], axis=1)
+    arrays["points"] = out["points"].cpu().numpy()
+    arrays = {k: _exact_float(np.asarray(v)) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = a.shape[0] * DUMP_BYTES // total
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -185,7 +217,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; --impl reference does not run it")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -217,13 +254,17 @@ def main():
     from gauspcc_b200.pcc_utils import calculate_morton_order
     x_dev = x_dev[calculate_morton_order(x_dev)]                     # as HAC hands it over (gaussian_model.py:1108-1109)
 
-    def step():
+    def step(keep=None):
         """one encode + decode; returns only scalars: a step must not keep the previous step's device buffers alive (the caching
-        allocator would cudaMalloc a second and third working set inside the timed region: 149-203 ms per step instead of 135)"""
-        bx, bo, _, aux = codec.encode(x_dev, download=False)
+        allocator would cudaMalloc a second and third working set inside the timed region: 149-203 ms per step instead of 135).
+        keep (a dict, only on the last timed step) receives the arrays a caller of the path gets back, for --dump-outputs.  With
+        --dump-outputs every step keeps its CDF words to the end, so the warm-up sizes the allocator's pool for the timed steps."""
+        bx, bo, _, aux = codec.encode(x_dev, download=False, keep_lohi=bool(args.dump_outputs))
         n_enc = codec.launches
         occs = [lv.occ for lv in aux["levels"][1:]]
         out = codec.decode(bx, bo, [b""] * (4 * len(occs)), forced_occ=occs)
+        if keep is not None:
+            keep.update(base_xyz=bx, base_occ=bo, occupancy=occs, lohi=aux["lohi"], points=out)
         return int(out.shape[0]), n_enc + codec.launches, (int(len(aux["levels"]) - 1), int(sum(l.n for l in aux["levels"][1:])))
 
     def barrier():
@@ -241,10 +282,11 @@ def main():
         sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     launches = 0
+    last = {} if args.dump_outputs and rank == 0 else None
     t_wall0 = time.perf_counter()
     e0.record(torch.cuda.current_stream(dev))
-    for _ in range(args.steps):
-        n_out, nl, (n_levels, n_symbol_rows) = step()
+    for it in range(args.steps):
+        n_out, nl, (n_levels, n_symbol_rows) = step(last if it == args.steps - 1 else None)
         launches += nl
     e1.record(torch.cuda.current_stream(dev))
     barrier()
@@ -252,6 +294,9 @@ def main():
     sampler.stop_flag.set()
     if sampler.is_alive():
         sampler.join()
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
+        last = None
     ms = e0.elapsed_time(e1)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:

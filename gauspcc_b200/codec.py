@@ -773,7 +773,8 @@ class GausPcgcCodec:
                                             sym_out.ctypes.data_as(C.c_void_p)), "gpc_ac_decode_h")
 
     # ------------------------------------------------------------------ encode
-    def _encode_level(self, d: int, parent: Level, gt: Level, collect: bool, download: bool, gpu_chunk: int, aux, carve, level_futs):
+    def _encode_level(self, d: int, parent: Level, gt: Level, collect: bool, download: bool, gpu_chunk: int, keep_lohi: bool, aux, carve,
+                      level_futs):
         """one octree level of the encoder on the current stream: features, four stages, (c_low, c_high) words on their way to the coder"""
         child, u = self.level_features(parent, gt.n, child_kmap=gt.kmap)      # same coordinate set, same row order
         if collect:
@@ -791,6 +792,8 @@ class GausPcgcCodec:
                 lohi_h = carve(gt.n * 4, torch.int32, (gt.n,))
                 lohi_h.copy_(lohi_d, non_blocking=True)
                 level_jobs.append(lohi_h)
+            elif keep_lohi:
+                aux["lohi"][4 * d + i] = lohi_d
             if collect:
                 aux["probs"][4 * d + i] = prob_d
                 aux["cdfs"][4 * d + i] = cdf_d
@@ -800,15 +803,19 @@ class GausPcgcCodec:
             # host range coding of this level overlaps the GPU work of the coarser levels
             level_futs[d] = [self.pool.submit(self._ac_encode_lohi, h.numpy().view(np.uint32), ready) for h in level_jobs]
 
-    def encode(self, xyz: torch.Tensor, collect: bool = False, download: bool = True, gpu_chunk: int = 0):
+    def encode(self, xyz: torch.Tensor, collect: bool = False, download: bool = True, gpu_chunk: int = 0, keep_lohi: bool = False):
         """[N,3] CUDA float32/int32 voxel indices -> (base_xyz int32 [n0,3], base_occ u8 [n0], streams, aux).
 
         download=False (bench, device-timed number): the CDF rows and symbols stay in HBM, nothing is copied to
         the host and the range coder does not run (streams is None); the device work is unchanged.
+        keep_lohi (download=False only): aux["lohi"][4 * d + i] holds what the range coder would take for stage i of level d, one
+        int32 c_low | c_high << 16 per row; otherwise each stage's buffer is released as soon as its level is done.
         gpu_chunk > 0 (container version 2, SURVEY 8f-3; NOT the reference bitstream): the streams are coded on the GPU in chunks
         of gpu_chunk symbols (csrc/attr_ac.cu: one warp per chunk) -- no host range coder, only compressed bytes cross PCIe.
         A stream is then `u16 bytes_of_chunk[chunks]` followed by the chunks' bytes.
         """
+        if keep_lohi and download:
+            raise ValueError("keep_lohi needs download=False: a downloading encode hands the words to the range coder")
         self._launch_base = int(self.lib.gpc_launch_count())
         self._segments = []
         self._stream_h = torch.cuda.current_stream(self.dev).cuda_stream
@@ -840,6 +847,8 @@ class GausPcgcCodec:
         cursor = 0
         futs = []
         aux = {"levels": levels, "probs": [], "cdfs": []} if (collect or not download) else None
+        if keep_lohi:
+            aux["lohi"] = [None] * (4 * L)
 
         def carve(nbytes, dtype, shape):
             nonlocal cursor
@@ -883,7 +892,7 @@ class GausPcgcCodec:
                 st = sides[slot - 1] if slot else None
             with (torch.cuda.stream(st) if st is not None else contextlib.nullcontext()):
                 self._stream_h = st.cuda_stream if st is not None else main_h
-                self._encode_level(d, parent, gt, collect, download, gpu_chunk, aux, carve, level_futs)
+                self._encode_level(d, parent, gt, collect, download, gpu_chunk, keep_lohi, aux, carve, level_futs)
         self._stream_h = main_h
         for st in sides:
             main.wait_stream(st)

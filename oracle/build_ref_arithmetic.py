@@ -5,7 +5,7 @@ the reference's own flags (setup.py: -O2) for sm_100a, and only the shared objec
 travels to the GPU box).  tests/test_attr_coder.py and tests/bench_attr_coder.py import it when present to compare the library's
 streams and symbols with the reference kernels' on the same B200; nothing in gauspcc_b200/ ever loads it.
 
-    python oracle/build_ref_arithmetic.py [/root/reference]
+    python oracle/build_ref_arithmetic.py <checkout of the reference>
 """
 import glob
 import os
@@ -18,7 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.path.join(HERE, "_ref", "arithmetic.so")
 
 
-def build(reference_root="/root/reference", force=False):
+def build(reference_root, force=False):
     zpath = os.path.join(reference_root, "src/gs_compress/HAC/submodules/arithmetic.zip")
     if not os.path.exists(zpath):
         return None
@@ -42,7 +42,7 @@ def build(reference_root="/root/reference", force=False):
 
 
 def load_module():
-    """import the built extension as a Python module, or None when it was never built (e.g. no /root/reference at build time)"""
+    """import the built extension as a Python module, or None when it was never built"""
     if not os.path.exists(OUT):
         return None
     import importlib.util
@@ -54,4 +54,6 @@ def load_module():
 
 
 if __name__ == "__main__":
-    print(build(sys.argv[1] if len(sys.argv) > 1 else "/root/reference", force=True))
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    print(build(sys.argv[1], force=True))

@@ -1,8 +1,9 @@
 """SURVEY 8f-4: HAC's chunked attribute coder (HAC/submodules/arithmetic.zip!arithmetic/arithmetic_kernel.cu, callers
 HAC/utils/encodings_cuda.py:317-500) -- the library's kernels (csrc/attr_ac.cu) behind gauspcc_b200.arithmetic /
-gauspcc_b200.encodings_cuda against the CPU oracle and, when oracle/_ref/arithmetic.so was built from the reference's own
-sources (oracle/build_ref_arithmetic.py), against the reference extension itself on the same GPU: bytes, per-chunk counts and
-decoded symbols must be identical."""
+gauspcc_b200.encodings_cuda against the CPU oracle, against the stored tables and streams of tests/golden/attr_golden.npz
+(tests/golden/make_attr_golden.py says where they come from) and, when oracle/_ref/arithmetic.so was built from the reference's
+own sources (GPC_REFERENCE_ROOT at build time), against the reference extension itself on the same GPU: bytes, per-chunk counts
+and decoded symbols must be identical."""
 import os
 import sys
 
@@ -11,6 +12,7 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CHUNK = 10000                                                               # encodings_cuda.py:6
+CASES = [(1, 0, False), (9999, 1, False), (10000, 2, False), (10001, 3, True), (123457, 4, True)]       # n, seed, tiny_scale
 
 
 def _case(n, seed, q=0.5, spread=3.0, tiny_scale=False):
@@ -78,7 +80,12 @@ def test_python_boundary_matches_reference_names():
 @pytest.fixture(scope="module")
 def ref_ext():
     from oracle import build_ref_arithmetic
-    return build_ref_arithmetic.load_module()                               # None when the reference was not present at build time
+    return build_ref_arithmetic.load_module()                               # None unless built (GPC_REFERENCE_ROOT at build time)
+
+
+@pytest.fixture(scope="module")
+def ref_golden(golden_dir):
+    return np.load(os.path.join(golden_dir, "attr_golden.npz"))
 
 
 def _dev(*arrays):
@@ -87,8 +94,8 @@ def _dev(*arrays):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("n,seed,tiny", [(1, 0, False), (9999, 1, False), (10000, 2, False), (10001, 3, True), (123457, 4, True)])
-def test_gaussian_coder_vs_oracle_and_reference(n, seed, tiny, ref_ext):
+@pytest.mark.parametrize("n,seed,tiny", CASES)
+def test_gaussian_coder_vs_oracle_and_reference(n, seed, tiny, ref_ext, ref_golden):
     import torch
     from gauspcc_b200 import arithmetic as A
     from oracle import oracle as O
@@ -112,7 +119,12 @@ def test_gaussian_coder_vs_oracle_and_reference(n, seed, tiny, ref_ext):
     g_stream, g_cnt = A.gaussian_encode(d_sym, d_mean, d_scale, d_Q, mn, mx, CHUNK)
     assert torch.equal(g_cnt, cnt) and torch.equal(g_stream, stream)
     assert np.array_equal(A.gaussian_decode(d_mean, d_scale, d_Q, g_stream, g_cnt, mn, mx, CHUNK).cpu().numpy(), sym)
-    # 4. the reference extension on the same GPU (built from the reference's own sources)
+    # 4. the stored tables and streams (provenance in tests/golden/make_attr_golden.py), and the reference extension itself on
+    # the same GPU when it was built from the reference's own sources
+    tag = f"n{n}_s{seed}"
+    rows = torch.from_numpy(ref_golden[tag + "_rows"]).cuda()
+    assert np.array_equal(lower[rows].cpu().numpy(), ref_golden[tag + "_lower"])
+    assert np.array_equal(cnt.cpu().numpy(), ref_golden[tag + "_cnt"]) and np.array_equal(stream.cpu().numpy(), ref_golden[tag + "_stream"])
     if ref_ext is not None:
         r_lower = ref_ext.calculate_cdf(d_mean, d_scale, d_Q, mn, mx)
         assert torch.equal(r_lower, lower)
