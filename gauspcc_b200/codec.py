@@ -32,6 +32,7 @@ STAGE_SHIFT = (7, 6, 4, 0)       # sym_i = (occ >> shift) & mask   (pcc_utils.py
 STAGE_MASK = (1, 1, 3, 15)
 CTX_SHIFT = (None, 7, 6, 4)      # ctx_i = occ >> shift            (pcc_utils.py:122,129,137)
 BASE_ROWS = 64                   # FOG loop stops when a level has < 64 rows (pcc_utils.py:87)
+UM_TILE_ROWS = 512               # output rows per CTA of the tcgen05 conv: the one tile height spconv_um.cu builds (DESIGN.md 5)
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -117,8 +118,6 @@ class GausPcgcCodec:
         self.adaptive_tiles = tile_rows is None       # tests: a fixed tile height / kernel variant of the mma.sync conv on every level
         self.tile_rows = int(tile_rows or 64)
         self.v6_variant = 42
-        self.um_order_tiles = True                    # tcgen05 conv: CTAs take the level's tiles heaviest first (shorter tail)
-        self.um_tile_rows = 512                       # output rows per CTA of the tcgen05 conv (256 / 384 / 512 / 1024 are built)
         self._fns: Dict[str, object] = {}
         self._stream_h = None
         n_thr = ac_threads or int(os.environ.get("GPC_AC_THREADS", min(16, len(os.sched_getaffinity(0)))))
@@ -132,19 +131,13 @@ class GausPcgcCodec:
         self.wave_decode = True
         self.wave_min_rows = 150_000
         self.wave_chunk_rows = 32768
-        self.wave_plane_lag = True                    # stage i+1 trails stage i by planes, not by two chunks
-        self.wave_streams = True
         self._wave_side: Optional[list] = None
         self._wave_buf: Optional[torch.Tensor] = None
-        self.enc_overlap = 1                          # encoder: side streams; the levels (independent work) take main and these in turn (0 / 1 / 2-6 side streams: 61.8 / 56.4 / 56.5-57.8 ms per 1M-anchor encode)
-        self._enc_sides = []
-        self.dec_overlap = True                       # decoder: children + their kernel map on a side stream beside the prior stack
-        self._dec_side = None
+        self._enc_side = None                         # encoder: levels run on the main stream and this one (encode())
+        self._dec_side = None                         # decoder: children + their kernel map beside the prior stack (level_features())
         self._coder_arena = None                      # (c_low, c_high) words of all streams of a scene (container version 2)
         self.wave_log: Optional[list] = None          # tools/wave_times.py: per-level record of the wavefront
         self.debug_dec_cdfs: Optional[dict] = None    # tests: (level, stage) -> CDF rows the stage-by-stage decoder computed
-        self.wave_first_rows = 8192                   # size / number of the small leading chunks
-        self.wave_first_chunks = 0                    # measured: small leading chunks cost more than they save (dec 0.242 vs 0.218 s)
         self._launch_base = 0
         self.last_stats: Dict[str, float] = {}
         self._segments: List[Tuple[torch.cuda.Event, torch.cuda.Event]] = []
@@ -363,9 +356,9 @@ class GausPcgcCodec:
         off = self._empty((max(n_pairs, 1),), torch.int32)
         self._call("gpc_kmap_um_fill", _ptr(dense), n, tr, _ptr(seg), _ptr(nbr), _ptr(off), self._stream())
         km = KMap(seg, None, n_pairs, tr, n_real=n_real, um_rows=tr, pair_nbr=nbr, pair_off=off)
-        if self.um_order_tiles:
-            starts = seg[::126].to(torch.int64)                  # first stream entry of every tile (+ the end of the last)
-            km.tile_order = torch.argsort(starts[1:] - starts[:-1], descending=True, stable=True).to(torch.int32)
+        # CTAs take the level's tiles heaviest first (shorter tail)
+        starts = seg[::126].to(torch.int64)                      # first stream entry of every tile (+ the end of the last)
+        km.tile_order = torch.argsort(starts[1:] - starts[:-1], descending=True, stable=True).to(torch.int32)
         return km
 
     def _sparse_map(self, dense: torch.Tensor, n: int) -> KMap:
@@ -425,13 +418,9 @@ class GausPcgcCodec:
             return self._sparse_map(self.dense_map(keys), n)
         # big level: the probes count the pairs per (tile of the tcgen05 conv, offset): density (pairs per row, centre included) and
         # the first pass of the pair stream in one
-        tr = self.um_tile_rows
-        if tr >= 256:
-            dense, cells = self.dense_map(keys, tr)
-            counted = self._scan_um(cells, n, tr)
-        else:
-            dense = self.dense_map(keys)
-            counted = self._count_um(dense, n, tr)
+        tr = UM_TILE_ROWS
+        dense, cells = self.dense_map(keys, tr)
+        counted = self._scan_um(cells, n, tr)
         density = counted[2] / max(n, 1)
         if family is None:
             if n >= self.sparse_min_rows and 0 < self.sparse_max_density and density < self.sparse_max_density and n < 30_000_000:
@@ -577,7 +566,7 @@ class GausPcgcCodec:
         with self._stage("embed", parent.n * 129):
             self._call("gpc_embed_rows", _ptr(parent.occ), parent.n, _ptr(self.w.prior_emb), None if pum else _ptr(f), _ptr(f) if pum else None,
                        self._stream())
-        if child_kmap is None and self.dec_overlap and self.conv_profile is None and n_child >= 20_000:
+        if child_kmap is None and self.conv_profile is None and n_child >= 20_000:
             # decoder: the children and their kernel map depend on the parents' occupancy only, not on the prior features --
             # they are built on a side stream (incl. the host round trip of the pair counts) while the prior stack runs
             main = torch.cuda.current_stream(self.dev)
@@ -746,15 +735,6 @@ class GausPcgcCodec:
         return sym
 
     # ------------------------------------------------------------------ host range coder
-    def _ac_encode(self, cdf: np.ndarray, sym: np.ndarray) -> bytes:
-        n, Lp = cdf.shape
-        cap = 4 * n + 64
-        out = np.empty(cap, dtype=np.uint8)
-        ln = C.c_int64(0)
-        _lib.check(self.lib.gpc_ac_encode_h(cdf.ctypes.data_as(C.c_void_p), sym.ctypes.data_as(C.c_void_p), n, Lp,
-                                            out.ctypes.data_as(C.c_void_p), cap, C.byref(ln)), "gpc_ac_encode_h")
-        return out[:ln.value].tobytes()
-
     def _ac_encode_lohi(self, lohi: np.ndarray, ready: Optional[torch.cuda.Event] = None) -> bytes:
         if ready is not None:
             ready.synchronize()                        # the level's D2H copies have landed (GPU keeps running later levels)
@@ -871,31 +851,28 @@ class GausPcgcCodec:
             self._chunk_begin([levels[k // 4 + 1].n for k in range(4 * L)], gpu_chunk)
         if collect:
             aux["child_keys"], aux["probs"], aux["cdfs"] = [None] * L, [None] * (4 * L), [None] * (4 * L)
-        # Every level of the encoder is independent work: the levels are spread over the main stream and enc_overlap side streams,
-        # so that one level's launch tails, pipeline ramps and small kernels (embeddings, heads, the 15-180 us launches of the coarse
-        # levels) run beside another level's convs.  Not while bench.py's per-stage profile is on (its event pairs assume one stream).
-        sides = []
+        # Every level of the encoder is independent work: the levels are spread over the main stream and one side stream, so that
+        # one level's launch tails, pipeline ramps and small kernels (embeddings, heads, the 15-180 us launches of the coarse levels)
+        # run beside another level's convs (0 / 1 / 2-6 side streams: 61.8 / 56.4 / 56.5-57.8 ms per 1M-anchor encode).  Not while
+        # bench.py's per-stage profile is on (its event pairs assume one stream).
+        side = None
         main = torch.cuda.current_stream(self.dev)
-        if self.enc_overlap and self.conv_profile is None and not collect and L > 1:
-            while len(self._enc_sides) < self.enc_overlap:
-                self._enc_sides.append(torch.cuda.Stream(self.dev))
-            sides = self._enc_sides[:self.enc_overlap]
-            for st in sides:
-                st.wait_stream(main)                                           # pyramid and kernel maps are complete
+        if self.conv_profile is None and not collect and L > 1:
+            if self._enc_side is None:
+                self._enc_side = torch.cuda.Stream(self.dev)
+            side = self._enc_side
+            side.wait_stream(main)                                             # pyramid and kernel maps are complete
         main_h = self._stream_h
         for d in range(L - 1, -1, -1):
             parent, gt = levels[d], levels[d + 1]
-            # big levels take main and the side streams in turn; the coarse levels all go to the last side stream
-            st = None
-            if sides:
-                slot = (L - 1 - d) % (len(sides) + 1) if gt.n >= self.um_min_rows else len(sides)
-                st = sides[slot - 1] if slot else None
+            # big levels alternate main, side, main, ... (finest first); the coarse levels all go to the side stream
+            st = side if side is not None and (gt.n < self.um_min_rows or (L - 1 - d) % 2) else None
             with (torch.cuda.stream(st) if st is not None else contextlib.nullcontext()):
                 self._stream_h = st.cuda_stream if st is not None else main_h
                 self._encode_level(d, parent, gt, collect, download, gpu_chunk, keep_lohi, aux, carve, level_futs)
         self._stream_h = main_h
-        for st in sides:
-            main.wait_stream(st)
+        if side is not None:
+            main.wait_stream(side)
         futs = [f for lf in level_futs for f in lf]            # stream order of the container: level-major coarse -> fine
         base = levels[0]
         base_xyz = self._empty((base.n, 3), torch.int32)
@@ -924,32 +901,23 @@ class GausPcgcCodec:
     # -> stage i+1.  The dependency is local, though: stage i+1 of a row needs the stage-i symbols of the rows within two 5^3 convs
     # of it, and rows are sorted by (z, y, x).  So stage 0 is handed to its decoder in chunks of rows; whenever decoder i reports a
     # piece, the GPU computes the stage-(i+1) CDFs of every row whose neighbourhood is now decoded (_wave_plan: a lag of a few
-    # z planes; wave_plane_lag = False: the older scheme with a lag of two whole chunks), and the four stage streams decode on four
-    # host threads, one piece behind each other.  Same kernels, same sums, same bitstream; the serial range decoder (0.28 s of a
-    # 0.35 s decode at 1M anchors) overlaps with itself.
+    # z planes), and the four stage streams decode on four host threads, one piece behind each other.  Same kernels, same sums,
+    # same bitstream; the serial range decoder (0.28 s of a 0.35 s decode at 1M anchors) overlaps with itself.
     def _wave_ok(self, child: Level, n: int) -> bool:
         km = child.kmap
         if not self.wave_decode or n < self.wave_min_rows:
             return False
-        if not (km.sparse or ((km.um_rows or km.v6_variant == 48) and self.wave_chunk_rows % km.tile_rows == 0
-                              and self.wave_first_rows % km.tile_rows == 0)):
+        if km.sparse:
+            tile = 8192                     # the sparse conv's row blocks
+        elif km.um_rows or km.v6_variant == 48:
+            tile = km.tile_rows
+        else:
             return False
-        if km.sparse and (self.wave_chunk_rows % 8192 or self.wave_first_rows % 8192):
-            return False
-        chunks = self._wave_chunks(n)
-        nc = len(chunks)
-        if self.wave_plane_lag:
-            return nc >= 2                  # the plan (_wave_plan) is valid for any geometry; it degenerates to stage by stage at worst
-        if nc < 3:
-            return False
-        # every 5^3 neighbour of a row of chunk c must lie in chunks c-1 .. c+1: first z of chunk c minus last z of chunk c-2 >= 3
-        idx = torch.tensor([r0 for r0, _ in chunks] + [r1 - 1 for _, r1 in chunks], device=self.dev)
-        z = (child.keys[idx] >> 42).cpu().numpy()
-        zf, zl = z[:nc], z[nc:]
-        return bool(np.all(zf[2:] - zl[:-2] >= 3))
+        # the plan (_wave_plan) is valid for any geometry; it degenerates to stage by stage at worst
+        return self.wave_chunk_rows % tile == 0 and len(self._wave_chunks(n)) >= 2
 
     def _wave_plan(self, keys: torch.Tensor, n: int, chunks: List[Tuple[int, int]], tile: int):
-        """Row ranges of the wavefront with a lag of PLANES instead of chunks.  Rows are sorted by (z, y, x); if stage i is known for
+        """Row ranges of the wavefront: each stage lags the previous one by a few z PLANES.  Rows are sorted by (z, y, x); if stage i is known for
         the rows < e, the first conv of stage i+1 is exact for every row whose 5^3 neighbours are all < e: the planes z <= z[e] - 3,
         i.e. the rows before the first row of plane z[e] - 2 (rounded down to the conv's tile height); the second conv, likewise, for
         the rows two more planes back; those rows' CDFs go to decoder i+1.  Returns per stage the piece ends E[i][c] (stage 0: the
@@ -972,20 +940,9 @@ class GausPcgcCodec:
         return flat[:4], flat[4:]
 
     def _wave_chunks(self, n: int) -> List[Tuple[int, int]]:
-        """Row chunks of a wavefront level: a few small ones first (stage i+1 starts three chunks behind stage i, so the first
-        chunks set how long the later stages' decoders wait at the start of a level), then wave_chunk_rows each."""
-        ch, small = self.wave_chunk_rows, self.wave_first_rows
-        sizes = [small] * self.wave_first_chunks if 0 < small < ch else []
-        out, r = [], 0
-        for sz in sizes:
-            if r + sz >= n:
-                break
-            out.append((r, r + sz))
-            r += sz
-        while r < n:
-            out.append((r, min(r + ch, n)))
-            r += ch
-        return out
+        """Row chunks of a wavefront level: wave_chunk_rows each, the last one ragged"""
+        ch = self.wave_chunk_rows
+        return [(r, min(r + ch, n)) for r in range(0, n, ch)]
 
     def _decode_level_wavefront(self, u, child: Level, n: int, streams: List[bytes], occ: torch.Tensor):
         km = child.kmap
@@ -1053,7 +1010,7 @@ class GausPcgcCodec:
         # 442 K rows) outlasted the decoders (0.55 ms).  Stage j's work runs on stream j; what it reads from other stages (symbols,
         # occupancy bits) has reached the host before it is enqueued, and at any moment the stages work on disjoint chunks.  The
         # sparse levels (decoder-bound, and their convs share the level's contribution scratch) stay on the one stream.
-        multi = self.wave_streams and not km.sparse
+        multi = not km.sparse
         if multi and self._wave_side is None:
             self._wave_side = [torch.cuda.Stream(device=self.dev) for _ in range(3)]
         S = [stream] + (self._wave_side if multi else [stream] * 3)
@@ -1078,12 +1035,8 @@ class GausPcgcCodec:
             ev.record(S[i])                                    # the launch thread needs)
             ev_q[i].put(ev)
 
-        plane = self.wave_plane_lag
-        if plane:
-            E, CA = self._wave_plan(child.keys, n, chunks, 8192 if km.sparse else km.tile_rows)
-            P = [[(E[i][c - 1] if c else 0, E[i][c]) for c in range(nc)] for i in range(4)]
-        else:
-            P = [chunks] * 4
+        E, CA = self._wave_plan(child.keys, n, chunks, 8192 if km.sparse else km.tile_rows)
+        P = [[(E[i][c - 1] if c else 0, E[i][c]) for c in range(nc)] for i in range(4)]
         workers = [self.pool.submit(worker, i) for i in range(4)]
         t_wait = 0.0
         try:
@@ -1108,41 +1061,23 @@ class GausPcgcCodec:
                 pending -= 1
                 j = min(i + 1, 3)
                 sh = self._stream_h = SH[j]           # everything this completion triggers goes to the next stage's stream
-                if plane:
-                    r0, r1 = P[i][c]
-                    if r1 > r0:
-                        call("gpc_copy_async", p_sym_d[i] + r0, p_sym_h[i] + r0, r1 - r0, sh)
-                        call("gpc_merge_symbol", p_occ + r0, r1 - r0, STAGE_SHIFT[i], p_sym_d[i] + r0, sh)
-                    if i == 3:
-                        continue
-                    k0, k1 = W.stage_convs(j)
-                    if r1 > r0:
-                        call("gpc_add_ctx_embed", p_u + r0 * 128, p_occ + r0, CTX_SHIFT[j], embs[j], r1 - r0,
-                             None if um else p_f[j] + r0 * 128, p_f[j] + r0 * 128 if um else None, sh)
-                    a0, a1 = (CA[j][c - 1] if c else 0), CA[j][c]
-                    if a1 > a0:
-                        self.conv(f[j], k0, km, relu=True, out=t0[j], rows=(a0, a1), fmt=cfmt)
-                    q0, q1 = P[j][c]
-                    if q1 > q0:
-                        self.conv(t0[j], k1, km, out=t1[j], rows=(q0, q1))
-                        emit_cdf(j, c, (q0, q1))
-                    continue
-                r0, r1 = chunks[c]
-                call("gpc_copy_async", p_sym_d[i] + r0, p_sym_h[i] + r0, r1 - r0, sh)
-                call("gpc_merge_symbol", p_occ + r0, r1 - r0, STAGE_SHIFT[i], p_sym_d[i] + r0, sh)
+                r0, r1 = P[i][c]
+                if r1 > r0:
+                    call("gpc_copy_async", p_sym_d[i] + r0, p_sym_h[i] + r0, r1 - r0, sh)
+                    call("gpc_merge_symbol", p_occ + r0, r1 - r0, STAGE_SHIFT[i], p_sym_d[i] + r0, sh)
                 if i == 3:
                     continue
                 k0, k1 = W.stage_convs(j)
-                call("gpc_add_ctx_embed", p_u + r0 * 128, p_occ + r0, CTX_SHIFT[j], embs[j], r1 - r0,
-                     None if um else p_f[j] + r0 * 128, p_f[j] + r0 * 128 if um else None, sh)
-                last = c == nc - 1
-                for cc in ([c - 1] if c >= 1 else []) + ([c] if last else []):          # first conv: inputs of chunks cc-1 .. cc+1 are there
-                    self.conv(f[j], k0, km, relu=True, out=t0[j], rows=chunks[cc], fmt=cfmt)
-                for cc in ([c - 2] if c >= 2 else []) + ([c - 1, c] if last else []):
-                    if cc < 0:
-                        continue
-                    self.conv(t0[j], k1, km, out=t1[j], rows=chunks[cc])
-                    emit_cdf(j, cc)
+                if r1 > r0:
+                    call("gpc_add_ctx_embed", p_u + r0 * 128, p_occ + r0, CTX_SHIFT[j], embs[j], r1 - r0,
+                         None if um else p_f[j] + r0 * 128, p_f[j] + r0 * 128 if um else None, sh)
+                a0, a1 = (CA[j][c - 1] if c else 0), CA[j][c]
+                if a1 > a0:
+                    self.conv(f[j], k0, km, relu=True, out=t0[j], rows=(a0, a1), fmt=cfmt)
+                q0, q1 = P[j][c]
+                if q1 > q0:
+                    self.conv(t0[j], k1, km, out=t1[j], rows=(q0, q1))
+                    emit_cdf(j, c, (q0, q1))
         except BaseException:
             for q in ev_q:
                 q.put(None)                       # let the decoder threads go

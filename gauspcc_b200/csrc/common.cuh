@@ -78,11 +78,6 @@ __host__ __device__ __forceinline__ u64 key_compact(u64 k, gpc_key_xform t) {
 }
 
 // ---------------------------------------------------------------- bf16 hi / lo split of fp32 (x = hi + lo + O(2^-17 x))
-__device__ __forceinline__ u32 pack_bf16x2(float lo, float hi) {
-    u32 r;
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));      // upper half <- first source
-    return r;
-}
 __device__ __forceinline__ float bf16_round(float v) {                       // round-to-nearest-even to bf16, as fp32
     u32 u = __float_as_uint(v);
     u += 0x7FFFu + ((u >> 16) & 1u);

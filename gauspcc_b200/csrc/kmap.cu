@@ -161,69 +161,12 @@ extern "C" int gpc_kmap_dense(const void *table, int64_t capacity, const uint64_
 
 // ---------------------------------------------------------------- per-tile pair lists grouped by offset
 // counts[t*126 + k] = number of rows of tile t with a neighbour at offset k (k = 125 is a zero pad so
-// that the exclusive scan leaves seg[t*126+125] == start of tile t+1).
-constexpr int KP_THREADS = 256;
-
-__global__ void __launch_bounds__(KP_THREADS) kmap_pairs_count_kernel(const i32 *__restrict__ map, i64 n, int tile_rows, int pad,
-                                                                     u32 *__restrict__ counts, u32 *__restrict__ n_real) {
-    __shared__ u32 cnt[GPC_K3 + 1];
-    const i64 t = blockIdx.x;
-    const i64 r0 = t * tile_rows;
-    const int rows = (int)min((i64)tile_rows, n - r0);
-    for (int i = threadIdx.x; i <= GPC_K3; i += KP_THREADS) cnt[i] = 0;
-    __syncthreads();
-    for (int k = 0; k < GPC_K3; ++k) {
-        u32 c = 0;
-        for (int r = threadIdx.x; r < rows; r += KP_THREADS) c += map[(i64)k * n + r0 + r] >= 0;
-        c = __reduce_add_sync(0xFFFFFFFFu, c);
-        if ((threadIdx.x & 31) == 0 && c) atomicAdd(&cnt[k], c);
-    }
-    __syncthreads();
-    // pad > 1: every non-empty segment is rounded up to a multiple of `pad` entries (8-pair MMA tiles of one offset)
-    for (int i = threadIdx.x; i <= GPC_K3; i += KP_THREADS) counts[t * (GPC_K3 + 1) + i] = (cnt[i] + pad - 1) / pad * pad;
-    if (threadIdx.x == 0) { u32 tot = 0; for (int i = 0; i < GPC_K3; ++i) tot += cnt[i]; atomicAdd(n_real, tot); }
-}
-
+// that the exclusive scan leaves seg[t*126+125] == start of tile t+1).  pad > 1: every non-empty count is rounded up to a
+// multiple of `pad` entries (8-pair MMA tiles of one offset).
 __global__ void kmap_total_kernel(const u32 *__restrict__ seg, i64 m, u32 *__restrict__ n_pairs) { *n_pairs = seg[m]; }
 
-__global__ void __launch_bounds__(KP_THREADS) kmap_pairs_fill_kernel(const i32 *__restrict__ map, i64 n, int tile_rows,
-                                                                    const u32 *__restrict__ seg, u32 *__restrict__ pair_nbr,
-                                                                    u16 *__restrict__ pair_row, u64 *__restrict__ pairs) {
-    __shared__ u32 warp_cnt[KP_THREADS / 32];
-    __shared__ u32 running;
-    const i64 t = blockIdx.x;
-    const i64 r0 = t * tile_rows;
-    const int rows = (int)min((i64)tile_rows, n - r0);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int k = 0; k < GPC_K3; ++k) {
-        const u32 seg_begin = seg[t * (GPC_K3 + 1) + k];
-        if (seg[t * (GPC_K3 + 1) + k + 1] == seg_begin) continue;          // block-uniform
-        if (threadIdx.x == 0) running = 0;
-        __syncthreads();
-        for (int rbase = 0; rbase < rows; rbase += KP_THREADS) {           // ascending row order inside a segment
-            const int r = rbase + threadIdx.x;
-            const i32 nb = r < rows ? map[(i64)k * n + r0 + r] : -1;
-            const u32 ballot = __ballot_sync(0xFFFFFFFFu, nb >= 0);
-            if (lane == 0) warp_cnt[warp] = __popc(ballot);
-            __syncthreads();
-            u32 before = running;
-            for (int w = 0; w < warp; ++w) before += warp_cnt[w];
-            if (nb >= 0) {
-                const u32 p = seg_begin + before + __popc(ballot & ((1u << lane) - 1u));
-                if (pair_nbr) { pair_nbr[p] = (u32)nb; pair_row[p] = (u16)r; }
-                if (pairs) pairs[p] = (u64)(u32)nb | ((u64)(u32)r << 32) | ((u64)(u32)k << 48);
-            }
-            __syncthreads();
-            if (threadIdx.x == 0) { u32 tot = 0; for (int w = 0; w < KP_THREADS / 32; ++w) tot += warp_cnt[w]; running += tot; }
-            __syncthreads();
-        }
-    }
-}
-
-
-// ---- warp-per-tile variants for small tiles (tile_rows = 32 * RPL, RPL = 1, 2, 4): no block barriers, each warp
-// streams its tile's 125 x tile_rows slice of the dense map with coalesced loads and ballots (the block-per-tile
-// kernels above spend their time in 125 x 3 __syncthreads with a quarter of the threads idle when tiles are small).
+// ---- warp-per-tile kernels (tile_rows = 32 * RPL, RPL = 1, 2, 4): no block barriers, each warp streams its tile's
+// 125 x tile_rows slice of the dense map with coalesced loads and ballots.
 template <int RPL>
 __global__ void __launch_bounds__(128) kmap_pairs_count_warp_kernel(const i32 *__restrict__ map, i64 n, i64 tiles, int pad,
                                                                    u32 *__restrict__ counts, u32 *__restrict__ n_real) {
@@ -323,7 +266,8 @@ extern "C" size_t gpc_kmap_pairs_workspace_bytes(int64_t n, int tile_rows) {
 extern "C" int gpc_kmap_pairs_count(const int32_t *map, int64_t n, int tile_rows, int pad, uint32_t *seg, uint32_t *n_pairs,
                                     void *ws, size_t ws_bytes, void *stream) {
     cudaStream_t st = as_stream(stream);
-    GPC_REQUIRE(tile_rows > 0 && tile_rows <= 65536 && pad >= 1, GPC_EINVAL, "tile_rows must be in 1..65536, pad >= 1");
+    GPC_REQUIRE((tile_rows == 8 || tile_rows == 16 || tile_rows == 32 || tile_rows == 64 || tile_rows == 128) && pad >= 1, GPC_EINVAL,
+                "tile_rows must be 8, 16, 32, 64 or 128, pad >= 1");
     if (n <= 0) { GPC_CUDA_CHECK(cudaMemsetAsync(n_pairs, 0, 8, st)); return GPC_OK; }
     GPC_REQUIRE(ws && ws_bytes >= gpc_kmap_pairs_workspace_bytes(n, tile_rows), GPC_ENOSPC, "workspace too small");
     const i64 tiles = (n + tile_rows - 1) / tile_rows;
@@ -335,8 +279,7 @@ extern "C" int gpc_kmap_pairs_count(const int32_t *map, int64_t n, int tile_rows
     else if (tile_rows == 16) kmap_pairs_count_sub_kernel<16><<<cdiv(tiles, 8), 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
     else if (tile_rows == 32) kmap_pairs_count_warp_kernel<1><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
     else if (tile_rows == 64) kmap_pairs_count_warp_kernel<2><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
-    else if (tile_rows == 128) kmap_pairs_count_warp_kernel<4><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
-    else kmap_pairs_count_kernel<<<(unsigned)tiles, KP_THREADS, 0, st>>>(map, n, tile_rows, pad, counts, n_pairs + 1);
+    else kmap_pairs_count_warp_kernel<4><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
     GPC_LAUNCH_CHECK();
     PtrLoad<u32> pl{counts};
     int rc = device_exclusive_scan<u32, PtrLoad<u32>>(pl, m, seg, scan_ws, st);      // seg has m+1 entries
@@ -348,6 +291,8 @@ extern "C" int gpc_kmap_pairs_count(const int32_t *map, int64_t n, int tile_rows
 extern "C" int gpc_kmap_pairs_fill(const int32_t *map, int64_t n, int tile_rows, const uint32_t *seg, uint32_t *pair_nbr,
                                    uint16_t *pair_row, uint64_t *pairs, int64_t n_entries, void *stream) {
     if (n <= 0) return GPC_OK;
+    GPC_REQUIRE(tile_rows == 8 || tile_rows == 16 || tile_rows == 32 || tile_rows == 64 || tile_rows == 128, GPC_EINVAL,
+                "tile_rows must be 8, 16, 32, 64 or 128");
     // padded streams: entries not written below stay INVALID (all ones)
     if (pairs && n_entries > 0) GPC_CUDA_CHECK(cudaMemsetAsync(pairs, 0xFF, (size_t)n_entries * 8, as_stream(stream)));
     if (pair_nbr && n_entries > 0) {               // split arrays: padding = row 0xFFFFFFFF (out of bounds for the TMA gather: zero fill) / 0xFFFF
@@ -360,8 +305,7 @@ extern "C" int gpc_kmap_pairs_fill(const int32_t *map, int64_t n, int tile_rows,
     else if (tile_rows == 16) kmap_pairs_fill_sub_kernel<16><<<cdiv(tiles, 8), 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
     else if (tile_rows == 32) kmap_pairs_fill_warp_kernel<1><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
     else if (tile_rows == 64) kmap_pairs_fill_warp_kernel<2><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
-    else if (tile_rows == 128) kmap_pairs_fill_warp_kernel<4><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
-    else kmap_pairs_fill_kernel<<<(unsigned)tiles, KP_THREADS, 0, st>>>(map, n, tile_rows, seg, pair_nbr, pair_row, pairs);
+    else kmap_pairs_fill_warp_kernel<4><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
     GPC_LAUNCH_CHECK();
     return GPC_OK;
 }
@@ -369,8 +313,7 @@ extern "C" int gpc_kmap_pairs_fill(const int32_t *map, int64_t n, int tile_rows,
 
 // ---------------------------------------------------------------- pair stream of the tcgen05 conv (spconv_um.cu)
 // Tiles of 256 .. 1024 output rows; one WARP per (tile, offset) cell: the cell's slice of the offset-major dense map is tile_rows
-// consecutive ints, read with coalesced loads and ranked with ballots (the block-per-tile kernels above walk the 125 offsets one
-// after the other with three block barriers each).  Every non-empty cell is padded to a multiple of 16 entries; the stream holds,
+// consecutive ints, read with coalesced loads and ranked with ballots.  Every non-empty cell is padded to a multiple of 16 entries; the stream holds,
 // per entry, the input row (padding: 0xFFFFFFFF = out of bounds for the gather) and the BYTE OFFSET of the pair's accumulator row
 // inside the tile (row * 128; padding: the dummy row tile_rows * 128).
 __global__ void __launch_bounds__(128) kmap_um_count_kernel(const i32 *__restrict__ map, i64 n, int tile_rows, i64 cells,

@@ -9,11 +9,11 @@
 //   A operand  W[k]^T, bf16 hi | lo, in TENSOR MEMORY (32 columns), the 32 output channels replicated into all four lane
 //              quadrants (M = 128): every epilogue warp finds the whole product in the quadrant it may read
 //   B operand  the gathered rows, K-major with 128 B swizzle, in shared memory.  The rows of a chunk are fetched by ONE producer
-//              warp with cp.async (eight lanes x 16 B per row, 16-byte piece j of row r at piece j ^ (r & 7)); completion is an
-//              asynchronous mbarrier arrival (cp.async.mbarrier.arrive.noinc), so the producers never wait for data.  The centre
-//              offset's rows are consecutive: one TMA tile load (cp.async.bulk.tensor, SWIZZLE_128B) per chunk.
-//              (TMA tile::gather4 for the other offsets was built and measured: ~47 clk per UTMALDG issue, lane by lane from
-//              uniform registers, 12 clk per row and SM -- profiles/r02_conv_um.md.)
+//              warp: for the non-centre offsets by TMA tile::gather4 (four arbitrary rows per instruction, issued by one elected
+//              lane), for the centre offset, whose rows are consecutive, by one TMA tile load (cp.async.bulk.tensor, SWIZZLE_128B).
+//              The rows land as transaction bytes on the chunk's mbarrier, with one asynchronous arrival per producer lane after
+//              its cp.async of the chunk's row offsets (cp.async.mbarrier.arrive.noinc), so the producers never wait for data.
+//              (A cp.async gather, eight lanes x 16 B per row, measured the same and was dropped -- profiles/r02_conv_um.md.)
 //   D          fp32 in tensor memory, N columns; six MMAs per chunk (K = 2 x 16 for Whi.xhi, Whi.xlo, Wlo.xhi)
 //   epilogue   tcgen05.ld gives lane = channel, register = pair.  Warp e takes 16 columns of every chunk and adds each to its
 //              output row's fp32 sum in shared memory: one conflict-free 128 B read-modify-write per pair.  Within a chunk the
@@ -28,32 +28,6 @@
 // every warp helps to write the tile out.
 #include <cuda.h>
 #include "umma.cuh"
-
-#ifndef UM512_NPW
-#define UM512_NPW 3         // producer warps / gather slots of the 512-row configuration (A/B)
-#define UM512_GS 4
-#endif
-#ifndef UM512_NMAX
-#define UM512_NMAX 64       // pairs per chunk of the 512-row configuration; 96 (with GS 3, DS 2, NEW 6) halves the chunks of cells of 65..96 pairs (A/B)
-#define UM512_DS 3
-#define UM512_NEW 8
-#endif
-#ifndef UM_MIX_DEN
-#define UM_MIX_DEN 2         // UM_GATHER_TMA == 2: chunks with c % UM_MIX_DEN < UM_MIX_TMA go through TMA, the others through cp.async
-#define UM_MIX_TMA 1
-#endif
-#ifndef UM_GATHER_TMA
-#define UM_GATHER_TMA 1      // 1: the rows of the non-centre offsets by TMA tile::gather4 (A/B, profiles/r02_conv_um.md); 0: cp.async
-#endif
-#ifndef UM_WAIT
-#define UM_WAIT mbar_wait_hint
-#endif
-#ifndef UM_SLEEP_W
-#define UM_SLEEP_W 400       // ns between polls of a weights warp (it waits for a whole offset's MMAs)
-#endif
-#ifndef UM_SLEEP_P
-#define UM_SLEEP_P 100       // ns between polls of a producer waiting for a free slot
-#endif
 
 template <int TM, int NMAX, int GS, int DS, int WS, int NPW>
 struct UmSmem {
@@ -90,7 +64,6 @@ __device__ __forceinline__ float um_lds(u32 addr) {
     return v;
 }
 __device__ __forceinline__ void um_sts(u32 addr, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v)); }
-__device__ __forceinline__ void cp_async4(u32 dst, const void *src) { asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src)); }
 // D[tmem] (+)= A[tmem] . B[smem]^T with the descriptor given as two 32-bit halves (the high half is a constant)
 __device__ __forceinline__ void um_mma(u32 tmem_d, u32 tmem_a, u32 desc_lo, u32 idesc, u32 accumulate) {
     asm volatile("{\n\t.reg .pred p;\n\t.reg .b64 d;\n\tsetp.ne.b32 p, %4, 0;\n\tmov.b64 d, {%2, %5};\n\t"
@@ -122,7 +95,6 @@ spconv_um_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant
                  const void *__restrict__ residual, int flags, float *__restrict__ y, u32 *__restrict__ ys) {
     constexpr int NWARPS = 8 + NEW + (NPW > 3 ? NPW - 3 : 0), NTHREADS = NWARPS * 32;
     constexpr int RS = GS + DS;                  // row-offset ring: a chunk's entries live from its gather to the start of its epilogue
-    constexpr int NQ = NMAX / 4;                 // quads (4 rows = one cp.async instruction) of a full chunk
     constexpr u32 A_COL = DS * NMAX;             // first weight column of tensor memory
     static_assert(A_COL + WS * 32 <= TCOLS, "TMEM columns");
     static_assert(NMAX == 16 * NEW || NMAX == 8 * NEW, "an epilogue warp takes 8 or 16 columns of a chunk");
@@ -202,13 +174,12 @@ spconv_um_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant
             const u32 e = s.tab[c], len = (e >> 12) & 0xFFu, wi = e >> 24, ws = wi % (u32)WS;
             const u32 gs = c % (u32)GS, ds = c % (u32)DS;
             UM_T(t0);
-            if (((e >> 8) & 0xFu) == 0) UM_WAIT(full_w0 + ws * 8, (wi / (u32)WS) & 1u);     // first chunk of an offset: its weights
+            if (((e >> 8) & 0xFu) == 0) mbar_wait_hint(full_w0 + ws * 8, (wi / (u32)WS) & 1u);     // first chunk of an offset: its weights
             UM_T(t1);
-            UM_WAIT(full_g0 + gs * 8, (c / (u32)GS) & 1u);
+            mbar_wait_hint(full_g0 + gs * 8, (c / (u32)GS) & 1u);
             UM_T(t2);
-            if (c >= (u32)DS) UM_WAIT(empty_d0 + ds * 8, ((c / (u32)DS) & 1u) ^ 1u);
+            if (c >= (u32)DS) mbar_wait_hint(empty_d0 + ds * 8, ((c / (u32)DS) & 1u) ^ 1u);
             UM_T(t3);
-            if (UM_GATHER_TMA != 1) fence_async_smem();          // rows written by cp.async (generic proxy) -> visible to the tensor core
             tmem_fence_after();
             if (elect_one()) {
                 const u32 idesc = IDESC | ((len >> 3) << 17);
@@ -269,7 +240,7 @@ spconv_um_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant
                     asm volatile("cp.async.bulk.tensor.2d.shared::cta.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
                                  ::"r"(slot), "l"(reinterpret_cast<u64>(&tmap)), "r"(bar), "r"(0), "r"((int)(t * TM + j * NMAX)) : "memory");
                 }
-            } else if (UM_GATHER_TMA == 1 || (UM_GATHER_TMA == 2 && (c % UM_MIX_DEN) < UM_MIX_TMA)) {
+            } else {
                 // TMA tile::gather4: four arbitrary rows per instruction, written with the 128 B swizzle; padding entries (row -1) are
                 // out of bounds = zero fill.  Issued by ONE elected lane inside warp-uniform control flow (per-lane issue makes ptxas
                 // emit an election loop with six R2UR.BROADCAST per instruction: ~50-100 clk each, profiles/r02_conv_um.md).
@@ -281,21 +252,6 @@ spconv_um_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant
                     if (elect_one())
                         asm volatile("cp.async.bulk.tensor.2d.shared::cta.global.tile::gather4.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
                                      ::"r"(slot + q * 512u), "l"(reinterpret_cast<u64>(&tmap_g)), "r"(bar), "r"(0), "r"((int)ix.x), "r"((int)ix.y), "r"((int)ix.z), "r"((int)ix.w) : "memory");
-                }
-            } else {
-                // cp.async: one instruction = four rows (eight lanes x 16 B each); 16-byte piece j of row r goes to piece j ^ (r & 7)
-                // (the 128 B swizzle the B descriptor expects).  Padding rows are not copied: their D columns go to the dummy row.
-                // One L1 wavefront per row; completion is the asynchronous mbarrier arrival below.
-                const u32 rl = (u32)lane >> 3, j8 = (u32)lane & 7u;
-                const unsigned char *xl = xs + j8 * 16;
-                const u32 d_even = slot + rl * 128u + ((j8 ^ rl) << 4), d_odd = slot + 512u + rl * 128u + ((j8 ^ (4u + rl)) << 4);
-                const u32 *ring = &s.idx[p][m & 3u][rl];
-#pragma unroll
-                for (int q = 0; q < NQ; ++q) {
-                    if (4u * q < len) {
-                        const u32 nb = ring[4 * q];
-                        if (nb != 0xFFFFFFFFu) cp_async16(((q & 1) ? d_odd : d_even) + (u32)(q >> 1) * 1024u, xl + (size_t)nb * 128);
-                    }
                 }
             }
             __syncwarp();
@@ -345,7 +301,7 @@ spconv_um_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant
         auto load = [&](u32 c, u32 (&d)[CPW], u32 (&ra)[CPW], bool &on) {
             const u32 ds = c % (u32)DS;
             on = e * CPW < ((s.tab[c] >> 12) & 0xFFu);           // len is a multiple of 16: my columns are inside or outside
-            UM_WAIT(full_d0 + ds * 8, (c / (u32)DS) & 1u);
+            mbar_wait_hint(full_d0 + ds * 8, (c / (u32)DS) & 1u);
             tmem_fence_after();
             if (on) {
                 if (CPW == 16) tmem_ld16(td + ds * NMAX, *reinterpret_cast<u32(*)[16]>(&d[0]));
@@ -501,7 +457,7 @@ static int launch_spconv_um(const CUtensorMap &tmap, const CUtensorMap &tmap_g, 
 }
 
 // xs = split rows [n][128 B]; Wp = this conv's slice of gpc_spconv_pack_weights_um; seg / pair_nbr = the pair stream built with
-// tile_rows (512 or 1024) and pad = 16 (padding entries 0xFFFFFFFF), pair_off (gpc_kmap_um_count / _fill).  Output rows
+// tile_rows = 512 and pad = 16 (padding entries 0xFFFFFFFF), pair_off (gpc_kmap_um_count / _fill).  Output rows
 // [row0, row1) (whole tiles; row1 <= 0 or >= n: to the end).  y (fp32 rows) and / or ys (split rows).
 extern "C" int gpc_spconv_fwd_um(const void *xs, const void *Wp, const uint32_t *seg, const uint32_t *pair_nbr,
                                  const uint32_t *pair_off, int64_t n, int tile_rows, const uint32_t *tile_order, const void *residual,
@@ -511,7 +467,7 @@ extern "C" int gpc_spconv_fwd_um(const void *xs, const void *Wp, const uint32_t 
     if (n <= 0) return GPC_OK;
     GPC_REQUIRE(y || ys, GPC_EINVAL, "no output requested");
     GPC_REQUIRE(xs != ys && xs != (const void *)y, GPC_EINVAL, "conv is out of place (rows are gathered from xs while y is written)");
-    GPC_REQUIRE(tile_rows == 256 || tile_rows == 384 || tile_rows == 512 || tile_rows == 1024, GPC_EINVAL, "tile_rows must be 256, 384, 512 or 1024");
+    GPC_REQUIRE(tile_rows == 512, GPC_EINVAL, "tile_rows must be 512");
     if (row1 <= 0 || row1 > n) row1 = n;
     GPC_REQUIRE(row0 >= 0 && row0 % tile_rows == 0 && (row1 % tile_rows == 0 || row1 == n), GPC_EINVAL, "row range must cover whole tiles");
     if (row0 >= row1) return GPC_OK;
@@ -520,7 +476,7 @@ extern "C" int gpc_spconv_fwd_um(const void *xs, const void *Wp, const uint32_t 
     CUtensorMap tmap;                                            // [n rows][64 bf16], box = one chunk of consecutive rows (the centre offset)
     const cuuint64_t gdim[2] = {64, (cuuint64_t)n};
     const cuuint64_t gstride[1] = {128};
-    const cuuint32_t box[2] = {64, (cuuint32_t)(tile_rows == 1024 ? 128 : (tile_rows == 512 ? UM512_NMAX : 64))};
+    const cuuint32_t box[2] = {64, 64};                          // 64 rows: NMAX of the launch below
     const cuuint32_t estr[2] = {1, 1};
     const CUresult rc = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(xs), gdim, gstride, box, estr,
                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
@@ -535,20 +491,8 @@ extern "C" int gpc_spconv_fwd_um(const void *xs, const void *Wp, const uint32_t 
     cudaStream_t st = as_stream(stream);
     const i64 tile0 = row0 / tile_rows, tiles = (row1 - row0 + tile_rows - 1) / tile_rows;
     const u32 *order = (row0 == 0 && row1 == n) ? tile_order : nullptr;            // a permutation of the level's tiles: full launches only
-    if (tile_rows == 256) {
-        if (prof) return launch_spconv_um<256, 64, 8, 3, 2, 3, 8, 256, 2, true>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
-        return launch_spconv_um<256, 64, 8, 3, 2, 3, 8, 256, 2>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
-    }
-    if (tile_rows == 384) {
-        if (prof) return launch_spconv_um<384, 64, 6, 3, 2, 3, 8, 256, 2, true>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
-        return launch_spconv_um<384, 64, 6, 3, 2, 3, 8, 256, 2>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
-    }
-    if (tile_rows == 512) {
-        if (prof) return launch_spconv_um<512, UM512_NMAX, UM512_GS, UM512_DS, 2, UM512_NPW, UM512_NEW, 256, 2, true>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
-        return launch_spconv_um<512, UM512_NMAX, UM512_GS, UM512_DS, 2, UM512_NPW, UM512_NEW, 256, 2>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
-    }
-    if (prof) return launch_spconv_um<1024, 128, 4, 3, 4, 4, 8, 512, 1, true>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
-    return launch_spconv_um<1024, 128, 4, 3, 4, 4, 8, 512, 1>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
+    if (prof) return launch_spconv_um<512, 64, 4, 3, 2, 3, 8, 256, 2, true>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
+    return launch_spconv_um<512, 64, 4, 3, 2, 3, 8, 256, 2>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
 }
 
 // W [n_kernels*125][32 ci][32 co] fp32 -> Wp [n_kernels*125][8 chunks][32 co][4 words]: channel co's TMEM lane is 32 words = 8 chunks of

@@ -3,22 +3,6 @@
 #pragma once
 #include "common.cuh"
 
-// ---- shared-memory matrix descriptor: K-major, SWIZZLE_NONE.  Element (row r, col c) of a [rows x 32] bf16 tile lives at
-//   (r / 8) * 512 + (c / 8) * 128 + (r % 8) * 16 + (c % 8) * 2     (8 x 16-byte core matrices; LBO = 128 B, SBO = 512 B)
-__host__ __device__ __forceinline__ u32 umma_tile_off(int r, int c) {
-    return (u32)((r >> 3) * 512 + (c >> 3) * 128 + (r & 7) * 16 + (c & 7) * 2);
-}
-__device__ __forceinline__ u64 umma_smem_desc(u32 smem_addr) {
-    return (u64)((smem_addr >> 4) & 0x3FFFu) | ((u64)(128u >> 4) << 16) | ((u64)(512u >> 4) << 32) | (1ull << 46);
-}
-// instruction descriptor, kind::f16: D = f32, A = B = bf16, both K-major, dense, M = 128, N = 32
-constexpr u32 UMMA_IDESC_BF16_M128_N32 = (1u << 4) | (1u << 7) | (1u << 10) | ((32u >> 3) << 17) | ((128u >> 4) << 24);
-
-// D[tmem] (+)= A[tmem] . B[smem]^T   (A: 128 lanes x 8 columns of packed bf16 pairs = K 16; B: N x K 16 from the descriptor)
-__device__ __forceinline__ void umma_bf16_ts(u32 tmem_d, u32 tmem_a, u64 bdesc, u32 idesc, u32 accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}\n"
-                 ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
 // all tcgen05.mma issued so far by this thread -> one arrival on the mbarrier when they have completed
 __device__ __forceinline__ void umma_commit(u32 bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
@@ -34,12 +18,6 @@ __device__ __forceinline__ bool elect_one() {
 __device__ __forceinline__ void tmem_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tmem_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// this thread's TMEM lane, 16 consecutive 32-bit columns
-__device__ __forceinline__ void tmem_st16(u32 taddr, const uint4 &a, const uint4 &b, const uint4 &c, const uint4 &d) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
-                 ::"r"(taddr), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w),
-                   "r"(c.x), "r"(c.y), "r"(c.z), "r"(c.w), "r"(d.x), "r"(d.y), "r"(d.z), "r"(d.w) : "memory");
-}
 __device__ __forceinline__ void tmem_ld16(u32 taddr, u32 (&d)[16]) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
                  : "=r"(d[0]), "=r"(d[1]), "=r"(d[2]), "=r"(d[3]), "=r"(d[4]), "=r"(d[5]), "=r"(d[6]), "=r"(d[7]), "=r"(d[8]),
@@ -53,30 +31,14 @@ __device__ __forceinline__ void tmem_ld8(u32 taddr, u32 (&d)[8]) {
 }
 
 // ---- mbarrier
-#ifndef TC_POLL_SLEEP_NS
-#define TC_POLL_SLEEP_NS 0
-#endif
 __device__ __forceinline__ void mbar_init(u32 bar, u32 count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
 }
 __device__ __forceinline__ void mbar_arrive(u32 bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
-// Bounded: a mis-programmed pipeline must fault the launch (trap), never hang the GPU.  (An explicit suspend-time hint on
-// try_wait was measured and did not help: the default already parks the warp.)
-__device__ __forceinline__ void mbar_wait(u32 bar, u32 parity) {
-#pragma unroll 1
-    for (u32 spins = 0; spins < (1u << 24); ++spins) {
-        u32 done;
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (done) return;
-        if (TC_POLL_SLEEP_NS) __nanosleep(TC_POLL_SLEEP_NS);
-    }
-    __trap();
-}
-
-// try_wait with an explicit suspend-time hint: the warp sleeps in hardware until the phase completes or the hint (ns) runs out
+// try_wait with an explicit suspend-time hint: the warp sleeps in hardware until the phase completes or the hint (ns) runs out.
+// Bounded: a mis-programmed pipeline must fault the launch (trap), never hang the GPU.
 __device__ __forceinline__ void mbar_wait_hint(u32 bar, u32 parity) {
 #pragma unroll 1
     for (u32 spins = 0; spins < (1u << 20); ++spins) {
@@ -87,39 +49,11 @@ __device__ __forceinline__ void mbar_wait_hint(u32 bar, u32 parity) {
     }
     __trap();
 }
-// pure polling (mbarrier.test_wait never suspends the warp): for the roles on the critical path of a short hand-off
-__device__ __forceinline__ void mbar_wait_spin(u32 bar, u32 parity) {
-#pragma unroll 1
-    for (u32 spins = 0; spins < (1u << 26); ++spins) {
-        u32 done;
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (done) return;
-    }
-    __trap();
-}
-// the same with a back-off between polls: for roles that wait long (a spinning warp's polls share the memory-instruction queue of its
-// scheduler with the loads and stores of the warps that do the work)
-template <int NS> __device__ __forceinline__ void mbar_wait_backoff(u32 bar, u32 parity) {
-#pragma unroll 1
-    for (u32 spins = 0; spins < (1u << 24); ++spins) {
-        u32 done;
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (done) return;
-        __nanosleep(NS);
-    }
-    __trap();
-}
 
 // ---- cp.async (no "memory" clobber: ordering against commit / wait / barrier statements is kept by their volatile-ness, and a
 // clobber here would chain every table load in front of a copy behind the previous copy)
 __device__ __forceinline__ void cp_async16(u32 dst, const void *src) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src));
 }
-__device__ __forceinline__ void cp_async8(u32 dst, const void *src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(dst), "l"(src));
-}
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }

@@ -118,7 +118,7 @@ int gpc_hash_lookup(const void *table, int64_t capacity, const uint64_t *query, 
  * pass of gpc_kmap_um_scan and the level's density (true pairs per row) without a second read of the map. */
 int gpc_kmap_dense(const void *table, int64_t capacity, const uint64_t *keys, int64_t n,
                    int32_t *map, int kernel_size, int tile_rows, uint32_t *cell_counts, void *stream);
-/* tile pair lists for the conv: tiles of `tile_rows` consecutive output rows; for tile t and offset
+/* tile pair lists for the mma.sync conv: tiles of `tile_rows` (8, 16, 32, 64 or 128) consecutive output rows; for tile t and offset
  * k the pairs are [seg[t*126+k], seg[t*126+k+1]) (seg[t*126+125] == next tile's start);
  * pair_nbr = input row, pair_row = output row - t*tile_rows.  Two calls: count (fills seg as an
  * exclusive scan, *n_pairs device u32), then fill. */
@@ -129,7 +129,7 @@ size_t gpc_kmap_pairs_workspace_bytes(int64_t n, int tile_rows);
 int gpc_kmap_pairs_count(const int32_t *map, int64_t n, int tile_rows, int pad, uint32_t *seg, uint32_t *n_pairs,
                          void *ws, size_t ws_bytes, void *stream);
 /* fill writes the split arrays (pair_nbr/pair_row, may be NULL) and/or the combined stream
- * pairs[p] = nbr | row_in_tile << 32 | k << 48 (may be NULL) consumed by gpc_spconv_fwd_v3 */
+ * pairs[p] = nbr | row_in_tile << 32 | k << 48 (may be NULL) consumed by gpc_spconv_fwd_v6 */
 int gpc_kmap_pairs_fill(const int32_t *map, int64_t n, int tile_rows, const uint32_t *seg,
                         uint32_t *pair_nbr, uint16_t *pair_row, uint64_t *pairs, int64_t n_entries, void *stream);
 
@@ -142,8 +142,8 @@ int gpc_spconv_pack_weights_frag(const float *W, int n_kernels, void *Wa, void *
 
 /* the mma.sync conv (spconv.cu): one warp per tile of tile_rows output rows over the combined pair stream padded to 8-entry MMA tiles
  * (pad = 8), W^T[k] as the MMA A operand, the gathered rows as the B operand (bf16 hi / lo split, three terms, fp32 accumulation).
- * variant 42: cp.async gather ring; 45 / 46 / 47: the offsets of a tile split over 2 / 8 / 16 warps (coarse levels); 48: rows loaded
- * straight into the MMA fragments (v6d, big levels) */
+ * variant 42 (tile_rows 64): cp.async gather ring; 46 (16, 32) / 47 (8): the offsets of a tile split over 8 / 16 warps (coarse
+ * levels); 48 (32, 64, 128): rows loaded straight into the MMA fragments (v6d, big levels).  Other pairs: GPC_EINVAL. */
 int gpc_spconv_fwd_v6(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs,
                       int64_t n, int tile_rows, const float *residual, int flags, float *y, int variant,
                       void *stream);
@@ -184,12 +184,12 @@ int gpc_rows_join(const void *xs, int64_t n, float *x, void *stream);
 
 /* ---- the tcgen05 sparse conv of the big levels (spconv_um.cu) ----
  * y[o,:] = act( sum_k W[k]^T xs[nbr_k(o),:] (+ residual[o,:]) ).  Transposed formulation: per (tile of tile_rows output rows, offset k)
- * the pairs are the N dimension of tcgen05.mma (chunks of 16..64/128 pairs), W[k]^T (bf16 hi | lo) is the A operand in tensor
- * memory, the gathered rows (cp.async into 128 B-swizzled tiles; TMA tile loads for the centre offset) are the B operand in shared
+ * the pairs are the N dimension of tcgen05.mma (chunks of 16..64 pairs), W[k]^T (bf16 hi | lo) is the A operand in tensor
+ * memory, the gathered rows (TMA tile::gather4 into 128 B-swizzled tiles; TMA tile loads for the centre offset) are the B operand in shared
  * memory, D in tensor memory; the epilogue adds every pair to its output row's fp32 sum in shared memory, offsets ascending (one
  * fixed summation order per row).
  * xs = split rows; Wp = this conv's slice of gpc_spconv_pack_weights_um ([125][32 co][128 B]); seg / pair_nbr = the pair stream
- * and accumulator-row offsets built by gpc_kmap_um_count / _fill with tile_rows = 256, 384, 512 or 1024.  Outputs y (fp32
+ * and accumulator-row offsets built by gpc_kmap_um_count / _fill with tile_rows = 512 (the only tile height).  Outputs y (fp32
  * rows) and / or ys (split rows).  Only the output rows [row0, row1) are computed (whole tiles; row1 <= 0 or >= n: to the end):
  * the decoder wavefront.  flags: GPC_CONV_RELU, GPC_CONV_RES_SPLIT, GPC_CONV_PROFILE. */
 #define GPC_CONV_PROFILE 256   /* flags bit: run the instrumented build (per-role cycle counters, gpc_debug_conv_um_profile) */

@@ -331,53 +331,50 @@ def env_umma(env):
     return dict(env, codec=codec)
 
 
-@pytest.mark.parametrize("n,ext,tile", [(30000, 16, 512), (30000, 16, 384), (30000, 16, 256), (30000, 16, 1024), (2000, 6, 512),
-                                        (1025, 5, 1024), (513, 5, 512), (77, 4, 512)])
+@pytest.mark.parametrize("n,ext,tile", [(30000, 16, 512), (2000, 6, 512), (513, 5, 512), (77, 4, 512), (12000, 5, 512),
+                                        (1025, 5, 512), (1024, 5, 512), (512, 5, 512)])
 def test_sparse_conv_tcgen05(env_umma, n, ext, tile):
     """tcgen05 / TMEM conv over split rows against the fp32 oracle conv: fp32 and split outputs, residual in both formats, row-range
-    launches (decoder wavefront) bit-identical to the whole launch, ragged last tile."""
+    launches (decoder wavefront) bit-identical to the whole launch, ragged last tile (down to one row), levels of exactly one and
+    two tiles, and a dense level (~40 pairs per row) whose (tile, offset) cells take several 64-pair chunks."""
     from gauspcc_b200.codec import _ptr
     from gauspcc_b200.synth import hac_like_cloud, uniform_unique_cloud
     from oracle import oracle as O
     codec, w = env_umma["codec"], env_umma["w"]
-    codec.um_tile_rows = tile
-    try:
-        xyz = uniform_unique_cloud(n, 5, extent_log2=ext) if ext < 10 else hac_like_cloud(n, 5, extent_log2=ext)
-        xyz = xyz[O.sort_zyx_perm(xyz)]
-        keys, _ = _keys_of(codec, xyz)
-        km = codec.build_kmap(keys)
-        assert km.um_rows == tile and km.tile_rows == tile
-        ref_km = O.kmap(xyz, 5)
-        assert km.n_real == int((ref_km >= 0).sum())
-        rng = np.random.default_rng(0)
-        x = rng.normal(size=(n, 32)).astype(np.float32)
-        res = rng.normal(size=(n, 32)).astype(np.float32)
-        xd, rd = torch.tensor(x, device=codec.dev), torch.tensor(res, device=codec.dev)
-        ref = O.conv(x, w["target_resnet.2.conv1.kernel"], ref_km)
-        scale = max(np.abs(ref).max(), 1.0)
-        y = codec.conv(xd, 7, km).cpu().numpy()
-        assert np.abs(y - ref).max() <= 3e-5 * scale
-        # split-row input / output / residual: same numbers up to the 2^-17 relative rounding of a split row
-        xs, rs = codec.split_rows(xd), codec.split_rows(rd)
-        y2f, y2s = codec.conv(xs, 7, km, residual=rs, relu=True, fmt="both")
-        y2 = y2f.cpu().numpy()
-        assert np.abs(y2 - np.maximum(ref + res, 0)).max() <= 6e-5 * scale
-        joined = torch.empty_like(y2f)
-        codec._call("gpc_rows_join", _ptr(y2s), n, _ptr(joined), codec._stream())
-        assert np.abs(joined.cpu().numpy() - y2).max() <= 2e-5 * scale
-        y3 = codec.conv(xs, 7, km, residual=rd, relu=True).cpu().numpy()          # fp32 residual
-        assert np.abs(y3 - y2).max() <= 3e-5 * scale
-        # deterministic: bit-identical on a second launch (encoder / decoder CDF identity depends on it)
-        assert np.array_equal(codec.conv(xd, 7, km).cpu().numpy(), y)
-        # row ranges (whole tiles): the same sums bit for bit
-        if n > tile:
-            cut = (n // 2) // tile * tile or tile
-            yr = torch.full((n, 32), float("nan"), device=codec.dev)
-            codec.conv(xs, 7, km, out=yr, rows=(0, cut))
-            codec.conv(xs, 7, km, out=yr, rows=(cut, n))
-            assert np.array_equal(yr.cpu().numpy(), y)
-    finally:
-        codec.um_tile_rows = 512
+    xyz = uniform_unique_cloud(n, 5, extent_log2=ext) if ext < 10 else hac_like_cloud(n, 5, extent_log2=ext)
+    xyz = xyz[O.sort_zyx_perm(xyz)]
+    keys, _ = _keys_of(codec, xyz)
+    km = codec.build_kmap(keys)
+    assert km.um_rows == tile and km.tile_rows == tile
+    ref_km = O.kmap(xyz, 5)
+    assert km.n_real == int((ref_km >= 0).sum())
+    rng = np.random.default_rng(0)
+    x = rng.normal(size=(n, 32)).astype(np.float32)
+    res = rng.normal(size=(n, 32)).astype(np.float32)
+    xd, rd = torch.tensor(x, device=codec.dev), torch.tensor(res, device=codec.dev)
+    ref = O.conv(x, w["target_resnet.2.conv1.kernel"], ref_km)
+    scale = max(np.abs(ref).max(), 1.0)
+    y = codec.conv(xd, 7, km).cpu().numpy()
+    assert np.abs(y - ref).max() <= 3e-5 * scale
+    # split-row input / output / residual: same numbers up to the 2^-17 relative rounding of a split row
+    xs, rs = codec.split_rows(xd), codec.split_rows(rd)
+    y2f, y2s = codec.conv(xs, 7, km, residual=rs, relu=True, fmt="both")
+    y2 = y2f.cpu().numpy()
+    assert np.abs(y2 - np.maximum(ref + res, 0)).max() <= 6e-5 * scale
+    joined = torch.empty_like(y2f)
+    codec._call("gpc_rows_join", _ptr(y2s), n, _ptr(joined), codec._stream())
+    assert np.abs(joined.cpu().numpy() - y2).max() <= 2e-5 * scale
+    y3 = codec.conv(xs, 7, km, residual=rd, relu=True).cpu().numpy()          # fp32 residual
+    assert np.abs(y3 - y2).max() <= 3e-5 * scale
+    # deterministic: bit-identical on a second launch (encoder / decoder CDF identity depends on it)
+    assert np.array_equal(codec.conv(xd, 7, km).cpu().numpy(), y)
+    # row ranges (whole tiles): the same sums bit for bit
+    if n > tile:
+        cut = (n // 2) // tile * tile or tile
+        yr = torch.full((n, 32), float("nan"), device=codec.dev)
+        codec.conv(xs, 7, km, out=yr, rows=(0, cut))
+        codec.conv(xs, 7, km, out=yr, rows=(cut, n))
+        assert np.array_equal(yr.cpu().numpy(), y)
 
 
 @pytest.mark.parametrize("n,seed,ext", [(20000, 1, 16), (2500, 5, 12)])
@@ -728,12 +725,13 @@ def test_cli_file_roundtrip(env, tmp_path):
         assert drows[0]["num_points"] > 0 and np.array_equal(back, q)
 
 
-@pytest.mark.parametrize("plane", [True, False])
+@pytest.mark.parametrize("scenes", [((120_000, 3), (30_000, 4)), ((30_000, 4), (120_000, 3))], ids=["shrinking", "growing"])
 @pytest.mark.parametrize("kind", ["um", "v6d", "sparse"])
-def test_decoder_wavefront(env, env_v6d, env_sparse, env_umma, kind, plane):
+def test_decoder_wavefront(env, env_v6d, env_sparse, env_umma, kind, scenes):
     """The decoder's stage wavefront (chunks of rows, four range-decoder threads) against the stage-by-stage decode of the same
-    streams: identical geometry row for row; levels of every chunk count (ragged last chunk, levels that fail the halo check or are
-    too small fall back).  All three conv families of the big levels."""
+    streams: identical geometry row for row; levels of every chunk count (ragged last chunk, levels too small for two chunks fall
+    back).  All three conv families of the big levels.  Two scenes on one codec, in both orders: the buffers the codec keeps
+    across calls (wavefront feature arrays, pinned staging) are reused by a smaller scene and grown for a bigger one."""
     from gauspcc_b200.codec import GausPcgcCodec
     from gauspcc_b200.synth import hac_like_cloud
     src = {"v6d": env_v6d, "sparse": env_sparse, "um": env_umma}[kind]["codec"]
@@ -741,10 +739,9 @@ def test_decoder_wavefront(env, env_v6d, env_sparse, env_umma, kind, plane):
     codec.v6_variant, codec.um_min_rows = src.v6_variant, src.um_min_rows
     codec.sparse_min_rows, codec.sparse_max_density = src.sparse_min_rows, src.sparse_max_density
     codec.wave_min_rows, codec.wave_chunk_rows = 1, 8192
-    codec.wave_plane_lag = plane                       # stage i+1 trails stage i by planes (default) / by two chunks
-    if kind == "sparse":                               # small leading chunks, then bigger ones
-        codec.wave_chunk_rows, codec.wave_first_rows, codec.wave_first_chunks = 16384, 8192, 2
-    for n, seed in ((120_000, 3), (30_000, 4)):
+    if kind == "sparse":
+        codec.wave_chunk_rows = 16384
+    for n, seed in scenes:
         x = torch.tensor(hac_like_cloud(n, seed), dtype=torch.float32, device=codec.dev)
         bx, bo, streams, _ = codec.encode(x)
         codec.wave_decode = True

@@ -1,5 +1,5 @@
 """Bring-up check + timing of the TMA / tcgen05 conv (spconv_um.cu) against a torch fp64 reference built from the dense kernel map and
-against the mma.sync conv (v6d) on the levels of a synthetic scene.  Run on the GPU box:  python tools/um_check.py [npts] [tile_rows]"""
+against the mma.sync conv (v6d) on the levels of a synthetic scene.  Run on the GPU box:  python tools/um_check.py [npts]"""
 import ctypes as C
 import os
 import sys
@@ -9,14 +9,13 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from gauspcc_b200 import _lib
-from gauspcc_b200.codec import DeviceWeights, GausPcgcCodec, _ptr
+from gauspcc_b200.codec import UM_TILE_ROWS, DeviceWeights, GausPcgcCodec, _ptr
 from gauspcc_b200.synth import hac_like_cloud
 from gauspcc_b200.weights import make_synthetic_state_dict
 
 
 def main():
     npts = int(sys.argv[1]) if len(sys.argv) > 1 else 200_000
-    tiles = [int(v) for v in (sys.argv[2].split(",") if len(sys.argv) > 2 else ["512", "1024"])]
     min_rows = int(os.environ.get("UM_MIN_ROWS", 3000))
     dev = torch.device("cuda:0")
     w = DeviceWeights(make_synthetic_state_dict(), dev)
@@ -65,51 +64,50 @@ def main():
         e1.record(); torch.cuda.synchronize()
         ms6 = e0.elapsed_time(e1) / reps
         err6 = float((y6.double() - torch.relu((ref - xj.double().new_zeros(1)) + res.double())).abs().max())
-        for tr in tiles:
-            tmag, gflag = 0, 0
-            km = codec._um_map(dense, n, tr)
-            poff = km.pair_off
-            y = torch.full((n, 32), float("nan"), device=dev)
-            ys = torch.zeros((n, 32), dtype=torch.int32, device=dev)
-            order = km.tile_order if os.environ.get("UM_ORDER", "1") != "0" else None
-            args = (_ptr(xs), _ptr(wp[widx]), _ptr(km.seg), _ptr(km.pair_nbr), _ptr(poff), n, tr, _ptr(order), _ptr(res), 1 | gflag, _ptr(y), _ptr(ys), 0, 0, st)
-            rc = lib.gpc_spconv_fwd_um(*args)
-            _lib.check(rc, "um")
-            torch.cuda.synchronize()
-            err = float((y.double() - ref_relu).abs().max())
-            yj = torch.empty_like(y)
-            codec._call("gpc_rows_join", _ptr(ys), n, _ptr(yj), codec._stream())
-            err_s = float((yj - y).abs().max())
-            scale = float(ref_relu.abs().max())
-            # determinism + row-range launches
-            y2 = torch.empty_like(y)
-            args2 = list(args); args2[10] = _ptr(y2); args2[11] = None
-            half = (n // 2) // tr * tr
-            a = list(args2); a[12], a[13] = 0, half
-            _lib.check(lib.gpc_spconv_fwd_um(*a), "um rows a")
-            a = list(args2); a[12], a[13] = half, 0
-            _lib.check(lib.gpc_spconv_fwd_um(*a), "um rows b")
-            torch.cuda.synchronize()
-            same = bool(torch.equal(y2, y))
-            e0.record()
-            for _ in range(reps):
-                lib.gpc_spconv_fwd_um(*args2)
-            e1.record(); torch.cuda.synchronize()
-            ms = e0.elapsed_time(e1) / reps
-            clk = ms * 1e-3 * 1.9e9 * 148 / max(n_pairs_real, 1)
-            if os.environ.get("UM_PROF", "1") != "0":
-                lib.gpc_debug_conv_um_profile(None, 1)
-                a = list(args2); a[9] = 1 | 256 | gflag
-                _lib.check(lib.gpc_spconv_fwd_um(*a), "um prof")
-                buf = (C.c_uint64 * 16)()
-                lib.gpc_debug_conv_um_profile(C.cast(buf, C.c_void_p), 1)
-                ch, ctas = max(buf[11], 1), max(buf[15], 1)
-                names = ["e.items", "p.empty_g", "p.issue", "m.full_w", "m.full_g", "m.empty_d", "m.issue", "e.loop", "e.full_d", "e.ldtm_issue", "e.rmw"]
-                print(f"   prof tile={tr} tma={tmag}: chunks/cta={ch / ctas:.0f} " + " ".join(f"{nm}={buf[i] / ch:.0f}" for i, nm in enumerate(names))
-                      + f" | per cta: total={buf[12] / ctas:.0f} setup={buf[13] / ctas:.0f} writeout={buf[14] / ctas:.0f}", flush=True)
-            print(f"n={n:8d} p/r={n_pairs_real / n:5.1f} tile={tr:4d} tma={tmag} entries/pairs={km.n_pairs / max(n_pairs_real, 1):.2f} "
-                  f"um {ms:.3f} ms ({clk:.1f} clk/pair)  v6d {ms6:.3f} ms  err={err:.2e} (v6d {err6:.2e}, scale {scale:.1f}) "
-                  f"split-out err={err_s:.2e} rows-identical={same}", flush=True)
+        tr = UM_TILE_ROWS
+        km = codec._um_map(dense, n, tr)
+        poff = km.pair_off
+        y = torch.full((n, 32), float("nan"), device=dev)
+        ys = torch.zeros((n, 32), dtype=torch.int32, device=dev)
+        order = km.tile_order if os.environ.get("UM_ORDER", "1") != "0" else None
+        args = (_ptr(xs), _ptr(wp[widx]), _ptr(km.seg), _ptr(km.pair_nbr), _ptr(poff), n, tr, _ptr(order), _ptr(res), 1, _ptr(y), _ptr(ys), 0, 0, st)
+        rc = lib.gpc_spconv_fwd_um(*args)
+        _lib.check(rc, "um")
+        torch.cuda.synchronize()
+        err = float((y.double() - ref_relu).abs().max())
+        yj = torch.empty_like(y)
+        codec._call("gpc_rows_join", _ptr(ys), n, _ptr(yj), codec._stream())
+        err_s = float((yj - y).abs().max())
+        scale = float(ref_relu.abs().max())
+        # determinism + row-range launches
+        y2 = torch.empty_like(y)
+        args2 = list(args); args2[10] = _ptr(y2); args2[11] = None
+        half = (n // 2) // tr * tr
+        a = list(args2); a[12], a[13] = 0, half
+        _lib.check(lib.gpc_spconv_fwd_um(*a), "um rows a")
+        a = list(args2); a[12], a[13] = half, 0
+        _lib.check(lib.gpc_spconv_fwd_um(*a), "um rows b")
+        torch.cuda.synchronize()
+        same = bool(torch.equal(y2, y))
+        e0.record()
+        for _ in range(reps):
+            lib.gpc_spconv_fwd_um(*args2)
+        e1.record(); torch.cuda.synchronize()
+        ms = e0.elapsed_time(e1) / reps
+        clk = ms * 1e-3 * 1.9e9 * 148 / max(n_pairs_real, 1)
+        if os.environ.get("UM_PROF", "1") != "0":
+            lib.gpc_debug_conv_um_profile(None, 1)
+            a = list(args2); a[9] = 1 | 256
+            _lib.check(lib.gpc_spconv_fwd_um(*a), "um prof")
+            buf = (C.c_uint64 * 16)()
+            lib.gpc_debug_conv_um_profile(C.cast(buf, C.c_void_p), 1)
+            ch, ctas = max(buf[11], 1), max(buf[15], 1)
+            names = ["e.items", "p.empty_g", "p.issue", "m.full_w", "m.full_g", "m.empty_d", "m.issue", "e.loop", "e.full_d", "e.ldtm_issue", "e.rmw"]
+            print(f"   prof tile={tr}: chunks/cta={ch / ctas:.0f} " + " ".join(f"{nm}={buf[i] / ch:.0f}" for i, nm in enumerate(names))
+                  + f" | per cta: total={buf[12] / ctas:.0f} setup={buf[13] / ctas:.0f} writeout={buf[14] / ctas:.0f}", flush=True)
+        print(f"n={n:8d} p/r={n_pairs_real / n:5.1f} tile={tr:4d} entries/pairs={km.n_pairs / max(n_pairs_real, 1):.2f} "
+              f"um {ms:.3f} ms ({clk:.1f} clk/pair)  v6d {ms6:.3f} ms  err={err:.2e} (v6d {err6:.2e}, scale {scale:.1f}) "
+              f"split-out err={err_s:.2e} rows-identical={same}", flush=True)
 
 
 if __name__ == "__main__":
