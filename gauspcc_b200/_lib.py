@@ -88,6 +88,10 @@ SIGNATURES = {
     "gpc_attr_encode_gaussian": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "gpc_attr_merge_chunks": (c_int, [c_vp, c_i64, c_int, c_vp, c_vp, c_vp]),
     "gpc_attr_decode_table": (c_int, [c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_mixture_encode": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_mixture_decode": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_row_encode": (c_int, [c_vp, c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_row_decode": (c_int, [c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
     "gpc_chunk_workspace_bytes": (c_sz, [c_int, c_int]),
     "gpc_chunk_encode_lohi": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "gpc_chunk_merge": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_vp]),

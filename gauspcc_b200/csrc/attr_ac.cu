@@ -15,7 +15,10 @@
 //  * a chunk's coder is one WARP whose lanes all carry the coder state: the 32 lanes fetch 32 symbols' inputs with one
 //    coalesced load and hand them round with shuffles; in the decoder the 32 lanes evaluate 32 candidate symbols at once
 //    (window centred on the mean, else a 32-ary search), where the reference walks a binary search of dependent loads;
-//  * bits leave through a 64-bit register, four bytes per store; chunks are merged by one CTA per chunk after a device scan.
+//  * bits leave through a 64-bit register, four bytes per store; chunks are merged by one CTA per chunk after a device scan;
+//  * HAC++'s mixture of K <= 4 Gaussians (encodings_cuda.py:203-314 builds the table as clamp(sum_k cdf_k * prob_k, 0, 1)) goes
+//    through the same two kernels with MixModel, which restates that float sum operation for operation; the Bernoulli mask
+//    coder (:435-500, a table whose rows are all [0, 1 - p, 1]) reads its one shared row (SharedRowModel).
 //
 // Arithmetic restated exactly (float erfc, the double product for the bin edge, round-to-nearest-even to int, the `+ symbol`
 // that keeps the integer CDF strictly increasing); `tests/test_attr_coder.py` checks the bytes against the C oracle and, on the
@@ -45,11 +48,14 @@ __global__ void attr_cdf_table_kernel(const float *__restrict__ mean, const floa
     lower[t] = attr_gauss_cdf(attr_edge(min_value, i, Q[row]), mean[row], attr_clamp_scale(scale[row]));
 }
 
-// ---- the two models a symbol's integer CDF entries come from:  v(row, m) = rn(cdf(row, m) * (2^16 - (Lp - 1))) + m
+// ---- the models a symbol's integer CDF entries come from:  v(row, m) = rn(cdf(row, m) * (2^16 - (Lp - 1))) + m.
+// A model's Row is what one symbol needs; shfl() hands lane src's row to the warp (the decoder fetches 32 rows with one coalesced
+// load), and the centred models give centre(): the symbol the decoder's first window of 32 candidates is centred on.
 struct TableModel {
     const float *cdf; int Lp; float scale16;
     struct Row { i64 base; };
     __device__ __forceinline__ Row row(i64 r) const { return Row{r * Lp}; }
+    __device__ __forceinline__ Row shfl(const Row &rw, int src) const { return Row{__shfl_sync(0xFFFFFFFFu, rw.base, src)}; }
     __device__ __forceinline__ u32 v(const Row &rw, int m) const { return (u32)(__float2int_rn(cdf[rw.base + m] * scale16) + m); }
 };
 // integer CDF rows as the geometry codec's head kernel writes them (uint16 bit pattern of kit/op.py:67-79; the top of the last
@@ -60,12 +66,73 @@ struct U16Model {
     __device__ __forceinline__ Row row(i64 r) const { return Row{r * Lp}; }
     __device__ __forceinline__ u32 v(const Row &rw, int m) const { return (u32)cdf[rw.base + m]; }
 };
+// ONE float CDF row shared by every symbol: the Bernoulli mask coder (encodings_cuda.py:435-500), whose table is [0, 1 - p, 1]
+// on every row.  The same v() as TableModel on that row.
+struct SharedRowModel {
+    const float *cdf; float scale16;
+    struct Row {};
+    __device__ __forceinline__ Row row(i64) const { return Row{}; }
+    __device__ __forceinline__ Row shfl(const Row &rw, int) const { return rw; }
+    __device__ __forceinline__ u32 v(const Row &, int m) const { return (u32)(__float2int_rn(cdf[m] * scale16) + m); }
+};
 struct GaussModel {
     const float *mean, *scale, *Q; int min_value; float scale16;
     struct Row { float mean, scale, q; };
     __device__ __forceinline__ Row row(i64 r) const { return Row{mean[r], attr_clamp_scale(scale[r]), Q[r]}; }
+    __device__ __forceinline__ Row shfl(const Row &rw, int src) const {
+        return Row{__shfl_sync(0xFFFFFFFFu, rw.mean, src), __shfl_sync(0xFFFFFFFFu, rw.scale, src), __shfl_sync(0xFFFFFFFFu, rw.q, src)};
+    }
+    __device__ __forceinline__ int centre(const Row &rw) const { return __float2int_rn(rw.mean / rw.q) - min_value; }
     __device__ __forceinline__ u32 v(const Row &rw, int m) const {
         return (u32)(__float2int_rn(attr_gauss_cdf(attr_edge(min_value, m, rw.q), rw.mean, rw.scale) * scale16) + m);
+    }
+};
+// mixture of K Gaussians (HAC++'s encoder_gaussian_mixed, encodings_cuda.py:203-314): the table the reference builds is
+//   lower = clamp(sum_k calculate_cdf(mean_k, scale_k) * prob_k, 0, 1)
+// in float32, one rounding per product and per sum, in list order.  v() restates exactly that: __fmul_rn / __fadd_rn keep nvcc
+// from contracting acc + c * p into an FMA, and the clamp is written with comparisons so that a NaN passes through as it does
+// in torch.clamp.  mean / scale / prob are [K][n].
+template <int K>
+struct MixModel {
+    const float *mean, *scale, *prob, *Q; i64 n; int min_value; float scale16;
+    struct Row { float mean[K], scale[K], prob[K], q; };
+    __device__ __forceinline__ Row row(i64 r) const {
+        Row rw;
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            rw.mean[k] = mean[k * n + r];
+            rw.scale[k] = attr_clamp_scale(scale[k * n + r]);
+            rw.prob[k] = prob[k * n + r];
+        }
+        rw.q = Q[r];
+        return rw;
+    }
+    __device__ __forceinline__ Row shfl(const Row &rw, int src) const {
+        Row o;
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            o.mean[k] = __shfl_sync(0xFFFFFFFFu, rw.mean[k], src);
+            o.scale[k] = __shfl_sync(0xFFFFFFFFu, rw.scale[k], src);
+            o.prob[k] = __shfl_sync(0xFFFFFFFFu, rw.prob[k], src);
+        }
+        o.q = __shfl_sync(0xFFFFFFFFu, rw.q, src);
+        return o;
+    }
+    // the mean of the most probable component (ties: the first): where most of the row's mass is when the components are apart
+    __device__ __forceinline__ int centre(const Row &rw) const {
+        float best = rw.prob[0], c = rw.mean[0];
+#pragma unroll
+        for (int k = 1; k < K; ++k)
+            if (rw.prob[k] > best) { best = rw.prob[k]; c = rw.mean[k]; }
+        return __float2int_rn(c / rw.q) - min_value;
+    }
+    __device__ __forceinline__ u32 v(const Row &rw, int m) const {
+        const float edge = attr_edge(min_value, m, rw.q);
+        float acc = __fmul_rn(attr_gauss_cdf(edge, rw.mean[0], rw.scale[0]), rw.prob[0]);
+#pragma unroll
+        for (int k = 1; k < K; ++k) acc = __fadd_rn(acc, __fmul_rn(attr_gauss_cdf(edge, rw.mean[k], rw.scale[k]), rw.prob[k]));
+        acc = acc < 0.0f ? 0.0f : (acc > 1.0f ? 1.0f : acc);
+        return (u32)(__float2int_rn(acc * scale16) + m);
     }
 };
 
@@ -258,14 +325,7 @@ __global__ void __launch_bounds__(128) attr_decode_chunks_kernel(Model md, const
         typename Model::Row mine = md.row(base + j0 + min(lane, m - 1));            // one coalesced fetch for 32 symbols
         int my_sym = 0;
         for (int j = 0; j < m; ++j) {
-            typename Model::Row rw;
-            if constexpr (CENTRED) {
-                rw.mean = __shfl_sync(0xFFFFFFFFu, mine.mean, j);
-                rw.scale = __shfl_sync(0xFFFFFFFFu, mine.scale, j);
-                rw.q = __shfl_sync(0xFFFFFFFFu, mine.q, j);
-            } else {
-                rw.base = __shfl_sync(0xFFFFFFFFu, mine.base, j);
-            }
+            const typename Model::Row rw = md.shfl(mine, j);
             const u64 span = (u64)high - (u64)low + 1ull;
             // count = uint16(((value - low + 1) * 2^16 - 1) / span), :318-319 -- float estimate, exact correction
             const u64 X = (((u64)value - (u64)low + 1ull) << ATTR_PRECISION) - 1ull;
@@ -280,8 +340,8 @@ __global__ void __launch_bounds__(128) attr_decode_chunks_kernel(Model md, const
             u32 c_low = 0, c_high = 0;
             bool have = false;
             if constexpr (CENTRED) {
-                // window of 32 candidates around the mean: exact when the answer falls inside (the usual case)
-                const int centre = __float2int_rn(rw.mean / rw.q) - md.min_value;
+                // window of 32 candidates around the model's centre: exact when the answer falls inside (the usual case)
+                const int centre = md.centre(rw);
                 const int w0 = max(0, min(centre - 15, max_symbol - 31));
                 const int mm = w0 + lane;
                 const u32 vv = mm <= max_symbol + 1 ? md.v(rw, min(mm, max_symbol + 1)) : 0u;
@@ -454,6 +514,60 @@ extern "C" int gpc_attr_decode_gaussian(const float *mean, const float *scale, c
     if (rc) return rc;
     GaussModel md{mean, scale, Q, min_value, (float)((1 << ATTR_PRECISION) - (Lp - 1))};
     return attr_decode<GaussModel, true, int16_t>(md, in, cnt, n, Lp, chunk_size, sym, ws, ws_bytes, as_stream(stream));
+}
+
+// ---- HAC++'s mixture coders and the Bernoulli mask coder without a per-symbol table: the same bytes as the table entry points fed
+// with the table the reference builds, through the same workspace and gpc_attr_merge_chunks
+// k = 1..4 components: calls run(MixModel<k>{...})
+template <typename Run>
+static int mixture_run(int k, const float *mean, const float *scale, const float *prob, const float *Q, i64 n, int min_value, int Lp,
+                       Run run) {
+    GPC_REQUIRE(k >= 1 && k <= 4, GPC_EINVAL, "mixture coder: 1 to 4 components are supported");
+    const float s16 = (float)((1 << ATTR_PRECISION) - (Lp - 1));
+    switch (k) {
+    case 1: return run(MixModel<1>{mean, scale, prob, Q, n, min_value, s16});
+    case 2: return run(MixModel<2>{mean, scale, prob, Q, n, min_value, s16});
+    case 3: return run(MixModel<3>{mean, scale, prob, Q, n, min_value, s16});
+    default: return run(MixModel<4>{mean, scale, prob, Q, n, min_value, s16});
+    }
+}
+
+extern "C" int gpc_mixture_encode(const int16_t *sym, const float *mean, const float *scale, const float *prob, const float *Q,
+                                  int64_t n, int k, int min_value, int max_value, int chunk_size, int32_t *cnt, uint32_t *offsets,
+                                  void *ws, size_t ws_bytes, void *stream) {
+    const int Lp = max_value - min_value + 2;
+    int rc = attr_check(n, Lp, chunk_size);
+    if (rc) return rc;
+    return mixture_run(k, mean, scale, prob, Q, n, min_value, Lp, [&](auto md) {
+        return attr_encode(md, sym, n, Lp, chunk_size, cnt, offsets, ws, ws_bytes, as_stream(stream));
+    });
+}
+
+extern "C" int gpc_mixture_decode(const float *mean, const float *scale, const float *prob, const float *Q, const uint8_t *in,
+                                  const int32_t *cnt, int64_t n, int k, int min_value, int max_value, int chunk_size, int16_t *sym,
+                                  void *ws, size_t ws_bytes, void *stream) {
+    const int Lp = max_value - min_value + 2;
+    int rc = attr_check(n, Lp, chunk_size);
+    if (rc) return rc;
+    return mixture_run(k, mean, scale, prob, Q, n, min_value, Lp, [&](auto md) {
+        return attr_decode<decltype(md), true, int16_t>(md, in, cnt, n, Lp, chunk_size, sym, ws, ws_bytes, as_stream(stream));
+    });
+}
+
+extern "C" int gpc_row_encode(const int16_t *sym, const float *row, int64_t n, int Lp, int chunk_size, int32_t *cnt, uint32_t *offsets,
+                              void *ws, size_t ws_bytes, void *stream) {
+    int rc = attr_check(n, Lp, chunk_size);
+    if (rc) return rc;
+    SharedRowModel md{row, (float)((1 << ATTR_PRECISION) - (Lp - 1))};
+    return attr_encode(md, sym, n, Lp, chunk_size, cnt, offsets, ws, ws_bytes, as_stream(stream));
+}
+
+extern "C" int gpc_row_decode(const float *row, const uint8_t *in, const int32_t *cnt, int64_t n, int Lp, int chunk_size, int16_t *sym,
+                              void *ws, size_t ws_bytes, void *stream) {
+    int rc = attr_check(n, Lp, chunk_size);
+    if (rc) return rc;
+    SharedRowModel md{row, (float)((1 << ATTR_PRECISION) - (Lp - 1))};
+    return attr_decode<SharedRowModel, false, int16_t>(md, in, cnt, n, Lp, chunk_size, sym, ws, ws_bytes, as_stream(stream));
 }
 
 // ---- the same chunked coder on the geometry codec's own symbols (container version 2, SURVEY 8f-3): the occupancy streams of a

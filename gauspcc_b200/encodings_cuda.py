@@ -4,8 +4,12 @@ so files written by either side are read by the other.
 
     HAC/scene/gaussian_model.py:37   from utils.encodings_cuda import encoder_gaussian_chunk, decoder_gaussian_chunk, encoder, decoder
 
-The single-Gaussian coders never build the reference's lower[N][Lp] table (arithmetic.gaussian_encode / gaussian_decode); the
-mixture coders build it with the same element-wise torch arithmetic as the reference and go through the table entry points.
+No coder here builds the reference's lower[N][Lp] table on the paths HAC and HAC++ take: the single-Gaussian coders evaluate
+each symbol's CDF entries on the fly (arithmetic.gaussian_encode / gaussian_decode), the mixture coders do the same for up to
+four components (arithmetic.mixture_encode / mixture_decode), and the Bernoulli mask coder codes every symbol against one
+shared row [0, 1 - p, 1] (arithmetic.row_encode / row_decode).  The bytes are those of the table path.  Mixture calls the fused
+path cannot reproduce bit for bit (more than four components, components not 1-D of the symbols' length, probabilities that are
+not float32 / float16 / bfloat16) still build the table with the reference's element-wise torch arithmetic (_mixed_lower).
 """
 from __future__ import annotations
 
@@ -106,6 +110,24 @@ def decoder_gaussian_chunk(mean, scale, Q, file_name='tmp.b', chunk_size=1000_00
     return torch.cat(out, dim=0).type_as(mean)
 
 
+_FUSED_PROB_DTYPES = (torch.float32, torch.float16, torch.bfloat16)      # exact in float32, as torch's promotion in `lower * prob`
+
+
+def _takes_fused_mixture(n, mean_list, scale_list, prob_list):
+    """True when arithmetic.mixture_* gives the bytes of the table _mixed_lower builds: 1 to 4 components, every mean / scale /
+    prob a 1-D tensor of length n (no broadcasting) and every prob float32, float16 or bfloat16."""
+    k = len(mean_list)
+    if not 1 <= k <= 4 or len(scale_list) != k or len(prob_list) != k:
+        return False
+    if not all(isinstance(t, torch.Tensor) and tuple(t.shape) == (n,) for t in (*mean_list, *scale_list, *prob_list)):
+        return False
+    return all(p.dtype in _FUSED_PROB_DTYPES for p in prob_list)
+
+
+def _stack_f32(ts):
+    return torch.stack([t.detach().to(torch.float32) for t in ts])      # [K, n], contiguous
+
+
 def _mixed_lower(mean_list, scale_list, prob_list, Q, min_value, max_value):
     lower_all = None                                                        # encodings_cuda.py:211-226
     for mean, scale, prob in zip(mean_list, scale_list, prob_list):
@@ -124,9 +146,13 @@ def encoder_gaussian_mixed(x, mean_list, scale_list, prob_list, Q, file_name='tm
     Q = _q_tensor(Q, x)
     assert x.shape == mean_list[0].shape == scale_list[0].shape == prob_list[0].shape == Q.shape
     x_int_round, min_value, max_value = _quantise(x, Q)
-    lower = _mixed_lower(mean_list, scale_list, prob_list, Q, int(min_value), int(max_value))
     sym = (x_int_round - min_value.to(x.device)).to(torch.int16)
-    stream, cnt = arithmetic.arithmetic_encode(sym.contiguous(), lower, chunk_size_cuda, int(lower.shape[0]), int(lower.shape[1]))
+    if _takes_fused_mixture(x.shape[0], mean_list, scale_list, prob_list):
+        stream, cnt = arithmetic.mixture_encode(sym.contiguous(), _stack_f32(mean_list), _stack_f32(scale_list), _stack_f32(prob_list),
+                                                _f32(Q), int(min_value), int(max_value), chunk_size_cuda)
+    else:
+        lower = _mixed_lower(mean_list, scale_list, prob_list, Q, int(min_value), int(max_value))
+        stream, cnt = arithmetic.arithmetic_encode(sym.contiguous(), lower, chunk_size_cuda, int(lower.shape[0]), int(lower.shape[1]))
     return _write(file_name, [min_value.to(torch.float32).numpy().tobytes(), max_value.to(torch.float32).numpy().tobytes()], cnt, stream)
 
 
@@ -137,8 +163,12 @@ def decoder_gaussian_mixed(mean_list, scale_list, prob_list, Q, file_name='tmp.b
     Q = _q_tensor(Q, m0)
     assert mean_list[0].shape == scale_list[0].shape == prob_list[0].shape == Q.shape
     (mn, mx), cnt, stream = _read(file_name, 2, m0.device)
-    lower = _mixed_lower(mean_list, scale_list, prob_list, Q, int(mn[0]), int(mx[0]))
-    sym = arithmetic.arithmetic_decode(lower, stream, cnt, chunk_size_cuda, int(lower.shape[0]), int(lower.shape[1]))
+    if _takes_fused_mixture(m0.numel(), mean_list, scale_list, prob_list):
+        sym = arithmetic.mixture_decode(_stack_f32(mean_list), _stack_f32(scale_list), _stack_f32(prob_list), _f32(Q), stream, cnt,
+                                        int(mn[0]), int(mx[0]), chunk_size_cuda)
+    else:
+        lower = _mixed_lower(mean_list, scale_list, prob_list, Q, int(mn[0]), int(mx[0]))
+        sym = arithmetic.arithmetic_decode(lower, stream, cnt, chunk_size_cuda, int(lower.shape[0]), int(lower.shape[1]))
     x = sym.to(m0.device).to(torch.float32) + float(mn[0])
     return x * Q
 
@@ -168,11 +198,9 @@ def decoder_gaussian_mixed_chunk(mean_list, scale_list, prob_list, Q, file_name=
     return torch.cat(out, dim=0).type_as(mean_list[0])
 
 
-def _bernoulli_cdf(prob_1, n, device):
-    p = torch.zeros(size=[n], dtype=torch.float32, device=device)           # encodings_cuda.py:439-446
-    p[...] = prob_1
-    p_u = 1 - p.unsqueeze(-1)
-    return torch.cat([torch.zeros_like(p_u), p_u, torch.ones_like(p_u)], dim=-1)
+def _bernoulli_row(prob_1, device):
+    p = torch.as_tensor(prob_1, dtype=torch.float32, device=device).reshape(1)     # encodings_cuda.py:439-446: every row of the
+    return torch.cat([torch.zeros_like(p), 1 - p, torch.ones_like(p)])             # reference's [n, 3] table is [0, 1 - p, 1]
 
 
 def encoder(x, file_name='tmp.b'):
@@ -180,9 +208,8 @@ def encoder(x, file_name='tmp.b'):
     assert file_name[-2:] == '.b'
     x = x.detach().view(-1)
     prob_1 = x.sum() / x.numel()
-    output_cdf = _bernoulli_cdf(prob_1.to(torch.float32), x.numel(), x.device)
     sym = torch.floor(x).to(torch.int16)
-    stream, cnt = arithmetic.arithmetic_encode(sym.contiguous(), output_cdf, chunk_size_cuda, int(output_cdf.shape[0]), 3)
+    stream, cnt = arithmetic.row_encode(sym.contiguous(), _bernoulli_row(prob_1.to(torch.float32), x.device), chunk_size_cuda)
     return _write(file_name, [prob_1.to(torch.float32).cpu().numpy().tobytes()], cnt, stream)
 
 
@@ -190,5 +217,4 @@ def decoder(N_len, file_name='tmp.b', device='cuda'):
     """encodings_cuda.py:470-500"""
     assert file_name[-2:] == '.b'
     (prob_1,), cnt, stream = _read(file_name, 1, device)
-    output_cdf = _bernoulli_cdf(torch.tensor(prob_1, device=device), N_len, device)
-    return arithmetic.arithmetic_decode(output_cdf, stream, cnt, chunk_size_cuda, int(output_cdf.shape[0]), 3)
+    return arithmetic.row_decode(_bernoulli_row(prob_1, device), stream, cnt, N_len, chunk_size_cuda)

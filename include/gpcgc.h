@@ -279,6 +279,22 @@ int gpc_attr_decode_table(const float *cdf, const uint8_t *in, const int32_t *cn
 int gpc_attr_decode_gaussian(const float *mean, const float *scale, const float *Q, const uint8_t *in, const int32_t *cnt,
                              int64_t n, int min_value, int max_value, int chunk_size, int16_t *sym, void *ws,
                              size_t ws_bytes, void *stream);
+/* HAC++'s mixture coder without the table: calculate_cdf per component, `* prob`, summed in list order and clamped to [0, 1]
+ * (encoder_gaussian_mixed / decoder_gaussian_mixed, encodings_cuda.py:203-314), then arithmetic_encode / arithmetic_decode --
+ * the same bytes and symbols, with each symbol's CDF entries evaluated on the fly.  mean / scale / prob: [k][n] float32,
+ * Q: [n].  1 <= k <= 4, else GPC_EINVAL.  Workspace and merge: gpc_attr_workspace_bytes / gpc_attr_merge_chunks. */
+int gpc_mixture_encode(const int16_t *sym, const float *mean, const float *scale, const float *prob, const float *Q,
+                       int64_t n, int k, int min_value, int max_value, int chunk_size, int32_t *cnt, uint32_t *offsets,
+                       void *ws, size_t ws_bytes, void *stream);
+int gpc_mixture_decode(const float *mean, const float *scale, const float *prob, const float *Q, const uint8_t *in,
+                       const int32_t *cnt, int64_t n, int k, int min_value, int max_value, int chunk_size, int16_t *sym,
+                       void *ws, size_t ws_bytes, void *stream);
+/* arithmetic_encode / arithmetic_decode of a table whose n rows are all the same float32 row[Lp]: the Bernoulli mask coder
+ * (encoder / decoder, encodings_cuda.py:435-500, row [0, 1 - p, 1]) without the [n][3] table */
+int gpc_row_encode(const int16_t *sym, const float *row, int64_t n, int Lp, int chunk_size, int32_t *cnt, uint32_t *offsets,
+                   void *ws, size_t ws_bytes, void *stream);
+int gpc_row_decode(const float *row, const uint8_t *in, const int32_t *cnt, int64_t n, int Lp, int chunk_size, int16_t *sym,
+                   void *ws, size_t ws_bytes, void *stream);
 
 /* ---- f-3: the chunked GPU coder on the geometry codec's own streams (container version 2; NOT the torchac bitstream: one coder
  * per chunk instead of one per stream).  Encode: lohi as gpc_head_cdf_sym writes it; no host synchronisation.  Decode: one stream
