@@ -51,15 +51,21 @@ SIGNATURES = {
     "gpc_kmap_pairs_workspace_bytes": (c_sz, [c_i64, c_int]),
     "gpc_kmap_pairs_count": (c_int, [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "gpc_kmap_pairs_fill": (c_int, [c_vp, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "gpc_kmap_pairs_count_range": (c_int, [c_vp, c_i64, c_i64, c_i64, c_int, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_kmap_pairs_fill_range": (c_int, [c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_vp, c_i64, c_vp]),
     "gpc_spconv_pack_weights_frag": (c_int, [c_vp, c_int, c_vp, c_vp]),
     "gpc_spconv_fwd_v6": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_vp, c_int, c_vp, c_int, c_vp]),
     "gpc_spconv_fwd_v6_rows": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_vp, c_int, c_vp, c_int, c_i64, c_i64, c_vp]),
+    "gpc_spconv_fwd_v6_range": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_int, c_vp, c_int, c_vp]),
     "gpc_kmap_sparse_segments": (c_i64, [c_i64]),
     "gpc_kmap_sparse_workspace_bytes": (c_sz, [c_i64]),
     "gpc_kmap_sparse_count": (c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "gpc_kmap_sparse_fill": (c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gpc_spconv_sparse_fwd": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_int, c_vp, c_vp]),
     "gpc_spconv_sparse_fwd_rows": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_int, c_vp, c_i64, c_i64, c_vp]),
+    "gpc_kmap_sparse_count_range": (c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_kmap_sparse_fill_range": (c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "gpc_spconv_sparse_fwd_range": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_int, c_vp, c_vp]),
     "gpc_rows_split": (c_int, [c_vp, c_i64, c_vp, c_vp]),
     "gpc_rows_join": (c_int, [c_vp, c_i64, c_vp, c_vp]),
     "gpc_debug_conv_um_profile": (c_int, [c_vp, c_int]),
@@ -69,6 +75,9 @@ SIGNATURES = {
     "gpc_kmap_um_fill": (c_int, [c_vp, c_i64, c_int, c_vp, c_vp, c_vp, c_vp]),
     "gpc_spconv_pack_weights_um": (c_int, [c_vp, c_int, c_vp, c_vp]),
     "gpc_spconv_fwd_um": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_vp, c_vp, c_int, c_vp, c_vp, c_i64, c_i64, c_vp]),
+    "gpc_kmap_um_count_range": (c_int, [c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_kmap_um_fill_range": (c_int, [c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_vp]),
+    "gpc_spconv_fwd_um_range": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_int, c_vp, c_vp, c_vp]),
     "gpc_embed_rows": (c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "gpc_gather_parent_add_octant": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "gpc_add_ctx_embed": (c_int, [c_vp, c_vp, c_int, c_vp, c_i64, c_vp, c_vp, c_vp]),

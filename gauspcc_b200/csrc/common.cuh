@@ -37,6 +37,9 @@ extern unsigned long long g_gpc_launches;     // kernels launched by this librar
             return code;                                                                  \
         }                                                                                 \
     } while (0)
+// [row0, row1) must be a row range of a level of n_level rows (the *_range entry points: one scene of a batch union level)
+#define GPC_RANGE_CHECK(n_level, row0, row1) \
+    GPC_REQUIRE((row0) >= 0 && (row0) <= (row1) && (row1) <= (n_level), GPC_EINVAL, "row range outside the level")
 
 static inline cudaStream_t as_stream(void *s) { return (cudaStream_t)s; }
 static inline unsigned cdiv(i64 a, i64 b) { return (unsigned)((a + b - 1) / b); }

@@ -168,7 +168,7 @@ __global__ void kmap_total_kernel(const u32 *__restrict__ seg, i64 m, u32 *__res
 // ---- warp-per-tile kernels (tile_rows = 32 * RPL, RPL = 1, 2, 4): no block barriers, each warp streams its tile's
 // 125 x tile_rows slice of the dense map with coalesced loads and ballots.
 template <int RPL>
-__global__ void __launch_bounds__(128) kmap_pairs_count_warp_kernel(const i32 *__restrict__ map, i64 n, i64 tiles, int pad,
+__global__ void __launch_bounds__(128) kmap_pairs_count_warp_kernel(const i32 *__restrict__ map, i64 n, i64 ld, i64 tiles, int pad,
                                                                    u32 *__restrict__ counts, u32 *__restrict__ n_real) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const i64 t = blockIdx.x;                       // one CTA per tile, warp w takes offsets w, w + 4, ... ((tile, offset) cells are independent)
@@ -180,7 +180,7 @@ __global__ void __launch_bounds__(128) kmap_pairs_count_warp_kernel(const i32 *_
 #pragma unroll
         for (int i = 0; i < RPL; ++i) {
             const i64 r = r0 + i * 32 + lane;
-            const bool v = r < n && map[(i64)k * n + r] >= 0;
+            const bool v = r < n && map[(i64)k * ld + r] >= 0;
             c += __popc(__ballot_sync(0xFFFFFFFFu, v));
         }
         real += c;
@@ -191,20 +191,21 @@ __global__ void __launch_bounds__(128) kmap_pairs_count_warp_kernel(const i32 *_
 }
 
 template <int RPL>
-__global__ void __launch_bounds__(128) kmap_pairs_fill_warp_kernel(const i32 *__restrict__ map, i64 n, i64 tiles,
+__global__ void __launch_bounds__(128) kmap_pairs_fill_warp_kernel(const i32 *__restrict__ map, i64 n, i64 ld, i64 tiles,
                                                                   const u32 *__restrict__ seg, u32 *__restrict__ pair_nbr,
                                                                   u16 *__restrict__ pair_row, u64 *__restrict__ pairs) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const i64 t = blockIdx.x;
     const i64 r0 = t * (32 * RPL);
     const u32 lt = (1u << lane) - 1u;
+    const i64 left = n - r0 - lane;                 // rows of this tile at or after this lane's first row
 #pragma unroll 4
     for (int k = wid; k < GPC_K3; k += 4) {
         u32 p = seg[t * (GPC_K3 + 1) + k];
+        const i32 *mk = map + (i64)k * ld + r0 + lane;
 #pragma unroll
         for (int i = 0; i < RPL; ++i) {
-            const i64 r = r0 + i * 32 + lane;
-            const i32 nb = r < n ? map[(i64)k * n + r] : -1;
+            const i32 nb = i * 32 < left ? mk[i * 32] : -1;
             const u32 bal = __ballot_sync(0xFFFFFFFFu, nb >= 0);
             if (nb >= 0) {
                 const u32 q = p + __popc(bal & lt);
@@ -219,7 +220,7 @@ __global__ void __launch_bounds__(128) kmap_pairs_fill_warp_kernel(const i32 *__
 // ---- sub-warp tiles (tile_rows = 8 or 16): one warp covers 32 / TW tiles, each group of TW lanes is one tile.
 // Small tiles give the conv enough warps on the coarse octree levels (a few hundred to a few ten-thousand rows).
 template <int TW>
-__global__ void __launch_bounds__(128) kmap_pairs_count_sub_kernel(const i32 *__restrict__ map, i64 n, i64 tiles, int pad,
+__global__ void __launch_bounds__(128) kmap_pairs_count_sub_kernel(const i32 *__restrict__ map, i64 n, i64 ld, i64 tiles, int pad,
                                                                   u32 *__restrict__ counts, u32 *__restrict__ n_real) {
     constexpr int SUB = 32 / TW;
     const int lane = threadIdx.x & 31, sub = lane / TW, rl = lane % TW;
@@ -229,7 +230,7 @@ __global__ void __launch_bounds__(128) kmap_pairs_count_sub_kernel(const i32 *__
     u32 real = 0;
 #pragma unroll 5
     for (int k = 0; k < GPC_K3; ++k) {
-        const bool v = live && r < n && map[(i64)k * n + r] >= 0;
+        const bool v = live && r < n && map[(i64)k * ld + r] >= 0;
         const u32 bits = (__ballot_sync(0xFFFFFFFFu, v) >> (TW * sub)) & ((1u << TW) - 1u);
         const u32 c = __popc(bits);
         real += c;
@@ -238,7 +239,7 @@ __global__ void __launch_bounds__(128) kmap_pairs_count_sub_kernel(const i32 *__
     if (live && rl == 0) { counts[t * (GPC_K3 + 1) + GPC_K3] = 0; atomicAdd(n_real, real); }
 }
 template <int TW>
-__global__ void __launch_bounds__(128) kmap_pairs_fill_sub_kernel(const i32 *__restrict__ map, i64 n, i64 tiles,
+__global__ void __launch_bounds__(128) kmap_pairs_fill_sub_kernel(const i32 *__restrict__ map, i64 n, i64 ld, i64 tiles,
                                                                  const u32 *__restrict__ seg, u32 *__restrict__ pair_nbr,
                                                                  u16 *__restrict__ pair_row, u64 *__restrict__ pairs) {
     constexpr int SUB = 32 / TW;
@@ -248,7 +249,7 @@ __global__ void __launch_bounds__(128) kmap_pairs_fill_sub_kernel(const i32 *__r
     const bool live = t < tiles;
 #pragma unroll 5
     for (int k = 0; k < GPC_K3; ++k) {
-        const i32 nb = (live && r < n) ? map[(i64)k * n + r] : -1;
+        const i32 nb = (live && r < n) ? map[(i64)k * ld + r] : -1;
         const u32 bits = (__ballot_sync(0xFFFFFFFFu, nb >= 0) >> (TW * sub)) & ((1u << TW) - 1u);
         if (nb >= 0) {
             const u32 q = seg[t * (GPC_K3 + 1) + k] + __popc(bits & ((1u << rl) - 1u));
@@ -263,8 +264,10 @@ extern "C" size_t gpc_kmap_pairs_workspace_bytes(int64_t n, int tile_rows) {
     const i64 m = tiles * (GPC_K3 + 1);
     return align_up((size_t)m * 4, 256) + align_up(scan_workspace_bytes<u32>(m), 256) + 1024;
 }
-extern "C" int gpc_kmap_pairs_count(const int32_t *map, int64_t n, int tile_rows, int pad, uint32_t *seg, uint32_t *n_pairs,
-                                    void *ws, size_t ws_bytes, void *stream) {
+// map: the rows [0, n) of a dense map whose offset planes are ld >= n ints apart (ld = n: a whole level; ld > n: a row range of a
+// level, map already advanced to its first row -- gpc_kmap_pairs_count_range)
+static int pairs_count(const int32_t *map, int64_t n, int64_t ld, int tile_rows, int pad, uint32_t *seg, uint32_t *n_pairs, void *ws,
+                       size_t ws_bytes, void *stream) {
     cudaStream_t st = as_stream(stream);
     GPC_REQUIRE((tile_rows == 8 || tile_rows == 16 || tile_rows == 32 || tile_rows == 64 || tile_rows == 128) && pad >= 1, GPC_EINVAL,
                 "tile_rows must be 8, 16, 32, 64 or 128, pad >= 1");
@@ -275,11 +278,11 @@ extern "C" int gpc_kmap_pairs_count(const int32_t *map, int64_t n, int tile_rows
     u32 *counts = (u32 *)ws;
     void *scan_ws = (char *)ws + align_up((size_t)m * 4, 256);
     GPC_CUDA_CHECK(cudaMemsetAsync(n_pairs, 0, 8, st));      // n_pairs[0] = stream entries (padded), n_pairs[1] = true pairs
-    if (tile_rows == 8) kmap_pairs_count_sub_kernel<8><<<cdiv(tiles, 16), 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
-    else if (tile_rows == 16) kmap_pairs_count_sub_kernel<16><<<cdiv(tiles, 8), 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
-    else if (tile_rows == 32) kmap_pairs_count_warp_kernel<1><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
-    else if (tile_rows == 64) kmap_pairs_count_warp_kernel<2><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
-    else kmap_pairs_count_warp_kernel<4><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, pad, counts, n_pairs + 1);
+    if (tile_rows == 8) kmap_pairs_count_sub_kernel<8><<<cdiv(tiles, 16), 128, 0, st>>>(map, n, ld, tiles, pad, counts, n_pairs + 1);
+    else if (tile_rows == 16) kmap_pairs_count_sub_kernel<16><<<cdiv(tiles, 8), 128, 0, st>>>(map, n, ld, tiles, pad, counts, n_pairs + 1);
+    else if (tile_rows == 32) kmap_pairs_count_warp_kernel<1><<<(unsigned)tiles, 128, 0, st>>>(map, n, ld, tiles, pad, counts, n_pairs + 1);
+    else if (tile_rows == 64) kmap_pairs_count_warp_kernel<2><<<(unsigned)tiles, 128, 0, st>>>(map, n, ld, tiles, pad, counts, n_pairs + 1);
+    else kmap_pairs_count_warp_kernel<4><<<(unsigned)tiles, 128, 0, st>>>(map, n, ld, tiles, pad, counts, n_pairs + 1);
     GPC_LAUNCH_CHECK();
     PtrLoad<u32> pl{counts};
     int rc = device_exclusive_scan<u32, PtrLoad<u32>>(pl, m, seg, scan_ws, st);      // seg has m+1 entries
@@ -288,8 +291,8 @@ extern "C" int gpc_kmap_pairs_count(const int32_t *map, int64_t n, int tile_rows
     GPC_LAUNCH_CHECK();
     return GPC_OK;
 }
-extern "C" int gpc_kmap_pairs_fill(const int32_t *map, int64_t n, int tile_rows, const uint32_t *seg, uint32_t *pair_nbr,
-                                   uint16_t *pair_row, uint64_t *pairs, int64_t n_entries, void *stream) {
+static int pairs_fill(const int32_t *map, int64_t n, int64_t ld, int tile_rows, const uint32_t *seg, uint32_t *pair_nbr,
+                      uint16_t *pair_row, uint64_t *pairs, int64_t n_entries, void *stream) {
     if (n <= 0) return GPC_OK;
     GPC_REQUIRE(tile_rows == 8 || tile_rows == 16 || tile_rows == 32 || tile_rows == 64 || tile_rows == 128, GPC_EINVAL,
                 "tile_rows must be 8, 16, 32, 64 or 128");
@@ -301,22 +304,41 @@ extern "C" int gpc_kmap_pairs_fill(const int32_t *map, int64_t n, int tile_rows,
     }
     const i64 tiles = (n + tile_rows - 1) / tile_rows;
     cudaStream_t st = as_stream(stream);
-    if (tile_rows == 8) kmap_pairs_fill_sub_kernel<8><<<cdiv(tiles, 16), 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
-    else if (tile_rows == 16) kmap_pairs_fill_sub_kernel<16><<<cdiv(tiles, 8), 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
-    else if (tile_rows == 32) kmap_pairs_fill_warp_kernel<1><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
-    else if (tile_rows == 64) kmap_pairs_fill_warp_kernel<2><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
-    else kmap_pairs_fill_warp_kernel<4><<<(unsigned)tiles, 128, 0, st>>>(map, n, tiles, seg, pair_nbr, pair_row, pairs);
+    if (tile_rows == 8) kmap_pairs_fill_sub_kernel<8><<<cdiv(tiles, 16), 128, 0, st>>>(map, n, ld, tiles, seg, pair_nbr, pair_row, pairs);
+    else if (tile_rows == 16) kmap_pairs_fill_sub_kernel<16><<<cdiv(tiles, 8), 128, 0, st>>>(map, n, ld, tiles, seg, pair_nbr, pair_row, pairs);
+    else if (tile_rows == 32) kmap_pairs_fill_warp_kernel<1><<<(unsigned)tiles, 128, 0, st>>>(map, n, ld, tiles, seg, pair_nbr, pair_row, pairs);
+    else if (tile_rows == 64) kmap_pairs_fill_warp_kernel<2><<<(unsigned)tiles, 128, 0, st>>>(map, n, ld, tiles, seg, pair_nbr, pair_row, pairs);
+    else kmap_pairs_fill_warp_kernel<4><<<(unsigned)tiles, 128, 0, st>>>(map, n, ld, tiles, seg, pair_nbr, pair_row, pairs);
     GPC_LAUNCH_CHECK();
     return GPC_OK;
 }
-
+extern "C" int gpc_kmap_pairs_count(const int32_t *map, int64_t n, int tile_rows, int pad, uint32_t *seg, uint32_t *n_pairs,
+                                    void *ws, size_t ws_bytes, void *stream) {
+    return pairs_count(map, n, n, tile_rows, pad, seg, n_pairs, ws, ws_bytes, stream);
+}
+extern "C" int gpc_kmap_pairs_fill(const int32_t *map, int64_t n, int tile_rows, const uint32_t *seg, uint32_t *pair_nbr,
+                                   uint16_t *pair_row, uint64_t *pairs, int64_t n_entries, void *stream) {
+    return pairs_fill(map, n, n, tile_rows, seg, pair_nbr, pair_row, pairs, n_entries, stream);
+}
+// row ranges [row0, row1) of a level of n_level rows (a batch of scenes coded as one union level): tiles start at row0, neighbour
+// indices stay the level's rows, and the totals are the range's own (entries, true pairs)
+extern "C" int gpc_kmap_pairs_count_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, int tile_rows, int pad,
+                                          uint32_t *seg, uint32_t *n_pairs, void *ws, size_t ws_bytes, void *stream) {
+    GPC_RANGE_CHECK(n_level, row0, row1);
+    return pairs_count(map + row0, row1 - row0, n_level, tile_rows, pad, seg, n_pairs, ws, ws_bytes, stream);
+}
+extern "C" int gpc_kmap_pairs_fill_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, int tile_rows,
+                                         const uint32_t *seg, uint64_t *pairs, int64_t n_entries, void *stream) {
+    GPC_RANGE_CHECK(n_level, row0, row1);
+    return pairs_fill(map + row0, row1 - row0, n_level, tile_rows, seg, nullptr, nullptr, pairs, n_entries, stream);
+}
 
 // ---------------------------------------------------------------- pair stream of the tcgen05 conv (spconv_um.cu)
 // Tiles of 256 .. 1024 output rows; one WARP per (tile, offset) cell: the cell's slice of the offset-major dense map is tile_rows
 // consecutive ints, read with coalesced loads and ranked with ballots.  Every non-empty cell is padded to a multiple of 16 entries; the stream holds,
 // per entry, the input row (padding: 0xFFFFFFFF = out of bounds for the gather) and the BYTE OFFSET of the pair's accumulator row
 // inside the tile (row * 128; padding: the dummy row tile_rows * 128).
-__global__ void __launch_bounds__(128) kmap_um_count_kernel(const i32 *__restrict__ map, i64 n, int tile_rows, i64 cells,
+__global__ void __launch_bounds__(128) kmap_um_count_kernel(const i32 *__restrict__ map, i64 n, i64 ld, int tile_rows, i64 cells,
                                                            u32 *__restrict__ counts) {
     const int lane = threadIdx.x & 31;
     const i64 cell = (i64)blockIdx.x * 4 + (threadIdx.x >> 5);           // = tile * 126 + k; k == 125 is the zero pad of the scan
@@ -327,7 +349,7 @@ __global__ void __launch_bounds__(128) kmap_um_count_kernel(const i32 *__restric
     if (k < GPC_K3) {
         const i64 r0 = t * tile_rows;
         const int rows = (int)min((i64)tile_rows, n - r0);
-        const i32 *m = map + (i64)k * n + r0;
+        const i32 *m = map + (i64)k * ld + r0;
         for (int r = lane; r < rows; r += 32) c += m[r] >= 0;
         c = __reduce_add_sync(0xFFFFFFFFu, c);
     }
@@ -351,7 +373,7 @@ struct Pad16Load {                                                       // ever
     const u32 *p;
     __device__ u32 operator()(i64 i) const { return (p[i] + 15u) & ~15u; }
 };
-__global__ void __launch_bounds__(128) kmap_um_fill_kernel(const i32 *__restrict__ map, i64 n, int tile_rows, i64 cells,
+__global__ void __launch_bounds__(128) kmap_um_fill_kernel(const i32 *__restrict__ map, i64 n, i64 ld, int tile_rows, i64 cells,
                                                           const u32 *__restrict__ seg, u32 *__restrict__ pair_nbr, u32 *__restrict__ pair_off) {
     const int lane = threadIdx.x & 31;
     const i64 cell = (i64)blockIdx.x * 4 + (threadIdx.x >> 5);
@@ -364,7 +386,7 @@ __global__ void __launch_bounds__(128) kmap_um_fill_kernel(const i32 *__restrict
     if (p == end) return;
     const i64 r0 = t * tile_rows;
     const int rows = (int)min((i64)tile_rows, n - r0);
-    const i32 *m = map + (i64)k * n + r0;
+    const i32 *m = map + (i64)k * ld + r0;
     const u32 lt = (1u << lane) - 1u;
     for (int rb = 0; rb < rows; rb += 32) {                               // ascending row order inside a cell
         const int r = rb + lane;
@@ -402,9 +424,9 @@ extern "C" int gpc_kmap_um_scan(const uint32_t *cell_counts, int64_t n, int tile
     GPC_CUDA_CHECK(cudaMemcpyAsync(totals, seg + m, 4, cudaMemcpyDeviceToDevice, st));
     return GPC_OK;
 }
-// the same from a dense map that was built without counting (any tile_rows in 32..1024; tools, tests)
-extern "C" int gpc_kmap_um_count(const int32_t *map, int64_t n, int tile_rows, uint32_t *seg, unsigned long long *totals, void *ws,
-                                 size_t ws_bytes, void *stream) {
+// the same from a dense map that was built without counting (any tile_rows in 32..1024; tools, tests).  ld as in pairs_count.
+static int um_count(const int32_t *map, int64_t n, int64_t ld, int tile_rows, uint32_t *seg, unsigned long long *totals, void *ws,
+                    size_t ws_bytes, void *stream) {
     cudaStream_t st = as_stream(stream);
     GPC_REQUIRE(tile_rows >= 32 && tile_rows <= 1024, GPC_EINVAL, "tile_rows must be in 32..1024");
     if (n <= 0) { GPC_CUDA_CHECK(cudaMemsetAsync(totals, 0, 16, st)); return GPC_OK; }
@@ -412,16 +434,34 @@ extern "C" int gpc_kmap_um_count(const int32_t *map, int64_t n, int tile_rows, u
     const i64 tiles = (n + tile_rows - 1) / tile_rows;
     const i64 m = tiles * (GPC_K3 + 1);
     u32 *counts = (u32 *)ws;
-    kmap_um_count_kernel<<<cdiv(m, 4), 128, 0, st>>>(map, n, tile_rows, m, counts);
+    kmap_um_count_kernel<<<cdiv(m, 4), 128, 0, st>>>(map, n, ld, tile_rows, m, counts);
     GPC_LAUNCH_CHECK();
     return gpc_kmap_um_scan(counts, n, tile_rows, seg, totals, ws, ws_bytes, stream);
 }
-extern "C" int gpc_kmap_um_fill(const int32_t *map, int64_t n, int tile_rows, const uint32_t *seg, uint32_t *pair_nbr,
-                                uint32_t *pair_off, void *stream) {
+static int um_fill(const int32_t *map, int64_t n, int64_t ld, int tile_rows, const uint32_t *seg, uint32_t *pair_nbr,
+                   uint32_t *pair_off, void *stream) {
     if (n <= 0) return GPC_OK;
     const i64 tiles = (n + tile_rows - 1) / tile_rows;
     const i64 m = tiles * (GPC_K3 + 1);
-    kmap_um_fill_kernel<<<cdiv(m, 4), 128, 0, as_stream(stream)>>>(map, n, tile_rows, m, seg, pair_nbr, pair_off);
+    kmap_um_fill_kernel<<<cdiv(m, 4), 128, 0, as_stream(stream)>>>(map, n, ld, tile_rows, m, seg, pair_nbr, pair_off);
     GPC_LAUNCH_CHECK();
     return GPC_OK;
+}
+extern "C" int gpc_kmap_um_count(const int32_t *map, int64_t n, int tile_rows, uint32_t *seg, unsigned long long *totals, void *ws,
+                                 size_t ws_bytes, void *stream) {
+    return um_count(map, n, n, tile_rows, seg, totals, ws, ws_bytes, stream);
+}
+extern "C" int gpc_kmap_um_fill(const int32_t *map, int64_t n, int tile_rows, const uint32_t *seg, uint32_t *pair_nbr,
+                                uint32_t *pair_off, void *stream) {
+    return um_fill(map, n, n, tile_rows, seg, pair_nbr, pair_off, stream);
+}
+extern "C" int gpc_kmap_um_count_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, int tile_rows, uint32_t *seg,
+                                       unsigned long long *totals, void *ws, size_t ws_bytes, void *stream) {
+    GPC_RANGE_CHECK(n_level, row0, row1);
+    return um_count(map + row0, row1 - row0, n_level, tile_rows, seg, totals, ws, ws_bytes, stream);
+}
+extern "C" int gpc_kmap_um_fill_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, int tile_rows,
+                                      const uint32_t *seg, uint32_t *pair_nbr, uint32_t *pair_off, void *stream) {
+    GPC_RANGE_CHECK(n_level, row0, row1);
+    return um_fill(map + row0, row1 - row0, n_level, tile_rows, seg, pair_nbr, pair_off, stream);
 }

@@ -442,4 +442,15 @@ extern "C" int gpc_spconv_fwd_v6_rows(const float *x, const void *Wa, const uint
     return GPC_OK;
 }
 
-
+// The conv of one scene of a batch union level: output rows [row0, row1) of a level of n_level rows, with the pair stream of that
+// range (gpc_kmap_pairs_count_range / _fill_range: tiles start at row0, neighbour indices are the level's rows).  x, y and residual
+// are the level's arrays; every (variant, tile_rows) of gpc_spconv_fwd_v6.  The kernels gather x[nbr] and write tile-relative output
+// rows, so the range is the whole-level launch on y + row0: its sums are the single scene's, bit for bit.
+extern "C" int gpc_spconv_fwd_v6_range(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs, int64_t n_level,
+                                       int64_t row0, int64_t row1, int tile_rows, const float *residual, int flags, float *y,
+                                       int variant, void *stream) {
+    GPC_RANGE_CHECK(n_level, row0, row1);
+    GPC_REQUIRE(x != y, GPC_EINVAL, "conv is out of place (rows are gathered from x while y is written)");
+    return gpc_spconv_fwd_v6(x, Wa, seg, pairs, row1 - row0, tile_rows, residual ? residual + row0 * GPC_C : nullptr, flags,
+                             y + row0 * GPC_C, variant, stream);
+}

@@ -39,7 +39,7 @@ __device__ __forceinline__ void sp_mma(float (&d)[4], const uint4 &a, u32 b0, u3
 
 // ---------------------------------------------------------------- sparse map: count
 // one warp per 32-row sub-tile: cnt2[(b * 124 + kk) * 256 + st] = rows of the sub-tile with a neighbour at offset kk; rowcnt[r]
-__global__ void __launch_bounds__(128) sp_count_kernel(const i32 *__restrict__ map, i64 n, i64 n_sub, u32 *__restrict__ cnt2,
+__global__ void __launch_bounds__(128) sp_count_kernel(const i32 *__restrict__ map, i64 n, i64 ld, i64 n_sub, u32 *__restrict__ cnt2,
                                                        u32 *__restrict__ rowcnt) {
     const int lane = threadIdx.x & 31;
     const i64 sg = (i64)blockIdx.x * 4 + (threadIdx.x >> 5);
@@ -50,7 +50,7 @@ __global__ void __launch_bounds__(128) sp_count_kernel(const i32 *__restrict__ m
     u32 rc = 0;
 #pragma unroll 4
     for (int kk = 0; kk < SP_KK; ++kk) {
-        const bool v = r < n && map[(i64)sp_offset(kk) * n + r] >= 0;
+        const bool v = r < n && map[(i64)sp_offset(kk) * ld + r] >= 0;
         const u32 c = __popc(__ballot_sync(0xFFFFFFFFu, v));
         rc += v ? 1u : 0u;
         if (lane == 0) cnt2[((size_t)b * SP_KK + kk) * SP_ST + st] = c;
@@ -79,7 +79,7 @@ __global__ void sp_totals_kernel(const u32 *__restrict__ seg, i64 m, const u32 *
     totals[1] = rowptr[n];       // true stragglers
 }
 // one warp per 32-row sub-tile: pairs[seg + pos2 + rank] = nbr | (rowptr[row] + rank of the offset within the row) << 32
-__global__ void __launch_bounds__(128) sp_fill_kernel(const i32 *__restrict__ map, i64 n, i64 n_sub, const u32 *__restrict__ seg,
+__global__ void __launch_bounds__(128) sp_fill_kernel(const i32 *__restrict__ map, i64 n, i64 ld, i64 n_sub, const u32 *__restrict__ seg,
                                                       const u32 *__restrict__ pos2, const u32 *__restrict__ rowptr,
                                                       u64 *__restrict__ pairs) {
     const int lane = threadIdx.x & 31;
@@ -92,7 +92,7 @@ __global__ void __launch_bounds__(128) sp_fill_kernel(const i32 *__restrict__ ma
     u32 dst = r < n ? rowptr[r] : 0u;
 #pragma unroll 4
     for (int kk = 0; kk < SP_KK; ++kk) {
-        const i32 nb = r < n ? map[(i64)sp_offset(kk) * n + r] : -1;
+        const i32 nb = r < n ? map[(i64)sp_offset(kk) * ld + r] : -1;
         const u32 bal = __ballot_sync(0xFFFFFFFFu, nb >= 0);
         if (bal == 0) continue;
         if (nb >= 0) {
@@ -328,8 +328,10 @@ extern "C" size_t gpc_kmap_sparse_workspace_bytes(int64_t n) { return sp_ws_layo
 
 // map: dense offset-major map [125][n] (gpc_kmap_dense).  seg: u32[segments + 1], rowptr: u32[n + 1], totals: device u32[2] =
 // {stream entries (padded to 8 per segment), true stragglers}.  ws is shared with gpc_kmap_sparse_fill (keep it alive).
-extern "C" int gpc_kmap_sparse_count(const int32_t *map, int64_t n, uint32_t *seg, uint32_t *rowptr, uint32_t *totals, void *ws,
-                                     size_t ws_bytes, void *stream) {
+// map: rows [0, n) of a dense map whose offset planes are ld ints apart (ld = n: a whole level; ld > n: a row range, map advanced
+// to its first row)
+static int sparse_count(const int32_t *map, int64_t n, int64_t ld, uint32_t *seg, uint32_t *rowptr, uint32_t *totals, void *ws,
+                        size_t ws_bytes, void *stream) {
     cudaStream_t st = as_stream(stream);
     if (n <= 0) { GPC_CUDA_CHECK(cudaMemsetAsync(totals, 0, 8, st)); return GPC_OK; }
     SpWs L = sp_ws_layout(ws, n);
@@ -338,7 +340,7 @@ extern "C" int gpc_kmap_sparse_count(const int32_t *map, int64_t n, uint32_t *se
     const i64 nb = (n + SP_TB - 1) / SP_TB, n_sub = (n + 31) / 32, n_seg = nb * SP_KK;
     GPC_CUDA_CHECK(cudaMemsetAsync(L.cnt2, 0, (size_t)nb * SP_KK * SP_ST * 4, st));        // sub-tiles past the end of the last block
     GPC_CUDA_CHECK(cudaMemsetAsync(L.tot8, 0, (size_t)nb * GPC_K3 * 4, st));
-    sp_count_kernel<<<cdiv(n_sub, 4), 128, 0, st>>>(map, n, n_sub, L.cnt2, L.rowcnt);
+    sp_count_kernel<<<cdiv(n_sub, 4), 128, 0, st>>>(map, n, ld, n_sub, L.cnt2, L.rowcnt);
     GPC_LAUNCH_CHECK();
     sp_segment_kernel<<<cdiv(n_seg, 4), 128, 0, st>>>(L.cnt2, n_seg, L.tot8);
     GPC_LAUNCH_CHECK();
@@ -352,25 +354,47 @@ extern "C" int gpc_kmap_sparse_count(const int32_t *map, int64_t n, uint32_t *se
     GPC_LAUNCH_CHECK();
     return GPC_OK;
 }
-extern "C" int gpc_kmap_sparse_fill(const int32_t *map, int64_t n, const uint32_t *seg, const uint32_t *rowptr, const void *ws,
-                                    uint64_t *pairs, int64_t n_entries, void *stream) {
+static int sparse_fill(const int32_t *map, int64_t n, int64_t ld, const uint32_t *seg, const uint32_t *rowptr, const void *ws,
+                       uint64_t *pairs, int64_t n_entries, void *stream) {
     if (n <= 0 || n_entries <= 0) return GPC_OK;
     cudaStream_t st = as_stream(stream);
     SpWs L = sp_ws_layout(const_cast<void *>(ws), n);
     GPC_CUDA_CHECK(cudaMemsetAsync(pairs, 0xFF, (size_t)n_entries * 8, st));
     const i64 n_sub = (n + 31) / 32;
-    sp_fill_kernel<<<cdiv(n_sub, 4), 128, 0, st>>>(map, n, n_sub, seg, L.cnt2, rowptr, pairs);
+    sp_fill_kernel<<<cdiv(n_sub, 4), 128, 0, st>>>(map, n, ld, n_sub, seg, L.cnt2, rowptr, pairs);
     GPC_LAUNCH_CHECK();
     return GPC_OK;
 }
 
+extern "C" int gpc_kmap_sparse_count(const int32_t *map, int64_t n, uint32_t *seg, uint32_t *rowptr, uint32_t *totals, void *ws,
+                                     size_t ws_bytes, void *stream) {
+    return sparse_count(map, n, n, seg, rowptr, totals, ws, ws_bytes, stream);
+}
+extern "C" int gpc_kmap_sparse_fill(const int32_t *map, int64_t n, const uint32_t *seg, const uint32_t *rowptr, const void *ws,
+                                    uint64_t *pairs, int64_t n_entries, void *stream) {
+    return sparse_fill(map, n, n, seg, rowptr, ws, pairs, n_entries, stream);
+}
+// the sparse map of the rows [row0, row1) of a level of n_level rows: blocks start at row0, rowptr / dst are range-local, neighbour
+// indices stay the level's rows; seg, rowptr and ws are sized for the range's row count (gpc_kmap_sparse_segments(row1 - row0), ...)
+extern "C" int gpc_kmap_sparse_count_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, uint32_t *seg,
+                                           uint32_t *rowptr, uint32_t *totals, void *ws, size_t ws_bytes, void *stream) {
+    GPC_RANGE_CHECK(n_level, row0, row1);
+    return sparse_count(map + row0, row1 - row0, n_level, seg, rowptr, totals, ws, ws_bytes, stream);
+}
+extern "C" int gpc_kmap_sparse_fill_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, const uint32_t *seg,
+                                          const uint32_t *rowptr, const void *ws, uint64_t *pairs, int64_t n_entries, void *stream) {
+    GPC_RANGE_CHECK(n_level, row0, row1);
+    return sparse_fill(map + row0, row1 - row0, n_level, seg, rowptr, ws, pairs, n_entries, stream);
+}
+
 // y[o,:] = act( W[centre]^T x[o,:] + sum over the row's stragglers, ascending offset (+ residual[o,:]) ).  Wa = this conv's slice of
 // gpc_spconv_pack_weights_frag; contrib = caller scratch of max(stragglers, 1) * 32 floats (fully rewritten by every call).
-static int sp_fwd_rows(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs, const uint32_t *rowptr, int64_t n,
+// xg: the rows the stragglers gather (x[nbr]); x: the centre rows, indexed like y (the same array but for a range of a union level).
+static int sp_fwd_rows(const float *xg, const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs, const uint32_t *rowptr, int64_t n,
                        int64_t n_entries, float *contrib, const float *residual, int flags, float *y, int64_t row0, int64_t row1,
                        void *stream) {
     if (n <= 0 || row1 <= row0) return GPC_OK;
-    GPC_REQUIRE(x != y, GPC_EINVAL, "conv is out of place (rows are gathered from x while y is written)");
+    GPC_REQUIRE(x != y && xg != y, GPC_EINVAL, "conv is out of place (rows are gathered from x while y is written)");
     GPC_REQUIRE(row0 >= 0 && row1 <= n && row0 % SP_TB == 0 && (row1 % SP_TB == 0 || row1 == n), GPC_EINVAL,
                 "row range must be made of whole 8192-row blocks");
     cudaStream_t st = as_stream(stream);
@@ -378,7 +402,7 @@ static int sp_fwd_rows(const float *x, const void *Wa, const uint32_t *seg, cons
     const i64 seg0 = row0 / SP_TB * SP_KK, seg1 = (row1 + SP_TB - 1) / SP_TB * SP_KK;
     if (n_entries > 0) {
         const int split = n_entries >= 256 * n_seg ? 8 : (n_entries >= 64 * n_seg ? 4 : 1);      // by the level, not by the range
-        sp_straggler_kernel<<<cdiv((seg1 - seg0) * split, 4), 128, 0, st>>>(x, (const uint4 *)Wa, seg, pairs, seg0, seg1, split, contrib);
+        sp_straggler_kernel<<<cdiv((seg1 - seg0) * split, 4), 128, 0, st>>>(xg, (const uint4 *)Wa, seg, pairs, seg0, seg1, split, contrib);
         GPC_LAUNCH_CHECK();
     }
     sp_centre_kernel<<<cdiv(row1 - row0, 4 * SP_ROWS), 128, 0, st>>>(x, (const uint4 *)Wa, rowptr, contrib, row0, row1, residual, flags, y);
@@ -388,12 +412,24 @@ static int sp_fwd_rows(const float *x, const void *Wa, const uint32_t *seg, cons
 extern "C" int gpc_spconv_sparse_fwd(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs,
                                      const uint32_t *rowptr, int64_t n, int64_t n_entries, float *contrib, const float *residual,
                                      int flags, float *y, void *stream) {
-    return sp_fwd_rows(x, Wa, seg, pairs, rowptr, n, n_entries, contrib, residual, flags, y, 0, n, stream);
+    return sp_fwd_rows(x, x, Wa, seg, pairs, rowptr, n, n_entries, contrib, residual, flags, y, 0, n, stream);
 }
 // The same conv for the output rows [row0, row1) only (whole 8192-row blocks; row1 may be n): x, y, residual, contrib and the map
 // are the level's, rows outside the range are neither read as outputs nor written.  Used by the decoder's stage wavefront.
 extern "C" int gpc_spconv_sparse_fwd_rows(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs,
                                           const uint32_t *rowptr, int64_t n, int64_t n_entries, float *contrib,
                                           const float *residual, int flags, float *y, int64_t row0, int64_t row1, void *stream) {
-    return sp_fwd_rows(x, Wa, seg, pairs, rowptr, n, n_entries, contrib, residual, flags, y, row0, row1, stream);
+    return sp_fwd_rows(x, x, Wa, seg, pairs, rowptr, n, n_entries, contrib, residual, flags, y, row0, row1, stream);
+}
+// The conv of one scene of a batch union level: output rows [row0, row1) of a level of n_level rows with the sparse map of that range
+// (gpc_kmap_sparse_count_range): the stragglers gather the level's rows x[nbr], the centre product and the outputs are the range's
+// rows.  x, y and residual are the level's arrays.
+extern "C" int gpc_spconv_sparse_fwd_range(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs,
+                                           const uint32_t *rowptr, int64_t n_level, int64_t row0, int64_t row1, int64_t n_entries,
+                                           float *contrib, const float *residual, int flags, float *y, void *stream) {
+    GPC_RANGE_CHECK(n_level, row0, row1);
+    GPC_REQUIRE(x != y, GPC_EINVAL, "conv is out of place (rows are gathered from x while y is written)");
+    const int64_t n = row1 - row0;
+    return sp_fwd_rows(x, x + row0 * GPC_C, Wa, seg, pairs, rowptr, n, n_entries, contrib, residual ? residual + row0 * GPC_C : nullptr,
+                       flags, y + row0 * GPC_C, 0, n, stream);
 }

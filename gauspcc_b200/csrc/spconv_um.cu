@@ -91,7 +91,7 @@ template <int TM, int NMAX, int GS, int DS, int WS, int NPW, int NEW, int TCOLS,
 __global__ void __launch_bounds__((8 + NEW + (NPW > 3 ? NPW - 3 : 0)) * 32, MINB)
 spconv_um_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_g, const unsigned char *__restrict__ xs, const uint4 *__restrict__ Wp,
                  const u32 *__restrict__ seg_g, const u32 *__restrict__ pair_nbr, const u32 *__restrict__ pair_off, i64 n, i64 tile0,
-                 const u32 *__restrict__ tile_order,
+                 const u32 *__restrict__ tile_order, int xrow0,
                  const void *__restrict__ residual, int flags, float *__restrict__ y, u32 *__restrict__ ys) {
     constexpr int NWARPS = 8 + NEW + (NPW > 3 ? NPW - 3 : 0), NTHREADS = NWARPS * 32;
     constexpr int RS = GS + DS;                  // row-offset ring: a chunk's entries live from its gather to the start of its epilogue
@@ -233,12 +233,14 @@ spconv_um_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant
             UM_T(t2);
             if (k == 62u) {
                 // centre offset: pair p is row (tile start + chunk start + p) itself: one TMA tile load of NMAX consecutive rows
-                // (rows past the end of the level are zero-filled; columns past len are never read)
+                // (rows past the end of the level are zero-filled; columns past len are never read).  xrow0: the launch's first output
+                // row is input row xrow0 (a scene of a union level; rows of the next scene may land in padding columns, whose products
+                // go to the dummy rows)
                 if (elect_one()) {
                     const u32 j = (e >> 8) & 0xFu;
                     asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"((u32)NMAX * 128u) : "memory");
                     asm volatile("cp.async.bulk.tensor.2d.shared::cta.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                                 ::"r"(slot), "l"(reinterpret_cast<u64>(&tmap)), "r"(bar), "r"(0), "r"((int)(t * TM + j * NMAX)) : "memory");
+                                 ::"r"(slot), "l"(reinterpret_cast<u64>(&tmap)), "r"(bar), "r"(0), "r"(xrow0 + (int)(t * TM + j * NMAX)) : "memory");
                 }
             } else {
                 // TMA tile::gather4: four arbitrary rows per instruction, written with the 128 B swizzle; padding entries (row -1) are
@@ -440,7 +442,8 @@ static um_encode_fn um_encoder() {
 
 template <int TM, int NMAX, int GS, int DS, int WS, int NPW, int NEW, int TCOLS, int MINB, bool PROF = false>
 static int launch_spconv_um(const CUtensorMap &tmap, const CUtensorMap &tmap_g, const void *xs, const void *Wp, const u32 *seg, const u32 *pair_nbr, const u32 *pair_off,
-                            i64 n, i64 tile0, i64 tiles, const u32 *tile_order, const void *residual, int flags, float *y, void *ys, cudaStream_t st) {
+                            i64 n, i64 tile0, i64 tiles, const u32 *tile_order, int xrow0, const void *residual, int flags, float *y, void *ys,
+                            cudaStream_t st) {
     static bool configured = false;
     typedef UmSmem<TM, NMAX, GS, DS, WS, NPW> Smem;
     constexpr size_t smem = sizeof(Smem);
@@ -451,7 +454,7 @@ static int launch_spconv_um(const CUtensorMap &tmap, const CUtensorMap &tmap_g, 
         configured = true;
     }
     spconv_um_kernel<TM, NMAX, GS, DS, WS, NPW, NEW, TCOLS, MINB, PROF><<<(unsigned)tiles, NTHREADS, smem, st>>>(
-        tmap, tmap_g, (const unsigned char *)xs, (const uint4 *)Wp, seg, pair_nbr, pair_off, n, tile0, tile_order, residual, flags, y, (u32 *)ys);
+        tmap, tmap_g, (const unsigned char *)xs, (const uint4 *)Wp, seg, pair_nbr, pair_off, n, tile0, tile_order, xrow0, residual, flags, y, (u32 *)ys);
     GPC_LAUNCH_CHECK();
     return GPC_OK;
 }
@@ -459,9 +462,11 @@ static int launch_spconv_um(const CUtensorMap &tmap, const CUtensorMap &tmap_g, 
 // xs = split rows [n][128 B]; Wp = this conv's slice of gpc_spconv_pack_weights_um; seg / pair_nbr = the pair stream built with
 // tile_rows = 512 and pad = 16 (padding entries 0xFFFFFFFF), pair_off (gpc_kmap_um_count / _fill).  Output rows
 // [row0, row1) (whole tiles; row1 <= 0 or >= n: to the end).  y (fp32 rows) and / or ys (split rows).
-extern "C" int gpc_spconv_fwd_um(const void *xs, const void *Wp, const uint32_t *seg, const uint32_t *pair_nbr,
-                                 const uint32_t *pair_off, int64_t n, int tile_rows, const uint32_t *tile_order, const void *residual,
-                                 int flags, float *y, void *ys, int64_t row0, int64_t row1, void *stream) {
+// n_in >= xrow0 + n: rows of xs (the TMA tensor); the launch's output row r reads the centre row xrow0 + r and writes y[r] / ys[r];
+// neighbour indices address all n_in rows.  (n_in = n, xrow0 = 0: a whole level.)
+static int um_fwd(const void *xs, int64_t n_in, int64_t xrow0, const void *Wp, const uint32_t *seg, const uint32_t *pair_nbr,
+                  const uint32_t *pair_off, int64_t n, int tile_rows, const uint32_t *tile_order, const void *residual, int flags, float *y,
+                  void *ys, int64_t row0, int64_t row1, void *stream) {
     const bool prof = (flags & GPC_CONV_PROFILE) != 0;
     flags &= ~GPC_CONV_PROFILE;
     if (n <= 0) return GPC_OK;
@@ -473,8 +478,9 @@ extern "C" int gpc_spconv_fwd_um(const void *xs, const void *Wp, const uint32_t 
     if (row0 >= row1) return GPC_OK;
     um_encode_fn enc = um_encoder();
     GPC_REQUIRE(enc != nullptr, GPC_ECUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    CUtensorMap tmap;                                            // [n rows][64 bf16], box = one chunk of consecutive rows (the centre offset)
-    const cuuint64_t gdim[2] = {64, (cuuint64_t)n};
+    CUtensorMap tmap;                                            // [n_in rows][64 bf16], box = one chunk of consecutive rows (the centre offset)
+    GPC_REQUIRE(n_in >= xrow0 + n && n_in < (1ll << 31), GPC_EINVAL, "input rows must cover the output rows and fit TMA coordinates");
+    const cuuint64_t gdim[2] = {64, (cuuint64_t)n_in};
     const cuuint64_t gstride[1] = {128};
     const cuuint32_t box[2] = {64, 64};                          // 64 rows: NMAX of the launch below
     const cuuint32_t estr[2] = {1, 1};
@@ -491,8 +497,28 @@ extern "C" int gpc_spconv_fwd_um(const void *xs, const void *Wp, const uint32_t 
     cudaStream_t st = as_stream(stream);
     const i64 tile0 = row0 / tile_rows, tiles = (row1 - row0 + tile_rows - 1) / tile_rows;
     const u32 *order = (row0 == 0 && row1 == n) ? tile_order : nullptr;            // a permutation of the level's tiles: full launches only
-    if (prof) return launch_spconv_um<512, 64, 4, 3, 2, 3, 8, 256, 2, true>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
-    return launch_spconv_um<512, 64, 4, 3, 2, 3, 8, 256, 2>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, residual, flags, y, ys, st);
+    const int xr0 = (int)xrow0;
+    if (prof) return launch_spconv_um<512, 64, 4, 3, 2, 3, 8, 256, 2, true>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, xr0, residual, flags, y, ys, st);
+    return launch_spconv_um<512, 64, 4, 3, 2, 3, 8, 256, 2>(tmap, tmap_g, xs, Wp, seg, pair_nbr, pair_off, n, tile0, tiles, order, xr0, residual, flags, y, ys, st);
+}
+extern "C" int gpc_spconv_fwd_um(const void *xs, const void *Wp, const uint32_t *seg, const uint32_t *pair_nbr,
+                                 const uint32_t *pair_off, int64_t n, int tile_rows, const uint32_t *tile_order, const void *residual,
+                                 int flags, float *y, void *ys, int64_t row0, int64_t row1, void *stream) {
+    return um_fwd(xs, n, 0, Wp, seg, pair_nbr, pair_off, n, tile_rows, tile_order, residual, flags, y, ys, row0, row1, stream);
+}
+// The conv of one scene of a batch union level: output rows [row0, row1) of a level of n_level rows, with the pair stream of that
+// range (gpc_kmap_um_count_range / _fill_range).  The TMA descriptors span all n_level rows of xs (out-of-bounds padding entries,
+// 0xFFFFFFFF, still read as zeros); the centre tiles start at row0.  xs, y, ys and residual are the level's arrays; tile_order (may be
+// NULL) is a permutation of the RANGE's tiles.
+extern "C" int gpc_spconv_fwd_um_range(const void *xs, const void *Wp, const uint32_t *seg, const uint32_t *pair_nbr,
+                                       const uint32_t *pair_off, int64_t n_level, int64_t row0, int64_t row1, const uint32_t *tile_order,
+                                       const void *residual, int flags, float *y, void *ys, void *stream) {
+    GPC_RANGE_CHECK(n_level, row0, row1);
+    GPC_REQUIRE(xs != ys && xs != (const void *)y, GPC_EINVAL, "conv is out of place (rows are gathered from xs while y is written)");
+    const int64_t n = row1 - row0;
+    return um_fwd(xs, n_level, row0, Wp, seg, pair_nbr, pair_off, n, 512, tile_order,
+                  residual ? (const void *)((const uint32_t *)residual + row0 * GPC_C) : nullptr, flags, y ? y + row0 * GPC_C : nullptr,
+                  ys ? (void *)((uint32_t *)ys + row0 * GPC_C) : nullptr, 0, n, stream);
 }
 
 // W [n_kernels*125][32 ci][32 co] fp32 -> Wp [n_kernels*125][8 chunks][32 co][4 words]: channel co's TMEM lane is 32 words = 8 chunks of

@@ -15,15 +15,17 @@ from __future__ import annotations
 import ctypes as C
 import os
 import time
-from typing import Dict
+from typing import Dict, List
 
 import numpy as np
 import torch
 
 from . import _lib, bitstream
+from .batch import BatchCodec
 from .codec import GausPcgcCodec, load_weights
 
 _CODECS: Dict[tuple, GausPcgcCodec] = {}
+_BATCH: Dict[int, BatchCodec] = {}
 
 
 def _require_cuda() -> torch.device:
@@ -39,6 +41,20 @@ def _codec(ckpt_path: str, channels: int, kernel_size: int) -> GausPcgcCodec:
     if key not in _CODECS:
         _CODECS[key] = GausPcgcCodec(w, dev)
     return _CODECS[key]
+
+
+def _batch(codec: GausPcgcCodec) -> BatchCodec:
+    """the batch driver over a codec: it follows the codec's kernel-family attributes, so both paths take the same decisions"""
+    if id(codec) not in _BATCH:
+        _BATCH[id(codec)] = BatchCodec(codec)
+    return _BATCH[id(codec)]
+
+
+def _to_device_xyz(xyz_quantized, dev):
+    xyz = torch.tensor(xyz_quantized) if isinstance(xyz_quantized, np.ndarray) else xyz_quantized.detach()
+    if xyz.is_floating_point():
+        return xyz.to(device=dev, dtype=torch.float32)
+    return xyz.to(device=dev, dtype=torch.int32)
 
 
 def calculate_morton_order(x: torch.Tensor) -> torch.Tensor:
@@ -196,3 +212,74 @@ def _save_ply_ascii_geo(coords: np.ndarray, path: str) -> None:
         f.write('property float x\nproperty float y\nproperty float z\nend_header\n')
         for p in coords:
             f.write(f'{p[0]} {p[1]} {p[2]}\n')
+
+
+def compress_point_clouds(xyz_list, ckpt_path, output_paths, channels=32, kernel_size=5, posQ=1) -> List[dict]:
+    """
+    Compress many point clouds in one call (extension, not in the reference): file i is byte-identical to
+    compress_point_cloud(xyz_list[i], ckpt_path, output_paths[i], channels, kernel_size, posQ).
+
+    The scenes are coded together as one union octree (gauspcc_b200/batch.py): one set of launches per level and the range coders
+    of all scenes side by side on the codec's thread pool, instead of one level loop per scene.  Returns one dict per scene with the
+    single call's keys; 'enc_time' and 'gpu_time' are 0.0 there (the scenes are coded together, there is no per-scene time) and
+    'batch_enc_time' is the wall-clock time of the whole batch, the same value in every dict.
+    """
+    xyz_list, output_paths = list(xyz_list), list(output_paths)
+    if len(xyz_list) != len(output_paths):
+        raise ValueError(f"compress_point_clouds: {len(xyz_list)} point clouds but {len(output_paths)} output paths")
+    if not xyz_list:
+        return []
+    codec = _codec(ckpt_path, channels, kernel_size)
+    dev = codec.dev
+    xyzs = [_to_device_xyz(x, dev) for x in xyz_list]
+    for p in output_paths:
+        os.makedirs(os.path.dirname(p), exist_ok=True)
+    torch.cuda.synchronize(dev)
+    t0 = time.time()
+    coded = _batch(codec).encode(xyzs)
+    torch.cuda.synchronize(dev)
+    batch_enc_time = time.time() - t0
+    out = []
+    for xyz, p, (base_xyz, base_occ, streams) in zip(xyzs, output_paths, coded):
+        with open(p, 'wb') as f:
+            f.write(bitstream.write_file(posQ, base_xyz, base_occ, streams))
+        N = xyz.shape[0]
+        bits = os.stat(p).st_size * 8
+        out.append({'bpp': bits / N, 'enc_time': 0.0, 'file_size_bits': bits, 'num_points': N, 'output_path': p, 'gpu_time': 0.0,
+                    'batch_enc_time': batch_enc_time})
+    return out
+
+
+def decompress_point_clouds(bin_paths, ckpt_path, channels=32, kernel_size=5, is_data_pre_quantized=True,
+                            sorted_output=False) -> List[dict]:
+    """
+    Decompress many files in one call (extension): result i's 'point_cloud' equals
+    decompress_point_cloud(bin_paths[i], ckpt_path, ...)['point_cloud'] row for row, in both row orders.  Container version 2 files
+    are not accepted here (ValueError naming the file).  'dec_time' and 'gpu_time' are 0.0; 'batch_dec_time' is the wall-clock time
+    of the whole batch, the same value in every dict.  No PLY output.
+    """
+    bin_paths = list(bin_paths)
+    if not bin_paths:
+        return []
+    codec = _codec(ckpt_path, channels, kernel_size)
+    dev = codec.dev
+    files = []
+    for p in bin_paths:
+        with open(p, 'rb') as f:
+            blob = f.read()
+        try:
+            posQ, base_xyz, base_occ, streams = bitstream.read_file(blob)
+        except ValueError as e:
+            raise ValueError(f"{p}: {e}") from e
+        if bitstream.split_v2(streams)[1]:
+            raise ValueError(f"{p}: container version 2 files cannot be decoded in a batch; use decompress_point_cloud")
+        files.append((float(posQ), base_xyz, base_occ, streams))
+    torch.cuda.synchronize(dev)
+    t0 = time.time()
+    scans = _batch(codec).decode(files, sorted_rows=bool(sorted_output))
+    if not is_data_pre_quantized:
+        scans = [(s - 131072) * 0.001 for s in scans]             # pcc_utils.py:381
+    torch.cuda.synchronize(dev)
+    batch_dec_time = time.time() - t0
+    return [{'dec_time': 0.0, 'num_points': s.shape[0], 'point_cloud': s, 'output_path': None, 'gpu_time': 0.0,
+             'batch_dec_time': batch_dec_time} for s in scans]

@@ -132,6 +132,14 @@ int gpc_kmap_pairs_count(const int32_t *map, int64_t n, int tile_rows, int pad, 
  * pairs[p] = nbr | row_in_tile << 32 | k << 48 (may be NULL) consumed by gpc_spconv_fwd_v6 */
 int gpc_kmap_pairs_fill(const int32_t *map, int64_t n, int tile_rows, const uint32_t *seg,
                         uint32_t *pair_nbr, uint16_t *pair_row, uint64_t *pairs, int64_t n_entries, void *stream);
+/* ---- row ranges of a level (a batch of scenes coded as one union level, pcc_utils.compress_point_clouds): the pair streams of the
+ * output rows [row0, row1) of a level of n_level rows whose dense map has leading dimension n_level.  Tiles / blocks start at row0,
+ * neighbour indices stay the level's rows, totals are the range's own; seg, rowptr and workspaces are sized for row1 - row0 rows.
+ * The streams are exactly those of the range's rows coded as a level of their own, with neighbour indices + row0. */
+int gpc_kmap_pairs_count_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, int tile_rows, int pad,
+                               uint32_t *seg, uint32_t *n_pairs, void *ws, size_t ws_bytes, void *stream);
+int gpc_kmap_pairs_fill_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, int tile_rows,
+                              const uint32_t *seg, uint64_t *pairs, int64_t n_entries, void *stream);
 
 /* ---- a-7/a-10/a-12: sparse conv (spnn.Conv3d(32,32,5), bias-less) ---- */
 /* y[o,:] = act( sum_k x[nbr_k(o),:] . W[k] (+ residual[o,:]) ); W [125,32,32] fp32;
@@ -154,6 +162,11 @@ int gpc_spconv_fwd_v6(const float *x, const void *Wa, const uint32_t *seg, const
 int gpc_spconv_fwd_v6_rows(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs,
                            int64_t n, int tile_rows, const float *residual, int flags, float *y, int variant,
                            int64_t row0, int64_t row1, void *stream);
+/* gpc_spconv_fwd_v6 for the output rows [row0, row1) of a level of n_level rows with the range's own pair stream
+ * (gpc_kmap_pairs_count_range): x, y and residual are the level's arrays, the tiling starts at row0 */
+int gpc_spconv_fwd_v6_range(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs, int64_t n_level,
+                            int64_t row0, int64_t row1, int tile_rows, const float *residual, int flags, float *y,
+                            int variant, void *stream);
 
 /* ---- the conv of the SPARSE big levels (spconv_sparse.cu): dense centre product + offset-sorted "stragglers" ----
  * For levels with ~1-4 neighbours per row (the finest octree levels).  Sparse map: seg u32[gpc_kmap_sparse_segments(n) + 1]
@@ -175,6 +188,15 @@ int gpc_spconv_sparse_fwd(const float *x, const void *Wa, const uint32_t *seg, c
 int gpc_spconv_sparse_fwd_rows(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs, const uint32_t *rowptr,
                                int64_t n, int64_t n_entries, float *contrib, const float *residual, int flags, float *y,
                                int64_t row0, int64_t row1, void *stream);
+/* row ranges (see gpc_kmap_pairs_count_range): the sparse map of the rows [row0, row1), and the conv of those rows over the level's
+ * arrays (stragglers gather the level's rows; the centre product and outputs are the range's rows) */
+int gpc_kmap_sparse_count_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, uint32_t *seg, uint32_t *rowptr,
+                                uint32_t *totals, void *ws, size_t ws_bytes, void *stream);
+int gpc_kmap_sparse_fill_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, const uint32_t *seg,
+                               const uint32_t *rowptr, const void *ws, uint64_t *pairs, int64_t n_entries, void *stream);
+int gpc_spconv_sparse_fwd_range(const float *x, const void *Wa, const uint32_t *seg, const uint64_t *pairs, const uint32_t *rowptr,
+                                int64_t n_level, int64_t row0, int64_t row1, int64_t n_entries, float *contrib, const float *residual,
+                                int flags, float *y, void *stream);
 
 /* ---- split rows (spconv_fmt.cu): an activation row stored as 32 x bf16 hi | 32 x bf16 lo (128 B, x = hi + lo to 16 mantissa bits):
  * a gathered row is a tensor-core operand row as it stands */
@@ -211,6 +233,15 @@ int gpc_kmap_um_fill(const int32_t *map, int64_t n, int tile_rows, const uint32_
 int gpc_spconv_fwd_um(const void *xs, const void *Wp, const uint32_t *seg, const uint32_t *pair_nbr, const uint32_t *pair_off,
                       int64_t n, int tile_rows, const uint32_t *tile_order, const void *residual, int flags, float *y, void *ys,
                       int64_t row0, int64_t row1, void *stream);
+/* row ranges (see gpc_kmap_pairs_count_range; tile_rows 512): the pair stream of the rows [row0, row1), and the conv of those rows
+ * over the level's arrays.  The TMA descriptors span all n_level rows of xs; tile_order (may be NULL) permutes the range's tiles. */
+int gpc_kmap_um_count_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, int tile_rows, uint32_t *seg,
+                            unsigned long long *totals, void *ws, size_t ws_bytes, void *stream);
+int gpc_kmap_um_fill_range(const int32_t *map, int64_t n_level, int64_t row0, int64_t row1, int tile_rows, const uint32_t *seg,
+                           uint32_t *pair_nbr, uint32_t *pair_off, void *stream);
+int gpc_spconv_fwd_um_range(const void *xs, const void *Wp, const uint32_t *seg, const uint32_t *pair_nbr, const uint32_t *pair_off,
+                            int64_t n_level, int64_t row0, int64_t row1, const uint32_t *tile_order, const void *residual, int flags,
+                            float *y, void *ys, void *stream);
 
 /* ---- a-6/a-9/a-12: embeddings ---- */
 /* Every producer of conv inputs writes fp32 rows (out), split rows (out_split: 32 x bf16 hi | 32 x bf16 lo, the operand format of
