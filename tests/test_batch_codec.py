@@ -184,3 +184,35 @@ def test_batch_decode_issues_fewer_launches(ckpt, tmp_path):
     pcc_utils.decompress_point_clouds(paths, ckpt)
     batch = pcc_utils._batch(codec).last_stats["launches"]
     assert batch < single, (batch, single)
+
+
+def test_production_size_default_families(ckpt, tmp_path):
+    """scenes of 400 K, 250 K and 160 K anchors under the default family thresholds: one union level has members on the sparse and on
+    the tcgen05 conv (recorded from BatchCodec._kmaps, so that the test keeps meaning it); files and decoded rows as the single path"""
+    from gauspcc_b200 import pcc_utils
+    from gauspcc_b200.synth import hac_like_cloud
+    codec = pcc_utils._codec(ckpt, 32, 5)
+    assert (codec.um_min_rows, codec.sparse_min_rows, codec.sparse_max_density) == (150_000, 150_000, 4.5)
+    bc = pcc_utils._batch(codec)
+    xyzs = [hac_like_cloud(n, seed=61 + i, extent_log2=16) for i, n in enumerate((400_000, 250_000, 160_000))]
+    single = _single(xyzs, ckpt, str(tmp_path))
+    levels = []
+    kmaps = bc._kmaps
+
+    def record(lv):
+        kms = kmaps(lv)
+        levels.append(["um" if k.um_rows else ("sparse" if k.sparse else "v6") for k in kms])
+        return kms
+    bc._kmaps = record
+    try:
+        paths, _ = _batch(xyzs, ckpt, str(tmp_path))
+        assert bc.last_stats["unions"] == 1
+        assert any("sparse" in f and "um" in f for f in levels), levels
+        levels.clear()
+        dec = pcc_utils.decompress_point_clouds(paths, ckpt)
+        assert any("sparse" in f and "um" in f for f in levels), levels
+    finally:
+        del bc._kmaps
+    _same_bytes(single, paths)
+    for p, d in zip(single, dec):
+        assert torch.equal(d["point_cloud"], pcc_utils.decompress_point_cloud(p, ckpt)["point_cloud"]), p
