@@ -81,8 +81,11 @@ __host__ __device__ __forceinline__ u64 key_compact(u64 k, gpc_key_xform t) {
 }
 
 // ---------------------------------------------------------------- bf16 hi / lo split of fp32 (x = hi + lo + O(2^-17 x))
-__device__ __forceinline__ float bf16_round(float v) {                       // round-to-nearest-even to bf16, as fp32
+// round-to-nearest-even to bf16, as fp32.  NaN gives the canonical bf16 NaN, as cvt.rn.bf16x2 does: the integer rounding would carry
+// the all-ones NaN mantissa into the sign bit (-0.0) and truncate a NaN whose payload lies in the low 16 bits to inf.
+__device__ __forceinline__ float bf16_round(float v) {
     u32 u = __float_as_uint(v);
+    if ((u & 0x7FFFFFFFu) > 0x7F800000u) return __uint_as_float(0x7FFF0000u);
     u += 0x7FFFu + ((u >> 16) & 1u);
     return __uint_as_float(u & 0xFFFF0000u);
 }
