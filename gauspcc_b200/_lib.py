@@ -105,6 +105,7 @@ SIGNATURES = {
     "gpc_chunk_encode_lohi": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "gpc_chunk_merge": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_vp]),
     "gpc_chunk_decode_u16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_vp, c_vp]),
+    "gpc_chunk_decode_u16_ranges": (c_int, [c_vp, c_int, c_vp, c_vp, c_vp, c_int, c_i64, c_vp, c_vp]),
     "gpc_attr_decode_gaussian": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
 }
 

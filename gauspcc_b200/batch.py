@@ -15,6 +15,13 @@ D2H and one H2D copy per stage.  What stays per scene: the conv family and its t
 pairs, _v6_config on its own row count), run by the *_range kernels (csrc/kmap.cu, spconv.cu, spconv_sparse.cu, spconv_um.cu) whose
 tiles start at r0_s while neighbour indices address the whole level -- so every row is summed exactly as in the scene's own level --
 and the range coder streams, coded on the codec's thread pool, one task per (scene, stage).
+
+Container version 2 (files of compress_point_cloud(..., gpu_coder_chunk=c)): a version-2 stream is cut into chunks by a rule on
+that stream's own row count (GausPcgcCodec.chunk_len), and a scene's rows of a union level are its own level's rows, so the streams
+of all members are coded side by side on the GPU.  Encode: the head kernels write every (scene, level, stage) stream's words into
+one arena, a union level's stage as one contiguous slot, and one chunk-coder launch codes all chunks at the end.  Decode: per union
+level one H2D copy of the four stages' chunk tables and payloads (v2_stage_tables), then per stage the head, one chunk decoder
+launch over all members' rows and the symbol merge -- no CDF row leaves the GPU and no host coder runs.
 """
 from __future__ import annotations
 
@@ -24,10 +31,43 @@ from typing import List, Optional, Sequence, Tuple
 import numpy as np
 import torch
 
+from . import bitstream
 from . import weights as W
 from .codec import COORD_LIMIT, CTX_SHIFT, STAGE_SHIFT, UM_TILE_ROWS, GausPcgcCodec, KMap, Level, _ptr
 
 Z_SHIFT = 42                      # z field of a voxel key (include/gpcgc.h)
+
+
+def v2_stage_tables(streams: Sequence[Tuple[str, int, int, bytes]], row0: int = 0) -> Tuple[np.ndarray, np.ndarray, bytes]:
+    """The chunk tables of one stage of a union level for gpc_chunk_decode_u16_ranges.  streams: per member scene, in union row
+    order, (name, rows n at this level, the file's chunk size, its version-2 stream of this level and stage); the members' rows
+    follow one another from row0.  Returns
+      rows    u32[chunks + 1]  chunk boundaries: every member's rows cut by chunk_len(n, its chunk size), offset by its first row
+      offsets u32[chunks + 1]  prefix sums of the chunks' u16 byte counts
+      payload                  the members' chunk bytes without their u16 count headers, one after the other.
+    A stream shorter than its count header, or whose counts do not sum to its length, raises ValueError naming the scene."""
+    rows = [np.array([row0], dtype=np.int64)]
+    cnts = [np.zeros(1, dtype=np.int64)]
+    payload = []
+    r = int(row0)
+    for name, n, chunk, sb in streams:
+        n = int(n)
+        cl = GausPcgcCodec.chunk_len(n, int(chunk))
+        chunks = (n + cl - 1) // cl
+        if len(sb) < 2 * chunks:
+            raise ValueError(f"{name}: truncated version-2 stream")
+        cnt = np.frombuffer(sb, dtype="<u2", count=chunks).astype(np.int64)
+        if int(cnt.sum()) != len(sb) - 2 * chunks:
+            raise ValueError(f"{name}: corrupt version-2 stream (chunk byte counts)")
+        rows.append(r + np.minimum(np.arange(1, chunks + 1, dtype=np.int64) * cl, n))
+        cnts.append(cnt)
+        payload.append(memoryview(sb)[2 * chunks:])
+        r += n
+    rows_a = np.concatenate(rows)
+    offs = np.cumsum(np.concatenate(cnts))
+    if int(rows_a[-1]) > 0xFFFFFFFF or int(offs[-1]) > 0xFFFFFFFF:
+        raise ValueError("a union level's version-2 chunk table exceeds u32 rows or bytes")
+    return rows_a.astype(np.uint32), offs.astype(np.uint32), b"".join(payload)
 
 
 # ---------------------------------------------------------------------------------------------------------------- planner
@@ -119,6 +159,9 @@ class _Scene:
     streams: Optional[List[bytes]] = None
     scale: float = 1.0
     tz: int = 0
+    n_unique: int = 0                             # encoder: distinct voxels (the version-2 trailer's count)
+    chunk: int = 0                                # decoder: the file's version-2 chunk size (0: version 1)
+    name: str = ""                                # decoder: how errors name the scene
 
 
 class BatchCodec:
@@ -131,6 +174,7 @@ class BatchCodec:
         # within ~70 GB.
         self.max_rows = 32_000_000
         self.last_stats: dict = {}
+        self._v2_pin: Optional[torch.Tensor] = None   # decoder: pinned staging of a union level's version-2 chunk tables
 
     # ------------------------------------------------------------------ kernel maps of the scenes of a level
     def _kmaps(self, lv: ULevel) -> List[KMap]:
@@ -334,10 +378,15 @@ class BatchCodec:
         return keys + (dz << Z_SHIFT) if dz else keys
 
     # ------------------------------------------------------------------ encode
-    def encode(self, xyz_list: List[torch.Tensor]) -> List[Tuple[np.ndarray, np.ndarray, List[bytes]]]:
-        """-> per scene (base_xyz, base_occ, streams), exactly GausPcgcCodec.encode's for that scene alone"""
+    def encode(self, xyz_list: List[torch.Tensor], gpu_chunk: int = 0) -> List[Tuple[np.ndarray, np.ndarray, List[bytes]]]:
+        """-> per scene (base_xyz, base_occ, streams), exactly GausPcgcCodec.encode's for that scene alone.  gpu_chunk > 0: container
+        version 2 -- the streams are compress_point_cloud(..., gpu_coder_chunk=gpu_chunk)'s, its trailer (bitstream.v2_trailer)
+        included"""
         c = self.c
         results: List[Optional[tuple]] = [None] * len(xyz_list)
+
+        def trail(streams: List[bytes], n_unique: int) -> List[bytes]:
+            return streams + [bitstream.v2_trailer(gpu_chunk, n_unique)] if gpu_chunk else streams
         n_unions = 0
         self._begin()
         try:
@@ -355,6 +404,7 @@ class BatchCodec:
                     meta_h = meta.cpu().numpy()
                 mm = meta_h[2:8].astype(np.uint32)
                 leaf = c.sort_unique(keys, mm)
+                sc.n_unique = int(leaf.shape[0])
                 sc.levels = c.build_pyramid(leaf, mm.astype(np.int64))
                 sc.depth = len(sc.levels)                     # the base voxels are 2^depth leaves wide
                 sc.zr = (int(mm[2]) - (1 << 20), int(mm[5]) - (1 << 20))
@@ -364,18 +414,18 @@ class BatchCodec:
                                           [sc.levels[-1].n for sc in multi], self.max_rows)
             for sc in scenes:
                 if sc.depth < 2:
-                    results[sc.idx] = self._finish_base(sc, [])
+                    results[sc.idx] = self._finish_base(sc, trail([], sc.n_unique))
             for j in singles:                              # a scene that fits no union: the single-scene path
                 sc = multi[j]
-                bx, bo, streams, _ = c.encode(xyz_list[sc.idx])
+                bx, bo, streams, _ = c.encode(xyz_list[sc.idx], gpu_chunk=gpu_chunk)
                 self._begin_again()
-                results[sc.idx] = (bx, bo, streams)
+                results[sc.idx] = (bx, bo, trail(streams, c.last_stats["n_unique"]))
             for up in unions:
                 members = [multi[j] for j in up.scenes]
                 for sc, t in zip(members, up.tz):
                     sc.tz = t
-                for sc, streams in zip(members, self._encode_union(members)):
-                    results[sc.idx] = self._finish_base(sc, streams)
+                for sc, streams in zip(members, self._encode_union(members, gpu_chunk)):
+                    results[sc.idx] = self._finish_base(sc, trail(streams, sc.n_unique))
             n_unions = len(unions)
         finally:
             self._end(unions=n_unions)
@@ -401,7 +451,7 @@ class BatchCodec:
             base_xyz_h = moved.astype(np.int32)
         return base_xyz_h, base.occ.cpu().numpy(), streams
 
-    def _encode_union(self, members: List[_Scene]) -> List[List[bytes]]:
+    def _encode_union(self, members: List[_Scene], gpu_chunk: int = 0) -> List[List[bytes]]:
         c = self.c
         D = max(sc.depth for sc in members)
         # U[sigma]: the members' levels at scale sigma (1 = parents of the leaves), translated; deepest scenes first = a prefix
@@ -423,7 +473,18 @@ class BatchCodec:
         futs = []
         K = {sg: sum(1 for sc in members if sc.depth >= sg + 1) for sg in range(1, D)}     # members with children at scale sg
         M = {sg: U[sg].ranges[K[sg] - 1][1] for sg in range(1, D)}                         # = the first M rows of U[sg]
-        pin = c._pin(sum(M.values()) * 16 + 4096 * 4 * D)
+        if gpu_chunk:
+            # version 2: the (scene, level, stage) streams in the order (union level, stage, member) in the codec's coder arena, so
+            # that the words of one stage of a union level (its first M rows, member after member) are one contiguous slot
+            first = {}
+            seg_rows: List[int] = []
+            for sg in range(1, D):
+                for i in range(4):
+                    first[sg, i] = len(seg_rows)
+                    seg_rows += [r1 - r0 for r0, r1 in U[sg].ranges[:K[sg]]]
+            c._chunk_begin(seg_rows, gpu_chunk)
+        else:
+            pin = c._pin(sum(M.values()) * 16 + 4096 * 4 * D)
         cursor = 0
         for sg in range(1, D):                              # finest first: its range coding overlaps the coarser levels' GPU work
             parent, child = U[sg + 1], U[sg]
@@ -434,15 +495,23 @@ class BatchCodec:
             hosts = []
             for i in range(4):
                 t = self._stage(u, occ, i, child, m, k)
-                lohi_d = c._empty((m,), torch.int32)
+                if gpu_chunk:
+                    a = c._coder_starts[first[sg, i]]
+                    lohi_d = c._coder_arena[a:a + m]
+                else:
+                    lohi_d = c._empty((m,), torch.int32)
                 w1, b1, w2, b2 = c.w.head[i]
                 c._call("gpc_head_cdf_sym", _ptr(t), m, _ptr(w1), _ptr(b1), _ptr(w2), _ptr(b2), W.STAGE_ALPHABETS[i], _ptr(occ),
                         STAGE_SHIFT[i], _ptr(lohi_d), None, None, c._stream())
+                if gpu_chunk:
+                    continue                               # coded with every other stream of the union at the end
                 start = (cursor + 63) // 64 * 64
                 cursor = start + m * 4
                 h = pin[start:start + m * 4].view(torch.int32)
                 h.copy_(lohi_d, non_blocking=True)
                 hosts.append(h)
+            if gpu_chunk:
+                continue
             ready = torch.cuda.Event(blocking=True)
             ready.record(torch.cuda.current_stream(c.dev))
             for j in range(k):
@@ -452,23 +521,37 @@ class BatchCodec:
                 for i in range(4):
                     futs.append((child.members[j], 4 * g + i,
                                  c.pool.submit(c._ac_encode_lohi, hosts[i].numpy()[r0:r1].view(np.uint32), ready)))
+        if gpu_chunk:
+            coded = c._chunk_finish(gpu_chunk)             # one launch codes every chunk of every scene's streams
+            for sg in range(1, D):
+                child = U[sg]
+                for i in range(4):
+                    for j in range(K[sg]):
+                        sc = members[child.members[j]]
+                        streams[child.members[j]][4 * (sc.depth - 1 - sg) + i] = coded[first[sg, i] + j]
         for j, q, f in futs:
             streams[j][q] = f.result()
         return streams
 
     # ------------------------------------------------------------------ decode
-    def decode(self, files: List[Tuple[float, np.ndarray, np.ndarray, List[bytes]]], sorted_rows: bool = False) -> List[torch.Tensor]:
-        """files: per scene (posQ, base_xyz, base_occ, streams) of container version 1 -> per scene GausPcgcCodec.decode's rows"""
+    def decode(self, files: List[tuple], sorted_rows: bool = False, names: Optional[Sequence[str]] = None) -> List[torch.Tensor]:
+        """files: per scene (posQ, base_xyz, base_occ, streams) of container version 1, or (posQ, base_xyz, base_occ, streams, chunk)
+        with the streams of a version-2 file (trailer removed, bitstream.split_v2) and its chunk size; all files of one call are of
+        one container version.  -> per scene GausPcgcCodec.decode's rows.  names: how errors name the scenes (default "scene i")."""
         c = self.c
         out: List[Optional[torch.Tensor]] = [None] * len(files)
+        chunks = [int(f[4]) if len(f) > 4 else 0 for f in files]
+        if any(chunks) and not all(chunks):
+            raise ValueError("container version 1 and version 2 files cannot be decoded in one call")
         self._begin()
         n_unions = 0
+        self._round_trips = 0
         try:
             scenes = []
-            for s, (posQ, bx, bo, streams) in enumerate(files):
+            for s, (posQ, bx, bo, streams) in enumerate(f[:4] for f in files):
                 if len(streams) % 4:
                     raise ValueError("stream count must be a multiple of 4 (one group per octree level)")
-                sc = _Scene(s, streams=streams, scale=float(posQ))
+                sc = _Scene(s, streams=streams, scale=float(posQ), chunk=chunks[s], name=names[s] if names else f"scene {s}")
                 sc.depth = L = len(streams) // 4 + 1
                 bx_h = np.array(bx, dtype=np.int32).reshape(-1, 3)
                 sc.base_occ = np.array(bo, dtype=np.uint8).reshape(-1)
@@ -493,10 +576,10 @@ class BatchCodec:
                     zhi.append(((int(b[:, 2].max()) + 1) << sc.depth) - 1)
                     est.append(sum(len(x) for x in sc.streams))
                 else:
-                    out[sc.idx] = self._single_decode(files[sc.idx], sorted_rows)
+                    out[sc.idx] = self._single_decode(files[sc.idx], sorted_rows, sc.name)
             unions, singles = plan_unions(zlo, zhi, [sc.depth for sc in multi], est, self.max_rows)
             for j in singles:
-                out[multi[j].idx] = self._single_decode(files[multi[j].idx], sorted_rows)
+                out[multi[j].idx] = self._single_decode(files[multi[j].idx], sorted_rows, multi[j].name)
             for up in unions:
                 members = [multi[j] for j in up.scenes]
                 for sc, t in zip(members, up.tz):
@@ -505,13 +588,22 @@ class BatchCodec:
                     out[sc.idx] = rows
             n_unions = len(unions)
         finally:
-            self._end(unions=n_unions)
+            # stage_round_trips: how often the union decoder waited for a stage's CDF rows on the host (version 1: four per union
+            # level; version 2 decodes on the GPU: none).  Child counts and kernel-map sizes are read back either way.
+            self._end(unions=n_unions, stage_round_trips=self._round_trips)
         return out
 
-    def _single_decode(self, f, sorted_rows: bool) -> torch.Tensor:
-        posQ, bx, bo, streams = f
-        rows = self.c.decode(bx, bo, streams, scale=float(posQ), sorted_rows=sorted_rows)
-        self._begin_again()
+    def _single_decode(self, f, sorted_rows: bool, name: str) -> torch.Tensor:
+        posQ, bx, bo, streams = f[:4]
+        chunk = int(f[4]) if len(f) > 4 else 0
+        try:
+            rows = self.c.decode(bx, bo, streams, scale=float(posQ), sorted_rows=sorted_rows, gpu_chunk=chunk)
+        except ValueError as e:
+            if not chunk:
+                raise
+            raise ValueError(f"{name}: {e}") from e                # a corrupt version-2 stream, named as the union decoder names it
+        finally:
+            self._begin_again()
         return rows
 
     def _base_level(self, sc: _Scene) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -533,6 +625,33 @@ class BatchCodec:
         ends = torch.tensor([r1 - 1 for _, r1 in lv.ranges], dtype=torch.int64, device=c.dev)
         e = cum[ends].tolist()
         return [int(a - b) for a, b in zip(e, [0] + e[:-1])]
+
+    def _v2_upload(self, tabs: List[Tuple[np.ndarray, np.ndarray, bytes]]) -> Tuple[torch.Tensor, List[tuple]]:
+        """the four stages' chunk tables and payloads of a union level -> device, in ONE copy from pinned staging.  Returns the
+        device buffer (the caller keeps it until the level's decoder launches are enqueued) and per stage the device addresses
+        (payload, offsets, rows) and its chunk count for gpc_chunk_decode_u16_ranges.
+
+        The staging buffer is rewritten once per level.  That is safe because the decoder calls this right after _counts, whose
+        read-back synchronises the stream: the previous level's copy out of this buffer has completed by then."""
+        c = self.c
+        place, total = [], 0
+        for rows, offs, payload in tabs:
+            p = []
+            for nbytes in (len(payload), offs.nbytes, rows.nbytes):
+                p.append(total)
+                total = (total + nbytes + 15) // 16 * 16
+            place.append(p)
+        if self._v2_pin is None or self._v2_pin.numel() < total:
+            self._v2_pin = torch.empty(int(total * 1.5) + 4096, dtype=torch.uint8, pin_memory=True)
+        host = self._v2_pin.numpy()
+        for (rows, offs, payload), (a, b, r) in zip(tabs, place):
+            host[a:a + len(payload)] = np.frombuffer(payload, dtype=np.uint8)
+            host[b:b + offs.nbytes] = offs.view(np.uint8)
+            host[r:r + rows.nbytes] = rows.view(np.uint8)
+        dev = c._empty((max(total, 16),), torch.uint8)
+        dev[:total].copy_(self._v2_pin[:total], non_blocking=True)
+        base = dev.data_ptr()
+        return dev, [(base + a, base + b, base + r, int(rows.shape[0]) - 1) for (rows, _, _), (a, b, r) in zip(tabs, place)]
 
     def _decode_union(self, members: List[_Scene], sorted_rows: bool) -> List[torch.Tensor]:
         c = self.c
@@ -556,10 +675,17 @@ class BatchCodec:
         cur = with_bases(None, None, [], [], D)
         cur.kmaps = self._kmaps(cur)
         Lps = [a + 1 for a in W.STAGE_ALPHABETS]
+        v2 = members[0].chunk > 0                            # decode() admits one container version per call
         for sg in range(D - 1, 0, -1):
-            cnt = self._counts(cur)
+            cnt = self._counts(cur)                          # synchronises the stream: see _v2_upload
             m = sum(cnt)
             k = len(cur.ranges)
+            if v2:
+                # every member of cur has children; their rows of the child level follow one another from 0.  v2_dev holds the
+                # uploaded tables until the next level replaces it, after the stream has passed this level's decoder launches
+                own = [members[j] for j in cur.members]
+                v2_dev, tabs = self._v2_upload([v2_stage_tables([(sc.name, n_, sc.chunk, sc.streams[4 * (sc.depth - 1 - sg) + i])
+                                                                 for sc, n_ in zip(own, cnt)]) for i in range(4)])
             ck, cp = c.expand(cur, m)
             ranges, r = [], 0
             for n_ in cnt:
@@ -569,6 +695,20 @@ class BatchCodec:
             child.kmaps = self._kmaps(child)
             u = self._level_features(cur, child, m, k, ck, cp)
             occ = torch.zeros(m, dtype=torch.uint8, device=c.dev)
+            if v2:
+                for i in range(4):
+                    t = self._stage(u, occ, i, child, m, k)
+                    cdf_d = c._empty((m, Lps[i]), torch.int16)
+                    w1, b1, w2, b2 = c.w.head[i]
+                    c._call("gpc_head_cdf", _ptr(t), m, _ptr(w1), _ptr(b1), _ptr(w2), _ptr(b2), W.STAGE_ALPHABETS[i], _ptr(cdf_d), None,
+                            c._stream())
+                    sym_d = c._empty((m,), torch.uint8)
+                    in_p, offs_p, rows_p, n_chunks = tabs[i]
+                    c._call("gpc_chunk_decode_u16_ranges", _ptr(cdf_d), Lps[i], in_p, offs_p, rows_p, n_chunks, m, _ptr(sym_d), c._stream())
+                    c._call("gpc_merge_symbol", _ptr(occ), m, STAGE_SHIFT[i], _ptr(sym_d), c._stream())
+                child.occ = torch.cat([occ] + [bases[j][1] for j in child.members[k:]]) if child.n > m else occ
+                cur = child
+                continue
             if c._pinned_dec is None or c._pinned_dec.numel() < m * 40:
                 c._pinned_dec = torch.empty(int(m * 40 * 1.5) + 4096, dtype=torch.uint8, pin_memory=True)
             pin = c._pinned_dec
@@ -581,6 +721,7 @@ class BatchCodec:
                 cdf_h = pin[:m * Lps[i] * 2].view(torch.int16).view(m, Lps[i])
                 cdf_h.copy_(cdf_d, non_blocking=True)
                 torch.cuda.current_stream(c.dev).synchronize()
+                self._round_trips += 1
                 sym_h = pin[m * 36:m * 37]
                 cdf_np, sym_np = cdf_h.numpy().view(np.uint16), sym_h.numpy()
                 jobs = []

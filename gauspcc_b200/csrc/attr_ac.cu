@@ -616,18 +616,31 @@ extern "C" int gpc_chunk_merge(const void *ws, int chunks, int max_chunk, const 
 // Decoder of the geometry streams: alphabets of 2 / 2 / 4 / 16 symbols, so a whole CDF row (Lp <= 32 entries) is ONE coalesced load,
 // lane m holding entry m, and the symbol is a ballot.  The rows do not depend on the decoded symbols: the row of symbol i + 1 is
 // requested before symbol i is decoded, which takes the load latency off the serial chain.
-template <int UNUSED = 0>
+// RANGES = false: chunk w is rows [w * chunk_size, min((w + 1) * chunk_size, n)) (one stream).  RANGES = true: chunk w is rows
+// [rows[w], rows[w + 1]) (many streams of their own chunk lengths side by side), clamped to [0, n) and to a non-negative byte
+// length whatever the table holds.
+template <bool RANGES>
 __global__ void __launch_bounds__(128) chunk_decode_u16_kernel(const u16 *__restrict__ cdf, int Lp, const u8 *__restrict__ in,
-                                                              const u32 *__restrict__ offsets, i64 n, int chunk_size, int chunks,
-                                                              u8 *__restrict__ out) {
+                                                              const u32 *__restrict__ offsets, const u32 *__restrict__ rows, i64 n,
+                                                              int chunk_size, int chunks, u8 *__restrict__ out) {
     const int lane = threadIdx.x & 31;
     const int w = blockIdx.x * 4 + (threadIdx.x >> 5);
     if (w >= chunks) return;
-    const i64 base = (i64)w * chunk_size;
-    const int len = (int)min((i64)chunk_size, n - base);
+    i64 base;
+    int len;
+    u32 o0 = offsets[w], o1 = offsets[w + 1];
+    if constexpr (RANGES) {
+        base = min((i64)rows[w], n);
+        len = (int)(min(max((i64)rows[w + 1], base), n) - base);
+        if (len == 0) return;                                                       // the whole warp: w is warp-uniform
+        o1 = max(o1, o0);
+    } else {
+        base = (i64)w * chunk_size;
+        len = (int)min((i64)chunk_size, n - base);
+    }
     const int max_symbol = Lp - 2;
     BitReader br;
-    br.init(in + offsets[w], (i64)(offsets[w + 1] - offsets[w]), lane);
+    br.init(in + o0, (i64)(o1 - o0), lane);
     u32 low = 0u, high = 0xFFFFFFFFu;
     u32 value = br.get(32, lane);
     const u16 *row = cdf + base * Lp;
@@ -680,7 +693,23 @@ extern "C" int gpc_chunk_decode_u16(const uint16_t *cdf, const uint8_t *in, cons
     GPC_REQUIRE(Lp <= 32, GPC_EINVAL, "a CDF row must fit one warp load (Lp <= 32)");
     if (n == 0) return GPC_OK;
     const int chunks = (int)((n + chunk_size - 1) / chunk_size);
-    chunk_decode_u16_kernel<0><<<cdiv(chunks, 4), 128, 0, as_stream(stream)>>>(cdf, Lp, in, offsets, n, chunk_size, chunks, sym);
+    chunk_decode_u16_kernel<false><<<cdiv(chunks, 4), 128, 0, as_stream(stream)>>>(cdf, Lp, in, offsets, nullptr, n, chunk_size, chunks,
+                                                                                  sym);
+    GPC_LAUNCH_CHECK();
+    return GPC_OK;
+}
+
+// many streams in one launch (the member scenes of a union level, each stream cut by its own chunk length): chunk w decodes rows
+// [rows[w], rows[w + 1]) of cdf / sym from bytes [offsets[w], offsets[w + 1]) of `in`
+extern "C" int gpc_chunk_decode_u16_ranges(const uint16_t *cdf, int Lp, const uint8_t *in, const uint32_t *offsets, const uint32_t *rows,
+                                           int chunks, int64_t n, uint8_t *sym, void *stream) {
+    int rc = attr_check(n, Lp, 1);
+    if (rc) return rc;
+    GPC_REQUIRE(Lp <= 32, GPC_EINVAL, "a CDF row must fit one warp load (Lp <= 32)");
+    GPC_REQUIRE(chunks >= 0, GPC_EINVAL, "chunks out of range");
+    if (n == 0 || chunks == 0) return GPC_OK;
+    GPC_REQUIRE(cdf && in && offsets && rows && sym, GPC_EINVAL, "null pointer");
+    chunk_decode_u16_kernel<true><<<cdiv(chunks, 4), 128, 0, as_stream(stream)>>>(cdf, Lp, in, offsets, rows, n, 0, chunks, sym);
     GPC_LAUNCH_CHECK();
     return GPC_OK;
 }

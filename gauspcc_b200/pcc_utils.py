@@ -50,6 +50,11 @@ def _batch(codec: GausPcgcCodec) -> BatchCodec:
     return _BATCH[id(codec)]
 
 
+def _check_chunk(gpu_coder_chunk) -> None:
+    if gpu_coder_chunk and not (32 <= int(gpu_coder_chunk) <= 16384):
+        raise ValueError("gpu_coder_chunk must be in 32..16384 (chunk byte counts are stored as u16)")
+
+
 def _to_device_xyz(xyz_quantized, dev):
     xyz = torch.tensor(xyz_quantized) if isinstance(xyz_quantized, np.ndarray) else xyz_quantized.detach()
     if xyz.is_floating_point():
@@ -111,8 +116,7 @@ def compress_point_cloud(
     container version 2 (bitstream.py) -- smaller PCIe traffic and no host range coder on either side, but NOT readable by the
     reference's decompress_point_cloud.  The default (0) writes the reference's own bitstream.
     """
-    if gpu_coder_chunk and not (32 <= int(gpu_coder_chunk) <= 16384):
-        raise ValueError("gpu_coder_chunk must be in 32..16384 (chunk byte counts are stored as u16)")
+    _check_chunk(gpu_coder_chunk)
     os.makedirs(os.path.dirname(output_path), exist_ok=True)
     codec = _codec(ckpt_path, channels, kernel_size)
     dev = codec.dev
@@ -214,16 +218,19 @@ def _save_ply_ascii_geo(coords: np.ndarray, path: str) -> None:
             f.write(f'{p[0]} {p[1]} {p[2]}\n')
 
 
-def compress_point_clouds(xyz_list, ckpt_path, output_paths, channels=32, kernel_size=5, posQ=1) -> List[dict]:
+def compress_point_clouds(xyz_list, ckpt_path, output_paths, channels=32, kernel_size=5, posQ=1, gpu_coder_chunk=0) -> List[dict]:
     """
     Compress many point clouds in one call (extension, not in the reference): file i is byte-identical to
-    compress_point_cloud(xyz_list[i], ckpt_path, output_paths[i], channels, kernel_size, posQ).
+    compress_point_cloud(xyz_list[i], ckpt_path, output_paths[i], channels, kernel_size, posQ, gpu_coder_chunk).
 
     The scenes are coded together as one union octree (gauspcc_b200/batch.py): one set of launches per level and the range coders
-    of all scenes side by side on the codec's thread pool, instead of one level loop per scene.  Returns one dict per scene with the
-    single call's keys; 'enc_time' and 'gpu_time' are 0.0 there (the scenes are coded together, there is no per-scene time) and
-    'batch_enc_time' is the wall-clock time of the whole batch, the same value in every dict.
+    of all scenes side by side on the codec's thread pool, instead of one level loop per scene.  With gpu_coder_chunk > 0 the files
+    are container version 2, as compress_point_cloud writes them: every chunk of every scene's streams is coded on the GPU by one
+    launch per union, and no host range coder runs.  Returns one dict per scene with the single call's keys; 'enc_time' and
+    'gpu_time' are 0.0 there (the scenes are coded together, there is no per-scene time) and 'batch_enc_time' is the wall-clock time
+    of the whole batch, the same value in every dict.
     """
+    _check_chunk(gpu_coder_chunk)
     xyz_list, output_paths = list(xyz_list), list(output_paths)
     if len(xyz_list) != len(output_paths):
         raise ValueError(f"compress_point_clouds: {len(xyz_list)} point clouds but {len(output_paths)} output paths")
@@ -236,7 +243,7 @@ def compress_point_clouds(xyz_list, ckpt_path, output_paths, channels=32, kernel
         os.makedirs(os.path.dirname(p), exist_ok=True)
     torch.cuda.synchronize(dev)
     t0 = time.time()
-    coded = _batch(codec).encode(xyzs)
+    coded = _batch(codec).encode(xyzs, gpu_chunk=int(gpu_coder_chunk))
     torch.cuda.synchronize(dev)
     batch_enc_time = time.time() - t0
     out = []
@@ -254,16 +261,19 @@ def decompress_point_clouds(bin_paths, ckpt_path, channels=32, kernel_size=5, is
                             sorted_output=False) -> List[dict]:
     """
     Decompress many files in one call (extension): result i's 'point_cloud' equals
-    decompress_point_cloud(bin_paths[i], ckpt_path, ...)['point_cloud'] row for row, in both row orders.  Container version 2 files
-    are not accepted here (ValueError naming the file).  'dec_time' and 'gpu_time' are 0.0; 'batch_dec_time' is the wall-clock time
-    of the whole batch, the same value in every dict.  No PLY output.
+    decompress_point_cloud(bin_paths[i], ckpt_path, ...)['point_cloud'] row for row, in both row orders.  The files of one call are
+    all container version 1 or all version 2 (their chunk sizes may differ); a call that mixes the two raises ValueError naming the
+    first file whose version differs from the first file's.  Version-2 files are decoded on the GPU chunk by chunk, every stage of a
+    union level by one launch, and each decoded count is checked against the file's trailer (ValueError naming the file, as
+    decompress_point_cloud raises).  'dec_time' and 'gpu_time' are 0.0; 'batch_dec_time' is the wall-clock time of the whole batch,
+    the same value in every dict.  No PLY output.
     """
     bin_paths = list(bin_paths)
     if not bin_paths:
         return []
     codec = _codec(ckpt_path, channels, kernel_size)
     dev = codec.dev
-    files = []
+    files, coded = [], []
     for p in bin_paths:
         with open(p, 'rb') as f:
             blob = f.read()
@@ -271,12 +281,20 @@ def decompress_point_clouds(bin_paths, ckpt_path, channels=32, kernel_size=5, is
             posQ, base_xyz, base_occ, streams = bitstream.read_file(blob)
         except ValueError as e:
             raise ValueError(f"{p}: {e}") from e
-        if bitstream.split_v2(streams)[1]:
-            raise ValueError(f"{p}: container version 2 files cannot be decoded in a batch; use decompress_point_cloud")
-        files.append((float(posQ), base_xyz, base_occ, streams))
+        streams, chunk, n_coded = bitstream.split_v2(streams)
+        if files and bool(chunk) != bool(files[0][4]):
+            # one container version per call keeps every union level on one decode discipline
+            raise ValueError(f"{p}: container version {2 if chunk else 1} file after version {2 if files[0][4] else 1} files; "
+                             "version 1 and version 2 files cannot be decoded in one call")
+        files.append((float(posQ), base_xyz, base_occ, streams, chunk))
+        coded.append(n_coded)
     torch.cuda.synchronize(dev)
     t0 = time.time()
-    scans = _batch(codec).decode(files, sorted_rows=bool(sorted_output))
+    scans = _batch(codec).decode(files, sorted_rows=bool(sorted_output), names=bin_paths)
+    for p, s, n_coded in zip(bin_paths, scans, coded):
+        if n_coded is not None and s.shape[0] != n_coded:
+            raise ValueError(f"{p}: version-2 file decodes to {s.shape[0]} voxels, its trailer says {n_coded}: corrupt file, wrong "
+                             "checkpoint or a library whose kernels sum in another order than the writer's")
     if not is_data_pre_quantized:
         scans = [(s - 131072) * 0.001 for s in scans]             # pcc_utils.py:381
     torch.cuda.synchronize(dev)

@@ -328,8 +328,9 @@ int gpc_row_decode(const float *row, const uint8_t *in, const int32_t *cnt, int6
                    void *ws, size_t ws_bytes, void *stream);
 
 /* ---- f-3: the chunked GPU coder on the geometry codec's own streams (container version 2; NOT the torchac bitstream: one coder
- * per chunk instead of one per stream).  Encode: lohi as gpc_head_cdf_sym writes it; no host synchronisation.  Decode: one stream
- * at a time (stage i + 1 needs stage i), cdf rows as gpc_head_cdf writes them. ---- */
+ * per chunk instead of one per stream).  Encode: lohi as gpc_head_cdf_sym writes it; no host synchronisation.  Decode: one stage
+ * at a time (stage i + 1 needs stage i) -- one stream, or with _ranges the streams of many scenes whose rows are one after the
+ * other in one level -- cdf rows as gpc_head_cdf writes them. ---- */
 size_t gpc_chunk_workspace_bytes(int chunks, int max_chunk);
 /* chunk w = symbols [starts[w], starts[w + 1]) of lohi (device u32[chunks + 1]; at most max_chunk symbols each): the streams of a
  * scene one after the other, every stream cut into chunks of its own length, all coded by ONE launch */
@@ -339,6 +340,11 @@ int gpc_chunk_merge(const void *ws, int chunks, int max_chunk, const uint32_t *o
 /* offsets: device u32[chunks + 1], first byte of every chunk in `in` (prefix sums of the stream's u16 byte counts); Lp <= 32 */
 int gpc_chunk_decode_u16(const uint16_t *cdf, const uint8_t *in, const uint32_t *offsets, int64_t n, int Lp, int chunk_size,
                          uint8_t *sym, void *stream);
+/* chunk w decodes rows [rows[w], rows[w + 1]) of cdf / sym from bytes [offsets[w], offsets[w + 1]) of `in`;
+ * rows, offsets: device u32[chunks + 1], non-decreasing; n = rows of cdf / sym; Lp <= 32.  Every chunk is clamped to rows [0, n)
+ * (a malformed table decodes garbage, never outside the arrays' rows); bytes past a chunk's length read as zeros. */
+int gpc_chunk_decode_u16_ranges(const uint16_t *cdf, int Lp, const uint8_t *in, const uint32_t *offsets, const uint32_t *rows,
+                                int chunks, int64_t n, uint8_t *sym, void *stream);
 
 #ifdef __cplusplus
 }
