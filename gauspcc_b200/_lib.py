@@ -107,6 +107,10 @@ SIGNATURES = {
     "gpc_chunk_decode_u16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_vp, c_vp]),
     "gpc_chunk_decode_u16_ranges": (c_int, [c_vp, c_int, c_vp, c_vp, c_vp, c_int, c_i64, c_vp, c_vp]),
     "gpc_attr_decode_gaussian": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_ply_format_workspace_bytes": (c_sz, [c_i64]),
+    "gpc_ply_format_f32": (c_int, [c_vp, c_i64, c_vp, C.c_uint64, C.POINTER(C.c_uint64), c_vp, c_sz, c_vp]),
+    "gpc_text_parse_workspace_bytes": (c_sz, [C.c_uint64]),
+    "gpc_text_parse_xyz": (c_int, [c_vp, C.c_uint64, c_vp, C.POINTER(C.c_uint32), c_vp, C.POINTER(C.c_uint32), c_vp, c_sz, c_vp]),
 }
 
 _lib = None

@@ -10,6 +10,15 @@ decompress_ue_4stage_conv.py:176-179), `.bin` container (one `<name>.bin` per in
 final `avg` row, :253-276) as the reference scripts.  `--kernel_size` defaults to 3 as in the reference scripts
 (compress_ue_4stage_conv.py:44; the HAC call sites use 5, pcc_utils.py:29): both are built, channels = 32 only.  Differences: point files are read in this process (the reference forks 64 workers); `h5` is not
 read (the reference lists the suffix but `kit/io.py:read_points` cannot parse it either).  No torchsparse / torchac.
+
+Text inputs (ASCII ply and other text) are parsed on the GPU (plyio.read_points_device: the rows `read_points` gives) and mapped
+to voxels there with the same float64 operations as `quantise`; decoded clouds are written as ASCII ply rows formatted on the GPU
+(plyio.write_ply_ascii: the bytes of the reference's writer).
+
+`--batch N` (default 1): with N > 1, consecutive groups of N files are coded in one call each (pcc_utils.compress_point_clouds /
+decompress_point_clouds: one union octree per group, the same `.bin` and `.ply` bytes as one file at a time).  A group has no
+per-file time, so each of its CSV rows reports `enc_time` / `dec_time` = the group's wall-clock coding time (`batch_enc_time` /
+`batch_dec_time`) divided by its number of files.  With N = 1 every file is coded by its own call and timed alone, as before.
 """
 from __future__ import annotations
 
@@ -24,7 +33,7 @@ from typing import Dict, List, Optional
 import numpy as np
 import torch
 
-from . import pcc_utils
+from . import pcc_utils, plyio
 
 SUFFIXES = (".h5", ".ply", ".bin", ".npy")
 
@@ -42,13 +51,9 @@ def read_points(path: str) -> np.ndarray:
     rows: List[List[float]] = []
     with open(path, "r", errors="ignore") as f:
         for line in f:
-            parts = line.split()
-            if len(parts) < 3:
-                continue
-            try:
-                rows.append([float(parts[0]), float(parts[1]), float(parts[2])])
-            except ValueError:
-                continue
+            xyz = plyio.xyz_of_line(line)
+            if xyz is not None:
+                rows.append(xyz)
     return np.asarray(rows, dtype=np.float64).reshape(-1, 3)
 
 
@@ -64,6 +69,20 @@ def quantise(xyz: np.ndarray, posQ: int, is_data_pre_quantized: bool) -> torch.T
     return torch.round(t / posQ).int()
 
 
+def quantise_device(xyz: torch.Tensor, posQ: int, is_data_pre_quantized: bool) -> torch.Tensor:
+    """`quantise` on a float64 CUDA tensor, with the same float64 operations: the divisors are device tensors, so the division is
+    an IEEE division (not a multiplication by the rounded reciprocal, which a host scalar divisor would give)."""
+    xyz = xyz.to(torch.float64)
+    t = xyz if is_data_pre_quantized else xyz / torch.tensor(0.001, dtype=torch.float64, device=xyz.device) + 131072
+    return torch.round(t / torch.tensor(float(posQ), dtype=torch.float64, device=xyz.device)).int()
+
+
+def _groups(items: List[str], batch: int) -> List[List[str]]:
+    if batch < 1:
+        raise ValueError(f"batch must be >= 1, got {batch}")
+    return [items[i:i + batch] for i in range(0, len(items), batch)]
+
+
 def _write_csv(path: str, rows: List[Dict[str, object]], numeric: List[str]) -> None:
     avg: Dict[str, object] = {k: float(np.mean([float(r[k]) for r in rows])) for k in numeric}
     avg["filedir"] = "avg"
@@ -76,20 +95,27 @@ def _write_csv(path: str, rows: List[Dict[str, object]], numeric: List[str]) -> 
 
 def compress_files(input_glob: str, output_folder: str, ckpt: str, posQ: int = 16, is_data_pre_quantized: bool = False,
                    channels: int = 32, kernel_size: int = 5, num_samples: int = -1, resultdir: Optional[str] = None,
-                   prefix: str = "ue_4stage_conv") -> List[Dict[str, object]]:
+                   prefix: str = "ue_4stage_conv", batch: int = 1) -> List[Dict[str, object]]:
     os.makedirs(output_folder, exist_ok=True)
     paths = list_inputs(input_glob, num_samples)
     if not paths:
         raise FileNotFoundError(f"no point-cloud files (h5 / ply / bin / npy) under {input_glob}")
+    dev = pcc_utils._require_cuda()
     rows: List[Dict[str, object]] = []
-    for p in paths:
-        name = os.path.split(p)[-1]
-        xyz = quantise(read_points(p), posQ, is_data_pre_quantized)
+    for group in _groups(paths, batch):
+        names = [os.path.split(p)[-1] for p in group]
+        xyzs = [quantise_device(plyio.read_points_device(p, dev), posQ, is_data_pre_quantized) for p in group]
+        outs = [os.path.join(output_folder, name + ".bin") for name in names]
+        if batch == 1:
+            rs = [pcc_utils.compress_point_cloud(xyzs[0], ckpt, outs[0], channels=channels, kernel_size=kernel_size, posQ=posQ)]
+        else:
+            rs = pcc_utils.compress_point_clouds(xyzs, ckpt, outs, channels=channels, kernel_size=kernel_size, posQ=posQ)
+            for r in rs:
+                r["enc_time"] = r["batch_enc_time"] / len(group)
         # the codec stores the SET of voxels; N of the report is the number of input points, as in the reference (:96, :246)
-        r = pcc_utils.compress_point_cloud(xyz, ckpt, os.path.join(output_folder, name + ".bin"), channels=channels,
-                                           kernel_size=kernel_size, posQ=posQ)
-        rows.append({"filedir": name, "bpp": r["file_size_bits"] / max(xyz.shape[0], 1), "enc_time": r["enc_time"],
-                     "file_size_bits": r["file_size_bits"], "num_points": int(xyz.shape[0])})
+        for name, xyz, r in zip(names, xyzs, rs):
+            rows.append({"filedir": name, "bpp": r["file_size_bits"] / max(xyz.shape[0], 1), "enc_time": r["enc_time"],
+                         "file_size_bits": r["file_size_bits"], "num_points": int(xyz.shape[0])})
     if resultdir:
         os.makedirs(resultdir, exist_ok=True)
         _write_csv(os.path.join(resultdir, f"{prefix}_data{len(paths)}.csv"), rows, ["bpp", "enc_time", "file_size_bits", "num_points"])
@@ -97,18 +123,26 @@ def compress_files(input_glob: str, output_folder: str, ckpt: str, posQ: int = 1
 
 
 def decompress_files(input_glob: str, output_folder: str, ckpt: str, is_data_pre_quantized: bool = False, channels: int = 32,
-                     kernel_size: int = 5, resultdir: Optional[str] = None, prefix: str = "ue_4stage_conv") -> List[Dict[str, object]]:
+                     kernel_size: int = 5, resultdir: Optional[str] = None, prefix: str = "ue_4stage_conv",
+                     batch: int = 1) -> List[Dict[str, object]]:
     os.makedirs(output_folder, exist_ok=True)
     paths = list_inputs(input_glob, suffixes=(".bin",))
     if not paths:
         raise FileNotFoundError(f"no .bin files under {input_glob}")
     rows: List[Dict[str, object]] = []
-    for p in paths:
-        name = os.path.split(p)[-1]
-        out_path = os.path.join(output_folder, name + ".ply")
-        r = pcc_utils.decompress_point_cloud(p, ckpt, out_path, channels=channels, kernel_size=kernel_size,
-                                             is_data_pre_quantized=is_data_pre_quantized)
-        rows.append({"filedir": name, "dec_time": r["dec_time"], "num_points": int(r["num_points"])})
+    for group in _groups(paths, batch):
+        names = [os.path.split(p)[-1] for p in group]
+        outs = [os.path.join(output_folder, name + ".ply") for name in names]
+        if batch == 1:
+            rs = [pcc_utils.decompress_point_cloud(group[0], ckpt, outs[0], channels=channels, kernel_size=kernel_size,
+                                                   is_data_pre_quantized=is_data_pre_quantized)]
+        else:
+            rs = pcc_utils.decompress_point_clouds(group, ckpt, channels=channels, kernel_size=kernel_size,
+                                                   is_data_pre_quantized=is_data_pre_quantized, output_paths=outs)
+            for r in rs:
+                r["dec_time"] = r["batch_dec_time"] / len(group)
+        for name, r in zip(names, rs):
+            rows.append({"filedir": name, "dec_time": r["dec_time"], "num_points": int(r["num_points"])})
     if resultdir:
         os.makedirs(resultdir, exist_ok=True)
         _write_csv(os.path.join(resultdir, f"{prefix}_dec_data{len(paths)}.csv"), rows, ["dec_time", "num_points"])
@@ -129,6 +163,9 @@ def main(argv: Optional[List[str]] = None) -> int:
         sp.add_argument("--kernel_size", type=int, default=3)      # the reference scripts' default; the checkpoint must match
         sp.add_argument("--resultdir", default=None, help="folder for the CSV report")
         sp.add_argument("--prefix", default="ue_4stage_conv")
+        sp.add_argument("--batch", type=int, default=1,
+                        help="files coded per call: N > 1 codes consecutive groups of N files together (same output bytes); each "
+                             "file's CSV time is then its group's wall-clock coding time divided by the group's file count")
         if cmd == "compress":
             sp.add_argument("--posQ", type=int, default=16, help="quantisation scale")
             sp.add_argument("--num_samples", type=int, default=-1, help="first N files only (-1 = all)")
@@ -136,13 +173,13 @@ def main(argv: Optional[List[str]] = None) -> int:
     t0 = time.time()
     if a.cmd == "compress":
         rows = compress_files(a.input_glob, a.output_folder, a.ckpt, a.posQ, a.is_data_pre_quantized, a.channels, a.kernel_size,
-                              a.num_samples, a.resultdir, a.prefix)
+                              a.num_samples, a.resultdir, a.prefix, a.batch)
         print("Total: {:d} | Average bitrate:{:.3f} | Encoding time:{:.3f}s | Max GPU memory:{:.2f}MB".format(
             len(rows), float(np.mean([r["bpp"] for r in rows])), float(np.mean([r["enc_time"] for r in rows])),
             torch.cuda.max_memory_allocated() / 1024 / 1024))
     else:
         rows = decompress_files(a.input_glob, a.output_folder, a.ckpt, a.is_data_pre_quantized, a.channels, a.kernel_size,
-                                a.resultdir, a.prefix)
+                                a.resultdir, a.prefix, a.batch)
         print("Total: {:d} | Decoding time:{:.3f}s | Max GPU memory:{:.2f}MB".format(
             len(rows), float(np.mean([r["dec_time"] for r in rows])), torch.cuda.max_memory_allocated() / 1024 / 1024))
     print(f"wall {time.time() - t0:.2f} s")

@@ -20,7 +20,7 @@ from typing import Dict, List
 import numpy as np
 import torch
 
-from . import _lib, bitstream
+from . import _lib, bitstream, plyio
 from .batch import BatchCodec
 from .codec import GausPcgcCodec, load_weights
 
@@ -197,8 +197,8 @@ def decompress_point_cloud(
     point_cloud = scan
     if output_path:
         # the reference calls io.save_ply_ascii_geo here but never imports `io` (pcc_utils.py:392 would raise
-        # NameError); write the same ASCII geometry PLY (kit/io.py:36-49) instead of failing.
-        _save_ply_ascii_geo(point_cloud.cpu().numpy(), output_path)
+        # NameError); write the same ASCII geometry PLY (kit/io.py:36-49) instead of failing, rows formatted on the GPU.
+        plyio.write_ply_ascii(point_cloud, output_path)
     return {
         'dec_time': dec_time,
         'num_points': point_cloud.shape[0],
@@ -206,16 +206,6 @@ def decompress_point_cloud(
         'output_path': output_path,
         'gpu_time': codec.last_stats.get("gpu_ms", 0.0) / 1e3,
     }
-
-
-def _save_ply_ascii_geo(coords: np.ndarray, path: str) -> None:
-    coords = coords.astype(np.float32)
-    with open(path, 'w') as f:
-        f.write('ply\nformat ascii 1.0\n')
-        f.write(f'element vertex {coords.shape[0]}\n')
-        f.write('property float x\nproperty float y\nproperty float z\nend_header\n')
-        for p in coords:
-            f.write(f'{p[0]} {p[1]} {p[2]}\n')
 
 
 def compress_point_clouds(xyz_list, ckpt_path, output_paths, channels=32, kernel_size=5, posQ=1, gpu_coder_chunk=0) -> List[dict]:
@@ -258,7 +248,7 @@ def compress_point_clouds(xyz_list, ckpt_path, output_paths, channels=32, kernel
 
 
 def decompress_point_clouds(bin_paths, ckpt_path, channels=32, kernel_size=5, is_data_pre_quantized=True,
-                            sorted_output=False) -> List[dict]:
+                            sorted_output=False, output_paths=None) -> List[dict]:
     """
     Decompress many files in one call (extension): result i's 'point_cloud' equals
     decompress_point_cloud(bin_paths[i], ckpt_path, ...)['point_cloud'] row for row, in both row orders.  The files of one call are
@@ -266,9 +256,18 @@ def decompress_point_clouds(bin_paths, ckpt_path, channels=32, kernel_size=5, is
     first file whose version differs from the first file's.  Version-2 files are decoded on the GPU chunk by chunk, every stage of a
     union level by one launch, and each decoded count is checked against the file's trailer (ValueError naming the file, as
     decompress_point_cloud raises).  'dec_time' and 'gpu_time' are 0.0; 'batch_dec_time' is the wall-clock time of the whole batch,
-    the same value in every dict.  No PLY output.
+    the same value in every dict.  With output_paths (one per file), scene i is also written to output_paths[i] as the ASCII PLY
+    decompress_point_cloud(bin_paths[i], ..., output_path=output_paths[i]) writes, byte for byte, after the timed batch; that path
+    is then result i's 'output_path'.
     """
     bin_paths = list(bin_paths)
+    if output_paths is not None:
+        output_paths = list(output_paths)
+        if len(output_paths) != len(bin_paths):
+            raise ValueError(f"decompress_point_clouds: {len(bin_paths)} files but {len(output_paths)} output paths")
+        for p in output_paths:
+            if p:
+                os.makedirs(os.path.dirname(p), exist_ok=True)
     if not bin_paths:
         return []
     codec = _codec(ckpt_path, channels, kernel_size)
@@ -299,5 +298,9 @@ def decompress_point_clouds(bin_paths, ckpt_path, channels=32, kernel_size=5, is
         scans = [(s - 131072) * 0.001 for s in scans]             # pcc_utils.py:381
     torch.cuda.synchronize(dev)
     batch_dec_time = time.time() - t0
-    return [{'dec_time': 0.0, 'num_points': s.shape[0], 'point_cloud': s, 'output_path': None, 'gpu_time': 0.0,
-             'batch_dec_time': batch_dec_time} for s in scans]
+    outs = output_paths if output_paths is not None else [None] * len(scans)
+    for s, p in zip(scans, outs):
+        if p:
+            plyio.write_ply_ascii(s, p)
+    return [{'dec_time': 0.0, 'num_points': s.shape[0], 'point_cloud': s, 'output_path': p, 'gpu_time': 0.0,
+             'batch_dec_time': batch_dec_time} for s, p in zip(scans, outs)]

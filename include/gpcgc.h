@@ -346,6 +346,24 @@ int gpc_chunk_decode_u16(const uint16_t *cdf, const uint8_t *in, const uint32_t 
 int gpc_chunk_decode_u16_ranges(const uint16_t *cdf, int Lp, const uint8_t *in, const uint32_t *offsets, const uint32_t *rows,
                                 int chunks, int64_t n, uint8_t *sym, void *stream);
 
+/* ---- ASCII PLY text (textio.cu).  Formatter: row r of xyz (float32 [n][3]) becomes "x y z\n", every value widened to double and
+ * written as Python's repr() writes it (shortest round-trip digits, positional for decimal exponents in [-4, 16), else d.ddde+XX),
+ * rows back to back in row order; at most 75 bytes a row.  *out_len_h (host) = bytes of text; a buffer of fewer than that many
+ * bytes (cap) gives GPC_EINVAL.  Synchronises `stream` (one read-back of the length).  n <= 2^32 / 75. ---- */
+size_t gpc_ply_format_workspace_bytes(int64_t n);
+int gpc_ply_format_f32(const float *xyz, int64_t n, char *out, uint64_t cap, uint64_t *out_len_h, void *ws, size_t ws_bytes,
+                       void *stream);
+/* Parser: the rows of cli.read_points' text branch.  Lines end at "\n", "\r\n" or a lone "\r"; a line of printable ASCII and
+ * tabs gives a row when its first three space / tab separated tokens are all [+-]?(d+(.d*)?|.d+)([eE][+-]?d+)? (correctly rounded
+ * to double, as float() does), no row when it has fewer than three tokens or one is not a float.  A line the GPU leaves to
+ * float() itself (any other byte, a token [+-]?(inf|infinity|nan) in any case or holding "_", or a rounding the 128-bit product
+ * cannot decide) is reported in host_lines as {first byte, end of its content (terminator excluded), rows before it}; its row, if
+ * any, belongs before row `rows before it` of rows.  rows: double [(nbytes + 1) / 6][3]; host_lines: u32 [(nbytes + 1) / 2][3];
+ * *n_rows_h, *n_host_h (host): counts.  nbytes < 2^32.  Synchronises `stream` (one read-back of the two counts). */
+size_t gpc_text_parse_workspace_bytes(uint64_t nbytes);
+int gpc_text_parse_xyz(const char *text, uint64_t nbytes, double *rows, uint32_t *n_rows_h, uint32_t *host_lines,
+                       uint32_t *n_host_h, void *ws, size_t ws_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
