@@ -3,6 +3,9 @@
 
     python -m gauspcc_b200.cli compress   --input_glob DIR --output_folder OUT --ckpt CKPT [--posQ 16] [--is_data_pre_quantized]
     python -m gauspcc_b200.cli decompress --input_glob OUT --output_folder DEC --ckpt CKPT [--is_data_pre_quantized]
+    python -m gauspcc_b200.cli train      --input_glob DIR --ckpt_out CKPT [--init CKPT] [--steps N] [--lr 5e-4] [--seed S]
+                                          [--kernel_size 3|5] [--posQ 16] [--is_data_pre_quantized] [--max_points 150000]
+                                          [--resultdir R]
 
 Same argument names, file discovery (recursive, sorted, h5 / ply / bin / npy; compress_ue_4stage_conv.py:57-63), coordinate
 mapping (`x / 0.001 + 131072` unless pre-quantised, then `round(x / posQ)`, :90-95; inverse `(c * posQ - 131072) * 0.001`,
@@ -14,6 +17,11 @@ read (the reference lists the suffix but `kit/io.py:read_points` cannot parse it
 Text inputs (ASCII ply and other text) are parsed on the GPU (plyio.read_points_device: the rows `read_points` gives) and mapped
 to voxels there with the same float64 operations as `quantise`; decoded clouds are written as ASCII ply rows formatted on the GPU
 (plyio.write_ply_ascii: the bytes of the reference's writer).
+
+`train` (not in the reference scripts, whose trainer runs on torchsparse): reads and quantises files exactly as `compress` does, cuts
+them into kd-tree patches of at most --max_points points and trains a checkpoint on the GPU (gauspcc_b200/train.py), written in the
+reference layout to --ckpt_out; `compress` / `decompress` load it with the same --kernel_size.  The CSV log
+(`<prefix>_train_data<N>.csv`: step, patch points, bpp, elapsed seconds) goes to --resultdir beside the other reports.
 
 `--batch N` (default 1): with N > 1, consecutive groups of N files are coded in one call each (pcc_utils.compress_point_clouds /
 decompress_point_clouds: one union octree per group, the same `.bin` and `.ply` bytes as one file at a time).  A group has no
@@ -149,7 +157,7 @@ def decompress_files(input_glob: str, output_folder: str, ckpt: str, is_data_pre
     return rows
 
 
-def main(argv: Optional[List[str]] = None) -> int:
+def build_parser() -> argparse.ArgumentParser:
     ap = argparse.ArgumentParser(prog="python -m gauspcc_b200.cli", description=__doc__.split("\n\n")[0],
                                  formatter_class=argparse.ArgumentDefaultsHelpFormatter)
     sub = ap.add_subparsers(dest="cmd", required=True)
@@ -169,9 +177,61 @@ def main(argv: Optional[List[str]] = None) -> int:
         if cmd == "compress":
             sp.add_argument("--posQ", type=int, default=16, help="quantisation scale")
             sp.add_argument("--num_samples", type=int, default=-1, help="first N files only (-1 = all)")
-    a = ap.parse_args(argv)
+    tp = sub.add_parser("train", formatter_class=argparse.ArgumentDefaultsHelpFormatter,
+                        help="train a checkpoint on the GPU (gauspcc_b200/train.py) from point-cloud files")
+    tp.add_argument("--input_glob", required=True, help="folder searched recursively for training files")
+    tp.add_argument("--ckpt_out", required=True, help="checkpoint written in the reference layout (every --save_every steps and at the end)")
+    tp.add_argument("--init", default=None, help="checkpoint to start from (default: make_synthetic_state_dict(--init_seed))")
+    tp.add_argument("--init_seed", type=int, default=5)
+    tp.add_argument("--steps", type=int, default=1000)
+    tp.add_argument("--lr", type=float, default=5e-4)
+    tp.add_argument("--seed", type=int, default=0, help="draws the patch order")
+    tp.add_argument("--kernel_size", type=int, default=3, choices=(3, 5))
+    tp.add_argument("--posQ", type=int, default=16, help="quantisation scale (as compress)")
+    tp.add_argument("--is_data_pre_quantized", action="store_true", help="inputs are integer voxel coordinates already")
+    tp.add_argument("--max_points", type=int, default=150_000, help="largest kd-tree patch")
+    tp.add_argument("--save_every", type=int, default=0)
+    tp.add_argument("--resultdir", default=None, help="folder for the CSV training log")
+    tp.add_argument("--prefix", default="ue_4stage_conv")
+    return ap
+
+
+def train_files(input_glob: str, ckpt_out: str, init: Optional[str] = None, steps: int = 1000, lr: float = 5e-4, seed: int = 0,
+                kernel_size: int = 3, posQ: int = 16, is_data_pre_quantized: bool = False, max_points: int = 150_000,
+                save_every: int = 0, resultdir: Optional[str] = None, prefix: str = "ue_4stage_conv",
+                init_seed: int = 5) -> List[Dict[str, object]]:
+    """Train a checkpoint (gauspcc_b200/train.py) on the files under input_glob, read and quantised exactly as `compress` reads them,
+    so that the checkpoint learns the voxels it will code.  Writes `<prefix>_train_data<N>.csv` (one row per step) to resultdir."""
+    from . import train as T
+    dev = pcc_utils._require_cuda()
+    paths = list_inputs(input_glob)
+    if not paths:
+        raise FileNotFoundError(f"no point-cloud files (h5 / ply / bin / npy) under {input_glob}")
+    clouds = [quantise_device(plyio.read_points_device(p, dev), posQ, is_data_pre_quantized) for p in paths]
+    d = os.path.dirname(os.path.abspath(ckpt_out))
+    os.makedirs(d, exist_ok=True)
+    _, rows = T.train(clouds, ckpt_out, init=init, steps=steps, lr=lr, seed=seed, kernel_size=kernel_size, max_points=max_points,
+                      save_every=save_every, synthetic_seed=init_seed)
+    if resultdir:
+        os.makedirs(resultdir, exist_ok=True)
+        with open(os.path.join(resultdir, f"{prefix}_train_data{len(paths)}.csv"), "w", newline="") as f:
+            w = csv.DictWriter(f, fieldnames=list(rows[0].keys()))
+            w.writeheader()
+            w.writerows(rows)
+    return rows
+
+
+def main(argv: Optional[List[str]] = None) -> int:
+    a = build_parser().parse_args(argv)
     t0 = time.time()
-    if a.cmd == "compress":
+    if a.cmd == "train":
+        rows = train_files(a.input_glob, a.ckpt_out, a.init, a.steps, a.lr, a.seed, a.kernel_size, a.posQ, a.is_data_pre_quantized,
+                           a.max_points, a.save_every, a.resultdir, a.prefix, a.init_seed)
+        tail = rows[-min(20, len(rows)):]
+        print("Steps: {:d} | bpp first {:.3f} last {:.3f} (mean of up to 20 steps) | Max GPU memory:{:.2f}MB".format(
+            len(rows), float(np.mean([r["bpp"] for r in rows[:20]])), float(np.mean([r["bpp"] for r in tail])),
+            torch.cuda.max_memory_allocated() / 1024 / 1024))
+    elif a.cmd == "compress":
         rows = compress_files(a.input_glob, a.output_folder, a.ckpt, a.posQ, a.is_data_pre_quantized, a.channels, a.kernel_size,
                               a.num_samples, a.resultdir, a.prefix, a.batch)
         print("Total: {:d} | Average bitrate:{:.3f} | Encoding time:{:.3f}s | Max GPU memory:{:.2f}MB".format(

@@ -1,0 +1,335 @@
+"""Training of GausPcgc checkpoints on the GPU, on the codec's own geometry and conv kernels.
+
+    SparseConvFn   autograd of one 5^3 sparse conv on the mma.sync family: forward gpc_spconv_fwd_v6, input gradient the same kernel
+                   with the mirrored, transposed weights W'[k] = W[124 - k]^T (a submanifold map is symmetric: nbr_k(o) = i exactly
+                   when nbr_{124-k}(i) = o), weight gradient gpc_spconv_wgrad_v6 (csrc/spconv_grad.cu)
+    GausPcgcNet    the model of SURVEY.md Appendix A as an nn.Module whose state_dict() is the reference layout
+                   (weights.reference_layout); forward(xyz) returns the code length of the file's occupancy streams under the
+                   coder's probabilities
+    partition      kd-tree patches (median split along the longest axis), the patching of the reference's dataset.py
+    train          Adam over patches, checkpoints in the reference layout
+
+The geometry (pyramid, children, kernel maps) comes from GausPcgcCodec exactly as the encoder builds it, so a checkpoint trained here
+is trained on the voxels, row orders and conv offsets it is later coded with: it loads with pcc_utils.compress_point_cloud unchanged.
+Every level runs the mma.sync conv family (the codec's family for levels below 150 K rows; patches are at most 150 K points).
+
+Determinism: the same seed, inputs and initial weights give a bit-identical checkpoint.  The convs sum in an order fixed by the map,
+and the torch backward steps that would accumulate with atomics (embedding rows, the children -> parent gather) are written as
+fixed-order sums instead.  No process-wide torch flag is touched.
+"""
+from __future__ import annotations
+
+import time
+from typing import Callable, Dict, List, Optional, Sequence, Union
+
+import numpy as np
+import torch
+from torch import nn
+
+from . import _lib
+from . import weights as W
+from .codec import CTX_SHIFT, STAGE_MASK, STAGE_SHIFT, GausPcgcCodec, KMap, Level, _ptr
+
+# the 27 offsets of a 3^3 kernel at their K = 5 indices ((dz+2)*5 + (dy+2))*5 + (dx+2), as DeviceWeights places them
+K5_OF_K3 = tuple(((dz + 2) * 5 + (dy + 2)) * 5 + (dx + 2) for dz in (-1, 0, 1) for dy in (-1, 0, 1) for dx in (-1, 0, 1))
+
+
+def _stream(dev: torch.device):
+    return torch.cuda.current_stream(dev).cuda_stream
+
+
+def pack_frag(W125: torch.Tensor) -> torch.Tensor:
+    """W [125,32,32] fp32 -> the mma.sync A fragments of W^T (gpc_spconv_pack_weights_frag, 512 000 bytes)"""
+    Wa = torch.empty_like(W125)
+    _lib.check(_lib.load().gpc_spconv_pack_weights_frag(_ptr(W125), 1, _ptr(Wa), _stream(W125.device)), "gpc_spconv_pack_weights_frag")
+    return Wa
+
+
+def conv_v6(x: torch.Tensor, Wa: torch.Tensor, km: KMap) -> torch.Tensor:
+    """y = sum_k x[nbr_k(o)] . W[k] over the level's mma.sync pair stream (no residual, no activation)"""
+    y = torch.empty_like(x)
+    _lib.check(_lib.load().gpc_spconv_fwd_v6(_ptr(x), _ptr(Wa), _ptr(km.seg), _ptr(km.pairs), x.shape[0], km.tile_rows, None, 0, _ptr(y),
+                                             km.v6_variant, _stream(x.device)), "gpc_spconv_fwd_v6")
+    return y
+
+
+def conv_dgrad(dy: torch.Tensor, W125: torch.Tensor, km: KMap) -> torch.Tensor:
+    """dx = sum_k dy[nbr_{124-k}(i)] . W[124-k]^T: the forward conv with W'[k] = W[124 - k]^T"""
+    return conv_v6(dy, pack_frag(W125.flip(0).transpose(1, 2).contiguous()), km)
+
+
+def conv_wgrad(x: torch.Tensor, dy: torch.Tensor, km: KMap) -> torch.Tensor:
+    """dW[k] = sum over the pairs (o, i) of offset k of x[i]^T dy[o]  ->  fp32 [125,32,32]"""
+    lib = _lib.load()
+    n = x.shape[0]
+    dW = torch.empty((125, 32, 32), dtype=torch.float32, device=x.device)
+    ws_b = int(lib.gpc_spconv_wgrad_workspace_bytes(n, km.tile_rows))
+    ws = torch.empty(max(ws_b, 256), dtype=torch.uint8, device=x.device)
+    _lib.check(lib.gpc_spconv_wgrad_v6(_ptr(x), _ptr(dy), _ptr(km.seg), _ptr(km.pairs), n, km.tile_rows, _ptr(dW), _ptr(ws), ws_b,
+                                       _stream(x.device)), "gpc_spconv_wgrad_v6")
+    return dW
+
+
+class SparseConvFn(torch.autograd.Function):
+    """y = conv(x, W) on the kernel map km (a KMap of the mma.sync family); W is [125,32,32] or [27,32,32] (kernel_size 3: the
+    27 matrices go to their K = 5 offsets, where the map holds the only present neighbours, and their gradient is gathered back)."""
+
+    @staticmethod
+    def forward(ctx, x: torch.Tensor, Wk: torch.Tensor, km: KMap):
+        if km.pairs is None or km.um_rows or km.sparse:
+            raise _lib.GpcError("SparseConvFn runs on the mma.sync conv's kernel map (build_kmap(..., family='v6'))")
+        x = x.contiguous()
+        W125 = _to125(Wk.detach())
+        ctx.km, ctx.k3 = km, Wk.shape[0] == 27
+        ctx.save_for_backward(x, W125)
+        return conv_v6(x, pack_frag(W125), km)
+
+    @staticmethod
+    def backward(ctx, dy: torch.Tensor):
+        x, W125 = ctx.saved_tensors
+        dy = dy.contiguous()
+        dx = conv_dgrad(dy, W125, ctx.km) if ctx.needs_input_grad[0] else None
+        dW = None
+        if ctx.needs_input_grad[1]:
+            dW = conv_wgrad(x, dy, ctx.km)
+            if ctx.k3:
+                dW = dW[torch.tensor(K5_OF_K3, device=dW.device)]
+        return dx, dW, None
+
+
+def _to125(Wk: torch.Tensor) -> torch.Tensor:
+    if Wk.shape[0] == 125:
+        return Wk.contiguous()
+    full = torch.zeros((125, 32, 32), dtype=Wk.dtype, device=Wk.device)
+    full[torch.tensor(K5_OF_K3, device=Wk.device)] = Wk
+    return full
+
+
+class EmbedFn(torch.autograd.Function):
+    """table[idx]; the table's gradient is one_hot(idx)^T @ grad as one fp64 matrix product (a fixed summation order, where
+    torch's embedding backward accumulates rows with atomics)"""
+
+    @staticmethod
+    def forward(ctx, table: torch.Tensor, idx: torch.Tensor):
+        ctx.save_for_backward(idx)
+        ctx.rows = table.shape[0]
+        return table[idx]
+
+    @staticmethod
+    def backward(ctx, g: torch.Tensor):
+        (idx,) = ctx.saved_tensors
+        oh = (idx[:, None] == torch.arange(ctx.rows, device=idx.device)[None, :]).to(torch.float64)
+        return (oh.t() @ g.to(torch.float64)).to(g.dtype), None
+
+
+class ChildGatherFn(torch.autograd.Function):
+    """children's rows of the parents' features, F[parent]; the gradient of a parent is the sum of its <= 8 children's, added in
+    octant order (torch's index_select backward is an atomic index_add_)"""
+
+    @staticmethod
+    def forward(ctx, f: torch.Tensor, parent: torch.Tensor, octant: torch.Tensor):
+        n_child = parent.shape[0]
+        slot = torch.full((f.shape[0] * 8,), n_child, dtype=torch.int64, device=f.device)
+        slot[parent * 8 + octant] = torch.arange(n_child, device=f.device)
+        ctx.save_for_backward(slot.view(-1, 8))
+        return f[parent]
+
+    @staticmethod
+    def backward(ctx, g: torch.Tensor):
+        (slot,) = ctx.saved_tensors
+        gp = torch.cat([g, g.new_zeros((1, g.shape[1]))])
+        acc = gp[slot[:, 0]]
+        for o in range(1, 8):
+            acc = acc + gp[slot[:, o]]
+        return acc, None, None
+
+
+class _Geometry:
+    """what GausPcgcCodec reads of its weights when it only builds geometry: the kernel size of the map"""
+
+    def __init__(self, kernel_size: int):
+        self.kernel_size = kernel_size
+
+
+def _octant(keys: torch.Tensor) -> torch.Tensor:
+    return (keys & 1) | (((keys >> 21) & 1) << 1) | (((keys >> 42) & 1) << 2)
+
+
+class GausPcgcNet(nn.Module):
+    """The GausPcgc network with the reference's state_dict layout (weights.reference_layout(32, kernel_size)).  Starts from
+    `state_dict` (a checkpoint in that layout) or from make_synthetic_state_dict(seed).  fog.conv.kernel is a constant buffer."""
+
+    def __init__(self, kernel_size: int = 5, state_dict: Optional[Dict[str, torch.Tensor]] = None, seed: int = 5):
+        super().__init__()
+        if kernel_size not in (3, 5):
+            raise ValueError("kernel_size must be 3 or 5")
+        self.kernel_size = kernel_size
+        sd = state_dict if state_dict is not None else W.make_synthetic_state_dict(seed, 32, kernel_size)
+        W.validate_state_dict(sd, 32, kernel_size)
+        for name in W.reference_layout(32, kernel_size):
+            *path, leaf = name.split(".")
+            mod = self
+            for p in path:
+                if not hasattr(mod, p):
+                    mod.add_module(p, nn.Module())
+                mod = getattr(mod, p)
+            t = sd[name].detach().to(torch.float32).clone()
+            if name == "fog.conv.kernel":
+                mod.register_buffer(leaf, t)
+            else:
+                mod.register_parameter(leaf, nn.Parameter(t))
+        self._codec: Optional[GausPcgcCodec] = None
+
+    def codec(self, dev: torch.device) -> GausPcgcCodec:
+        if self._codec is None or self._codec.dev != dev:
+            self._codec = GausPcgcCodec(_Geometry(self.kernel_size), dev, ac_threads=1)
+        return self._codec
+
+    def geometry(self, xyz: torch.Tensor) -> List[Level]:
+        """the encoder's octree of a voxel cloud (GausPcgcCodec.encode): levels coarsest -> finest, each with its mma.sync kernel
+        map; levels[d + 1] are the children of levels[d] in (z, y, x) order"""
+        dev = next(self.parameters()).device
+        codec = self.codec(dev)
+        with torch.no_grad():
+            xyz = xyz.to(device=dev, dtype=torch.int32).contiguous()
+            keys, meta = codec.pack_keys(xyz)
+            meta_h = meta.cpu().numpy()
+            if meta_h[0] & 2:
+                xyz, _ = codec._recentre(xyz)
+                keys, meta = codec.pack_keys(xyz)
+                meta_h = meta.cpu().numpy()
+            mm = meta_h[2:8].astype(np.uint32)
+            levels = codec.build_pyramid(codec.sort_unique(keys, mm), mm.astype(np.int64))
+            for lv in levels:
+                lv.kmap = codec.build_kmap(lv.keys, family="v6")
+        return levels
+
+    def _stack(self, x: torch.Tensor, P: Dict[str, torch.Tensor], ids: Sequence[int], km: KMap) -> torch.Tensor:
+        cw = lambda i: P[W.CONV_KEYS[i]]
+        x = torch.relu(SparseConvFn.apply(x, cw(ids[0]), km))
+        for a, b in ((ids[1], ids[2]), (ids[3], ids[4])):
+            t = torch.relu(SparseConvFn.apply(x, cw(a), km))
+            x = torch.relu(SparseConvFn.apply(t, cw(b), km) + x)
+        return x
+
+    def forward(self, xyz: torch.Tensor, collect: bool = False) -> Dict[str, object]:
+        """xyz int [N,3] voxel coordinates -> {"bits": code length of the occupancy streams, sum of -log2 of the coder's
+        probability of every true symbol, (p * (65536 - A) + 1) / 65536 (fp32 scalar, differentiable),
+        "bpp": bits / N, "points": N, "levels": coded levels}; collect=True adds "probs": the softmax rows of every (level, stage)
+        in the codec's stream order (encode(..., collect=True)'s aux["probs"])."""
+        levels = self.geometry(xyz)
+        P = dict(self.named_parameters())
+        dev = levels[0].keys.device
+        bits = torch.zeros((), dtype=torch.float32, device=dev)
+        probs: List[torch.Tensor] = []
+        codec = self.codec(dev)
+        for d in range(len(levels) - 1):
+            parent, gt = levels[d], levels[d + 1]
+            with torch.no_grad():
+                _, cp = codec.expand(parent, gt.n)                     # children == gt.keys row for row
+                cp = cp.to(torch.int64)
+                occ = gt.occ.to(torch.int64)
+            f = EmbedFn.apply(P["prior_embedding.weight"], parent.occ.to(torch.int64))
+            f = self._stack(f, P, W.PRIOR_CONVS, parent.kmap)
+            u = ChildGatherFn.apply(f, cp, _octant(gt.keys)) + EmbedFn.apply(P["target_embedding.target_res_embedding.weight"], _octant(gt.keys))
+            u = self._stack(u, P, W.TARGET_CONVS, gt.kmap)
+            for i in range(4):
+                f = u if i == 0 else u + EmbedFn.apply(P[f"pred_head_s{i}_emb.weight"], occ >> CTX_SHIFT[i])
+                c0, c1 = W.stage_convs(i)
+                t = torch.relu(SparseConvFn.apply(f, P[W.CONV_KEYS[c0]], gt.kmap))
+                t = SparseConvFn.apply(t, P[W.CONV_KEYS[c1]], gt.kmap)
+                h = torch.relu(nn.functional.linear(t, P[f"pred_head_s{i}.0.weight"], P[f"pred_head_s{i}.0.bias"]))
+                logits = nn.functional.linear(h, P[f"pred_head_s{i}.2.weight"], P[f"pred_head_s{i}.2.bias"])
+                p = torch.softmax(logits, dim=1)
+                A = W.STAGE_ALPHABETS[i]
+                sym = (occ >> STAGE_SHIFT[i]) & STAGE_MASK[i]
+                hot = sym[:, None] == torch.arange(A, device=dev)[None, :]
+                # the coder's probability of the symbol: q[k] = round(cdf[k] * (65536 - A)) + k (kit/op.py) gives it
+                # (p * (65536 - A) + 1) / 65536 up to rounding, so a symbol never costs more than 16 bits
+                bits = bits - torch.log2(((p * hot).sum(1) * (65536 - A) + 1) / 65536).sum()
+                if collect:
+                    probs.append(p.detach())
+        n = int(xyz.shape[0])
+        out = {"bits": bits, "bpp": bits / max(n, 1), "points": n, "levels": len(levels) - 1}
+        if collect:
+            out["probs"] = probs
+        return out
+
+    def checkpoint(self) -> Dict[str, torch.Tensor]:
+        """state_dict in the reference layout, on the CPU (what torch.save writes and compress_point_cloud loads)"""
+        return {k: v.detach().to("cpu").clone() for k, v in self.state_dict().items()}
+
+
+def partition(xyz: torch.Tensor, max_points: int = 150_000) -> List[torch.Tensor]:
+    """kd-tree patches of a cloud: a patch of more than max_points points is split at its median along its longest axis (the first
+    such axis on ties), points of equal coordinate in input order.  Returns the row indices (int64, on xyz's device) of every patch,
+    left before right; every row is in exactly one patch.  Device-agnostic and deterministic."""
+    if max_points < 1:
+        raise ValueError("max_points must be >= 1")
+    n = int(xyz.shape[0])
+    out: List[torch.Tensor] = []
+    todo = [torch.arange(n, device=xyz.device)]
+    while todo:
+        idx = todo.pop()
+        if idx.numel() <= max_points:
+            if idx.numel():
+                out.append(idx)
+            continue
+        p = xyz[idx]
+        ext = (p.amax(0) - p.amin(0)).tolist()
+        axis = ext.index(max(ext))
+        srt = idx[torch.sort(p[:, axis], stable=True).indices]
+        half = idx.numel() // 2
+        todo.append(srt[half:])
+        todo.append(srt[:half])
+    return out
+
+
+def _load_init(init) -> Optional[Dict[str, torch.Tensor]]:
+    if init is None or isinstance(init, dict):
+        return init
+    return torch.load(init, map_location="cpu")
+
+
+def train(clouds: Sequence[torch.Tensor], ckpt_out: Optional[str] = None, init: Union[None, str, Dict[str, torch.Tensor]] = None,
+          steps: int = 1000, lr: float = 5e-4, seed: int = 0, kernel_size: int = 5, max_points: int = 150_000, save_every: int = 0,
+          synthetic_seed: int = 5, log: Optional[Callable[[Dict[str, float]], None]] = None):
+    """Train on voxel clouds (int [N,3] each): the clouds are cut into kd-tree patches of at most max_points points, and every
+    step codes one patch (the order a permutation per pass, drawn from `seed`) and takes one Adam step (lr 5e-4 as the reference)
+    on its bits per point.  Starts from `init` (checkpoint path or state_dict) or make_synthetic_state_dict(synthetic_seed).
+    Saves torch.save(state_dict) in the reference layout to ckpt_out every save_every steps (0: never) and at the end.
+    Returns (state_dict, rows) with one row {"step", "points", "bpp", "time"} per step; `log` is called with each row."""
+    if not torch.cuda.is_available():
+        raise _lib.GpcError("training needs a CUDA device (B200, sm_100a); there is no CPU fallback")
+    dev = torch.device("cuda", torch.cuda.current_device())
+    patches: List[torch.Tensor] = []
+    for c in clouds:
+        xyz = c.to(device=dev, dtype=torch.int32)
+        patches += [xyz[i].contiguous() for i in partition(xyz, max_points)]
+    if not patches:
+        raise ValueError("no points to train on")
+    net = GausPcgcNet(kernel_size, _load_init(init), synthetic_seed).to(dev)
+    opt = torch.optim.Adam(net.parameters(), lr=lr)
+    gen = torch.Generator().manual_seed(int(seed))
+    order: List[int] = []
+    rows: List[Dict[str, float]] = []
+    t0 = time.time()
+    for step in range(1, steps + 1):
+        if not order:
+            order = torch.randperm(len(patches), generator=gen).tolist()
+        xyz = patches[order.pop(0)]
+        opt.zero_grad(set_to_none=True)
+        out = net(xyz)
+        if out["bpp"].requires_grad:
+            out["bpp"].backward()
+            opt.step()
+        row = {"step": step, "points": int(xyz.shape[0]), "bpp": float(out["bpp"].detach()), "time": time.time() - t0}
+        rows.append(row)
+        if log is not None:
+            log(row)
+        if ckpt_out and save_every and step % save_every == 0 and step < steps:
+            torch.save(net.checkpoint(), ckpt_out)
+    sd = net.checkpoint()
+    if ckpt_out:
+        torch.save(sd, ckpt_out)
+    return sd, rows

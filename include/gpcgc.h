@@ -168,6 +168,16 @@ int gpc_spconv_fwd_v6_range(const float *x, const void *Wa, const uint32_t *seg,
                             int64_t row0, int64_t row1, int tile_rows, const float *residual, int flags, float *y,
                             int variant, void *stream);
 
+/* ---- training (spconv_grad.cu): weight gradient of gpc_spconv_fwd_v6 over the same pair stream (pad = 8) and tiling ----
+ * dW[k][ci][co] = sum over the pairs (o, i) of offset k of x[i][ci] * dy[o][co]; x, dy fp32 [n,32], dW fp32 [125,32,32] (every offset
+ * is written; offsets without pairs give exact zeros).  bf16 hi / lo split, three terms, fp32 accumulation as the forward; no atomics,
+ * the summation order depends on (n, tile_rows) and the map only.  ws: gpc_spconv_wgrad_workspace_bytes(n, tile_rows) bytes.
+ * The input gradient is gpc_spconv_fwd_v6 itself with W'[k] = W[124 - k]^T (a submanifold map is symmetric: nbr_k(o) = i <=>
+ * nbr_{124-k}(i) = o). */
+size_t gpc_spconv_wgrad_workspace_bytes(int64_t n, int tile_rows);
+int gpc_spconv_wgrad_v6(const float *x, const float *dy, const uint32_t *seg, const uint64_t *pairs, int64_t n, int tile_rows,
+                        float *dW, void *ws, size_t ws_bytes, void *stream);
+
 /* ---- the conv of the SPARSE big levels (spconv_sparse.cu): dense centre product + offset-sorted "stragglers" ----
  * For levels with ~1-4 neighbours per row (the finest octree levels).  Sparse map: seg u32[gpc_kmap_sparse_segments(n) + 1]
  * (first entry of every (block of 8192 rows, offset != centre) segment, padded to 8 entries), pairs u64[entries] = nbr | dst << 32
