@@ -26,7 +26,7 @@ launch over all members' rows and the symbol merge -- no CDF row leaves the GPU 
 from __future__ import annotations
 
 from dataclasses import dataclass, field
-from typing import List, Optional, Sequence, Tuple
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -137,6 +137,31 @@ class ULevel:
     @property
     def n(self) -> int:
         return int(self.keys.shape[0])
+
+
+def union_levels(levels: Sequence[Sequence[Level]], tz: Sequence[int]) -> Tuple[Dict[int, ULevel], Dict[int, int], Dict[int, int]]:
+    """The union levels of the members of one union (plan_unions order, deepest first).  levels[j]: member j's pyramid, coarsest
+    first (its base voxels are 2^len(levels[j]) leaves wide); tz[j]: its z translation in leaf voxels.  Returns (U, K, M):
+      U[sg]  for sg = 1 .. D (1 = parents of the leaves): the members' levels at scale sg, keys translated by tz >> sg, one after the
+             other, with each member's row range (kernel maps not built)
+      K[sg]  for sg = 1 .. D - 1: the members with a level at scale sg + 1, i.e. those whose rows at scale sg are children (a prefix)
+      M[sg]  their rows: the first M[sg] rows of U[sg]."""
+    depths = [len(lv) for lv in levels]
+    D = max(depths)
+    U: Dict[int, ULevel] = {}
+    for sg in range(1, D + 1):
+        part = [j for j, d in enumerate(depths) if d >= sg]
+        keys, occs, ranges, r = [], [], [], 0
+        for j in part:
+            lvl = levels[j][depths[j] - sg]
+            keys.append(BatchCodec._translate(lvl.keys, tz[j] >> sg))
+            occs.append(lvl.occ)
+            ranges.append((r, r + lvl.n))
+            r += lvl.n
+        U[sg] = ULevel(torch.cat(keys), torch.cat(occs), part, ranges)
+    K = {sg: sum(1 for d in depths if d >= sg + 1) for sg in range(1, D)}
+    M = {sg: U[sg].ranges[K[sg] - 1][1] for sg in range(1, D)}
+    return U, K, M
 
 
 @dataclass
@@ -454,25 +479,12 @@ class BatchCodec:
     def _encode_union(self, members: List[_Scene], gpu_chunk: int = 0) -> List[List[bytes]]:
         c = self.c
         D = max(sc.depth for sc in members)
-        # U[sigma]: the members' levels at scale sigma (1 = parents of the leaves), translated; deepest scenes first = a prefix
-        U = {}
-        for sg in range(1, D + 1):
-            part = [(j, sc) for j, sc in enumerate(members) if sc.depth >= sg]
-            keys, occs, ranges, r = [], [], [], 0
-            for j, sc in part:
-                lvl = sc.levels[sc.depth - sg]
-                keys.append(self._translate(lvl.keys, sc.tz >> sg))
-                occs.append(lvl.occ)
-                ranges.append((r, r + lvl.n))
-                r += lvl.n
-            U[sg] = ULevel(torch.cat(keys), torch.cat(occs), [j for j, _ in part], ranges)
+        U, K, M = union_levels([sc.levels for sc in members], [sc.tz for sc in members])
         for sg in range(1, D + 1):
             # scale 1 is only ever a child level: the members with deeper levels (all of them: base-only scenes are not in unions)
             U[sg].kmaps = self._kmaps(U[sg])
         streams: List[List[Optional[bytes]]] = [[None] * (4 * (sc.depth - 1)) for sc in members]
         futs = []
-        K = {sg: sum(1 for sc in members if sc.depth >= sg + 1) for sg in range(1, D)}     # members with children at scale sg
-        M = {sg: U[sg].ranges[K[sg] - 1][1] for sg in range(1, D)}                         # = the first M rows of U[sg]
         if gpu_chunk:
             # version 2: the (scene, level, stage) streams in the order (union level, stage, member) in the codec's coder arena, so
             # that the words of one stage of a union level (its first M rows, member after member) are one contiguous slot

@@ -13,6 +13,13 @@
 // terms hi.lo + lo.hi + hi.hi are accumulated in fp32, as in the forward (DESIGN.md 5).  The four warps' sums are added in warp
 // order, each group writes its partial to the workspace and a second kernel adds the groups in group order: no atomics, and the
 // summation order depends on (n, tile_rows) and the map only, so two calls give the same bits.
+//
+// The balanced variant (gpc_spconv_wgrad_v6_balanced) splits the same work by pairs instead of by tiles.  On the sparse finest levels
+// nearly every pair belongs to the centre offset, and 64 groups of tiles leave that offset as 256 serial chains of 8-pair units.
+// Here a plan kernel counts every offset's units per tile (ucum[k][tiles + 1], running sums), every offset's units are cut into
+// chunks of WGB_UNITS consecutive units (a chunk never spans two offsets), and one warp per chunk walks its units across tiles with
+// the same MMA body.  The chunk partials of an offset are added in chunk order by a fixed tree of fan-in WGB_FANIN (the tree's
+// shape depends on the chunk counts only).  No atomics, nothing is read back: the grid is sized from the entry count.
 #include "common.cuh"
 
 constexpr int WG_WARPS = 4;
@@ -29,6 +36,38 @@ __device__ __forceinline__ void mma_bf16_k8(float (&d)[4], u32 a0, u32 a1, u32 b
     asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5}, {%6}, {%0,%1,%2,%3};"
                  : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
                  : "r"(a0), "r"(a1), "r"(b0));
+}
+
+// one 8-entry unit of the pair stream at p (output rows of the unit's tile start at obase): acc += x^T dy over its pairs
+__device__ __forceinline__ void wgrad_unit(float (&acc)[2][4][4], const float *__restrict__ x, const float *__restrict__ dy,
+                                           const u64 *__restrict__ pairs, u32 p, i64 obase, int g, int t) {
+    // lane (g, t) holds pairs 2t and 2t + 1 of the unit, channels g + 8 j of their x and dy rows
+    const u64 ea = __ldg(pairs + p + 2 * t), eb = __ldg(pairs + p + 2 * t + 1);
+    const u32 na = (u32)ea, nb = (u32)eb;
+    float xa[4], xb[4], da[4], db[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) xa[j] = xb[j] = da[j] = db[j] = 0.f;
+    if (na != 0xFFFFFFFFu) {
+        const float *xr = x + (i64)na * GPC_C + g, *dr = dy + (obase + (i64)((ea >> 32) & 0xFFFFu)) * GPC_C + g;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { xa[j] = __ldg(xr + 8 * j); da[j] = __ldg(dr + 8 * j); }
+    }
+    if (nb != 0xFFFFFFFFu) {
+        const float *xr = x + (i64)nb * GPC_C + g, *dr = dy + (obase + (i64)((eb >> 32) & 0xFFFFu)) * GPC_C + g;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { xb[j] = __ldg(xr + 8 * j); db[j] = __ldg(dr + 8 * j); }
+    }
+    u32 ah[4], al[4], bh[4], bl[4];                      // A: (ci g + 8 j, pairs 2t, 2t + 1); B: (pairs 2t, 2t + 1, co g + 8 j)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) { split_bf16(xa[j], xb[j], ah[j], al[j]); split_bf16(da[j], db[j], bh[j], bl[j]); }
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt) {
+            mma_bf16_k8(acc[mt][nt], ah[2 * mt], ah[2 * mt + 1], bl[nt]);
+            mma_bf16_k8(acc[mt][nt], al[2 * mt], al[2 * mt + 1], bh[nt]);
+            mma_bf16_k8(acc[mt][nt], ah[2 * mt], ah[2 * mt + 1], bh[nt]);
+        }
 }
 
 // partial[grp][k][ci][co] of the tiles [grp * tiles / G, (grp + 1) * tiles / G)
@@ -49,35 +88,7 @@ __global__ void __launch_bounds__(32 * WG_WARPS) spconv_wgrad_partial_kernel(con
         const u32 p0 = __ldg(seg + tile * (GPC_K3 + 1) + k), p1 = __ldg(seg + tile * (GPC_K3 + 1) + k + 1);
         const i64 obase = tile * tile_rows;
 #pragma unroll 2
-        for (u32 p = p0; p < p1; p += 8) {
-            // lane (g, t) holds pairs 2t and 2t + 1 of the unit, channels g + 8 j of their x and dy rows
-            const u64 ea = __ldg(pairs + p + 2 * t), eb = __ldg(pairs + p + 2 * t + 1);
-            const u32 na = (u32)ea, nb = (u32)eb;
-            float xa[4], xb[4], da[4], db[4];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) xa[j] = xb[j] = da[j] = db[j] = 0.f;
-            if (na != 0xFFFFFFFFu) {
-                const float *xr = x + (i64)na * GPC_C + g, *dr = dy + (obase + (i64)((ea >> 32) & 0xFFFFu)) * GPC_C + g;
-#pragma unroll
-                for (int j = 0; j < 4; ++j) { xa[j] = __ldg(xr + 8 * j); da[j] = __ldg(dr + 8 * j); }
-            }
-            if (nb != 0xFFFFFFFFu) {
-                const float *xr = x + (i64)nb * GPC_C + g, *dr = dy + (obase + (i64)((eb >> 32) & 0xFFFFu)) * GPC_C + g;
-#pragma unroll
-                for (int j = 0; j < 4; ++j) { xb[j] = __ldg(xr + 8 * j); db[j] = __ldg(dr + 8 * j); }
-            }
-            u32 ah[4], al[4], bh[4], bl[4];              // A: (ci g + 8 j, pairs 2t, 2t + 1); B: (pairs 2t, 2t + 1, co g + 8 j)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) { split_bf16(xa[j], xb[j], ah[j], al[j]); split_bf16(da[j], db[j], bh[j], bl[j]); }
-#pragma unroll
-            for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-                for (int nt = 0; nt < 4; ++nt) {
-                    mma_bf16_k8(acc[mt][nt], ah[2 * mt], ah[2 * mt + 1], bl[nt]);
-                    mma_bf16_k8(acc[mt][nt], al[2 * mt], al[2 * mt + 1], bh[nt]);
-                    mma_bf16_k8(acc[mt][nt], ah[2 * mt], ah[2 * mt + 1], bh[nt]);
-                }
-        }
+        for (u32 p = p0; p < p1; p += 8) wgrad_unit(acc, x, dy, pairs, p, obase, g, t);
     }
     // D fragment: [0] = (ci 16mt + g, co 8nt + 2t), [1] = co + 1, [2] / [3] = ci + 8
 #pragma unroll
@@ -128,6 +139,206 @@ extern "C" int gpc_spconv_wgrad_v6(const float *x, const float *dy, const uint32
     spconv_wgrad_partial_kernel<<<dim3(GPC_K3, G), 32 * WG_WARPS, 0, st>>>(x, dy, seg, pairs, tiles, tile_rows, (float *)ws);
     GPC_LAUNCH_CHECK();
     spconv_wgrad_reduce_kernel<<<cdiv((i64)GPC_K3 * GPC_C * GPC_C, 256), 256, 0, st>>>((const float *)ws, G, dW);
+    GPC_LAUNCH_CHECK();
+    return GPC_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------- balanced by pairs
+#ifndef WGB_UNITS
+#define WGB_UNITS 4                                      // 8-entry units per chunk (one warp), the fastest of 4..64 measured
+#endif
+constexpr int WGB_WARPS = 4;                             // independent warps (chunks) per CTA of the partial kernel
+constexpr int WGB_FANIN = 32;                            // partials added per step of the reduction tree
+
+// the balanced kernel's workspace: ucum u32[125][tiles + 1], plan i32[levels + 1][126] (per tree level the exclusive prefix of
+// every offset's partial count; level 0 = the chunks), then per tree level its partials [count bound][32 * 32] fp32.
+struct WgbLayout {
+    i64 tiles = 0;
+    int levels = 0;                                      // tree steps before the final one; then <= WGB_FANIN partials per offset
+    size_t ucum = 0, plan = 0, part[8] = {}, bytes = 0;
+    i64 bound[8] = {};                                   // partials of each level, at most
+};
+
+static inline size_t wgb_align(size_t b) { return (b + 255) / 256 * 256; }
+
+static WgbLayout wgb_layout(i64 n, int tile_rows, i64 n_entries) {
+    WgbLayout L;
+    L.tiles = (n + tile_rows - 1) / tile_rows;
+    const i64 units = (n_entries + 7) / 8;
+    L.bound[0] = GPC_K3 + (units + WGB_UNITS - 1) / WGB_UNITS;     // sum over offsets of ceil(units_k / U)
+    i64 per_offset = (units + WGB_UNITS - 1) / WGB_UNITS;          // chunks of one offset, at most
+    while (per_offset > WGB_FANIN) {
+        per_offset = (per_offset + WGB_FANIN - 1) / WGB_FANIN;
+        L.bound[L.levels + 1] = GPC_K3 + (L.bound[L.levels] + WGB_FANIN - 1) / WGB_FANIN;
+        ++L.levels;
+    }
+    size_t off = 0;
+    L.ucum = off; off = wgb_align(off + (size_t)GPC_K3 * (L.tiles + 1) * sizeof(u32));
+    L.plan = off; off = wgb_align(off + (size_t)(L.levels + 1) * (GPC_K3 + 1) * sizeof(int));
+    for (int l = 0; l <= L.levels; ++l) { L.part[l] = off; off = wgb_align(off + (size_t)L.bound[l] * GPC_C * GPC_C * sizeof(float)); }
+    L.bytes = off;
+    return L;
+}
+
+// ucum[k][t] = units of offset k in the tiles before t; one CTA per offset, a block scan over the tiles
+__global__ void __launch_bounds__(1024) spconv_wgrad_units_kernel(const u32 *__restrict__ seg, i64 tiles, u32 *__restrict__ ucum) {
+    __shared__ u32 wsum[32];
+    const int k = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    u32 *out = ucum + (i64)k * (tiles + 1);
+    if (threadIdx.x == 0) out[0] = 0;
+    u32 carry = 0;
+    for (i64 base = 0; base < tiles; base += 1024) {
+        const i64 tile = base + threadIdx.x;
+        u32 v = tile < tiles ? (__ldg(seg + tile * (GPC_K3 + 1) + k + 1) - __ldg(seg + tile * (GPC_K3 + 1) + k)) >> 3 : 0u;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const u32 o = __shfl_up_sync(0xFFFFFFFFu, v, d);
+            if (lane >= d) v += o;
+        }
+        if (lane == 31) wsum[wid] = v;
+        __syncthreads();
+        u32 before = carry;
+        for (int w = 0; w < wid; ++w) before += wsum[w];
+        if (tile < tiles) out[tile + 1] = before + v;
+        u32 total = 0;
+#pragma unroll
+        for (int w = 0; w < 32; ++w) total += wsum[w];
+        carry += total;
+        __syncthreads();
+    }
+}
+
+// plan[0][k] = first chunk of offset k (chunks of WGB_UNITS units), plan[l][k] = first partial of offset k at tree level l.
+// The counts are read in parallel; one thread scans them in shared memory.
+__global__ void __launch_bounds__(128) spconv_wgrad_plan_kernel(const u32 *__restrict__ ucum, i64 tiles, int levels,
+                                                                int *__restrict__ plan) {
+    __shared__ int cnt[GPC_K3], first[8][GPC_K3 + 1];
+    const int k = threadIdx.x;
+    if (k < GPC_K3) cnt[k] = (int)((__ldg(ucum + (i64)k * (tiles + 1) + tiles) + WGB_UNITS - 1) / WGB_UNITS);
+    __syncthreads();
+    if (k == 0) {
+        for (int l = 0; l <= levels; ++l) {
+            int c = 0;
+            for (int j = 0; j < GPC_K3; ++j) {
+                first[l][j] = c;
+                c += l == 0 ? cnt[j] : (first[l - 1][j + 1] - first[l - 1][j] + WGB_FANIN - 1) / WGB_FANIN;
+            }
+            first[l][GPC_K3] = c;
+        }
+    }
+    __syncthreads();
+    for (int l = 0; l <= levels; ++l)
+        if (k <= GPC_K3) plan[l * (GPC_K3 + 1) + k] = first[l][k];
+}
+
+// largest k in [0, 125) with first[k] <= i (first[] ascending): the offset whose partials hold index i
+__device__ __forceinline__ int wgb_offset_of(const int *__restrict__ first, int i) {
+    int lo = 0, hi = GPC_K3;
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (__ldg(first + mid) <= i) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
+// one warp per chunk: units [j U, (j + 1) U) of offset k, walked across tiles -> partial[chunk][ci][co]
+__global__ void __launch_bounds__(32 * WGB_WARPS) spconv_wgrad_chunk_kernel(const float *__restrict__ x, const float *__restrict__ dy,
+                                                                           const u32 *__restrict__ seg, const u64 *__restrict__ pairs,
+                                                                           i64 tiles, int tile_rows, const u32 *__restrict__ ucum,
+                                                                           const int *__restrict__ plan, float *__restrict__ partial) {
+    const int chunk = blockIdx.x * WGB_WARPS + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+    if (chunk >= __ldg(plan + GPC_K3)) return;          // surplus warps of the host-sized grid
+    const int k = wgb_offset_of(plan, chunk);
+    const u32 *uc = ucum + (i64)k * (tiles + 1);
+    u32 u = (u32)(chunk - __ldg(plan + k)) * WGB_UNITS;
+    const u32 uend = min(u + (u32)WGB_UNITS, __ldg(uc + tiles));
+    i64 lo = 0, hi = tiles;                              // the tile holding unit u: largest tile with uc[tile] <= u
+    while (hi - lo > 1) {
+        const i64 mid = (lo + hi) >> 1;
+        if (__ldg(uc + mid) <= u) lo = mid; else hi = mid;
+    }
+    float acc[2][4][4];
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt) acc[mt][nt][0] = acc[mt][nt][1] = acc[mt][nt][2] = acc[mt][nt][3] = 0.f;
+    for (i64 tile = lo; u < uend; ++tile) {
+        const u32 first = __ldg(uc + tile), stop = min(uend, __ldg(uc + tile + 1));
+        u32 p = __ldg(seg + tile * (GPC_K3 + 1) + k) + 8 * (u - first);
+        const i64 obase = tile * tile_rows;
+#pragma unroll 2
+        for (; u < stop; ++u, p += 8) wgrad_unit(acc, x, dy, pairs, p, obase, g, t);
+    }
+    float *out = partial + (i64)chunk * (GPC_C * GPC_C);
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt) {
+            float *r = out + (16 * mt + g) * GPC_C + 8 * nt + 2 * t;
+            *reinterpret_cast<float2 *>(r) = make_float2(acc[mt][nt][0], acc[mt][nt][1]);
+            *reinterpret_cast<float2 *>(r + 8 * GPC_C) = make_float2(acc[mt][nt][2], acc[mt][nt][3]);
+        }
+}
+
+// one step of the tree: output partial i of offset k = the sum, in order, of its inputs [j F, (j + 1) F) (j = i - first_out[k]).
+// final: one CTA per offset writes dW[k] (+0 for an offset without partials)
+__global__ void __launch_bounds__(256) spconv_wgrad_tree_kernel(const float *__restrict__ in, const int *__restrict__ first_in,
+                                                               const int *__restrict__ first_out, float *__restrict__ out, int final_) {
+    int k, i;
+    if (final_) {
+        k = blockIdx.x;
+        i = k;
+    } else {
+        i = blockIdx.x;
+        if (i >= __ldg(first_out + GPC_K3)) return;
+        k = wgb_offset_of(first_out, i);
+    }
+    const int a0 = __ldg(first_in + k), a1 = __ldg(first_in + k + 1);
+    const int j = final_ ? 0 : i - __ldg(first_out + k);
+    const int b0 = a0 + j * WGB_FANIN, b1 = final_ ? a1 : min(a1, b0 + WGB_FANIN);
+    float *o = out + (i64)i * (GPC_C * GPC_C);
+    for (int e = threadIdx.x; e < GPC_C * GPC_C; e += 256) {
+        float v = 0.f;
+        for (int b = b0; b < b1; ++b) v += in[(i64)b * (GPC_C * GPC_C) + e];
+        o[e] = v;
+    }
+}
+
+extern "C" size_t gpc_spconv_wgrad_balanced_workspace_bytes(int64_t n, int tile_rows, int64_t n_entries) {
+    if (n <= 0 || tile_rows <= 0 || n_entries < 0) return 0;
+    return wgb_layout(n, tile_rows, n_entries).bytes;
+}
+
+extern "C" int gpc_spconv_wgrad_v6_balanced(const float *x, const float *dy, const uint32_t *seg, const uint64_t *pairs, int64_t n,
+                                            int tile_rows, int64_t n_entries, float *dW, void *ws, size_t ws_bytes, void *stream) {
+    GPC_REQUIRE(n >= 0, GPC_EINVAL, "n < 0");
+    GPC_REQUIRE(tile_rows == 8 || tile_rows == 16 || tile_rows == 32 || tile_rows == 64 || tile_rows == 128, GPC_EINVAL,
+                "tile_rows must be 8, 16, 32, 64 or 128 (the mma.sync conv's tile heights)");
+    GPC_REQUIRE(n_entries >= 0 && n_entries <= 0xFFFFFFFFll, GPC_EINVAL, "n_entries outside [0, 2^32)");
+    cudaStream_t st = as_stream(stream);
+    if (n == 0) {
+        GPC_CUDA_CHECK(cudaMemsetAsync(dW, 0, (size_t)GPC_K3 * GPC_C * GPC_C * sizeof(float), st));
+        return GPC_OK;
+    }
+    const WgbLayout L = wgb_layout(n, tile_rows, n_entries);
+    GPC_REQUIRE(ws_bytes >= L.bytes, GPC_ENOSPC, "wgrad workspace too small");
+    char *w = (char *)ws;
+    u32 *ucum = (u32 *)(w + L.ucum);
+    int *plan = (int *)(w + L.plan);
+    spconv_wgrad_units_kernel<<<GPC_K3, 1024, 0, st>>>(seg, L.tiles, ucum);
+    GPC_LAUNCH_CHECK();
+    spconv_wgrad_plan_kernel<<<1, 128, 0, st>>>(ucum, L.tiles, L.levels, plan);
+    GPC_LAUNCH_CHECK();
+    spconv_wgrad_chunk_kernel<<<cdiv(L.bound[0], WGB_WARPS), 32 * WGB_WARPS, 0, st>>>(x, dy, seg, pairs, L.tiles, tile_rows, ucum, plan,
+                                                                                     (float *)(w + L.part[0]));
+    GPC_LAUNCH_CHECK();
+    for (int l = 1; l <= L.levels; ++l) {
+        spconv_wgrad_tree_kernel<<<(unsigned)L.bound[l], 256, 0, st>>>((const float *)(w + L.part[l - 1]), plan + (l - 1) * (GPC_K3 + 1),
+                                                                       plan + l * (GPC_K3 + 1), (float *)(w + L.part[l]), 0);
+        GPC_LAUNCH_CHECK();
+    }
+    spconv_wgrad_tree_kernel<<<GPC_K3, 256, 0, st>>>((const float *)(w + L.part[L.levels]), plan + L.levels * (GPC_K3 + 1), nullptr, dW, 1);
     GPC_LAUNCH_CHECK();
     return GPC_OK;
 }

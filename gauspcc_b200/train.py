@@ -2,12 +2,14 @@
 
     SparseConvFn   autograd of one 5^3 sparse conv on the mma.sync family: forward gpc_spconv_fwd_v6, input gradient the same kernel
                    with the mirrored, transposed weights W'[k] = W[124 - k]^T (a submanifold map is symmetric: nbr_k(o) = i exactly
-                   when nbr_{124-k}(i) = o), weight gradient gpc_spconv_wgrad_v6 (csrc/spconv_grad.cu)
+                   when nbr_{124-k}(i) = o), weight gradient gpc_spconv_wgrad_v6, or gpc_spconv_wgrad_v6_balanced on levels of at
+                   least GausPcgcNet.wgrad_balanced_min_rows rows (csrc/spconv_grad.cu)
+    WeightPack     one conv weight's fragment packs, built once per forward pass and shared by every conv on every level
     GausPcgcNet    the model of SURVEY.md Appendix A as an nn.Module whose state_dict() is the reference layout
                    (weights.reference_layout); forward(xyz) returns the code length of the file's occupancy streams under the
-                   coder's probabilities
+                   coder's probabilities; forward_batch(patches) the same for many patches, run as union octrees (batch.py)
     partition      kd-tree patches (median split along the longest axis), the patching of the reference's dataset.py
-    train          Adam over patches, checkpoints in the reference layout
+    train          Adam over minibatches of patches, checkpoints in the reference layout
 
 The geometry (pyramid, children, kernel maps) comes from GausPcgcCodec exactly as the encoder builds it, so a checkpoint trained here
 is trained on the voxels, row orders and conv offsets it is later coded with: it loads with pcc_utils.compress_point_cloud unchanged.
@@ -20,7 +22,7 @@ fixed-order sums instead.  No process-wide torch flag is touched.
 from __future__ import annotations
 
 import time
-from typing import Callable, Dict, List, Optional, Sequence, Union
+from typing import Callable, Dict, Iterator, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -28,6 +30,7 @@ from torch import nn
 
 from . import _lib
 from . import weights as W
+from .batch import plan_unions, union_levels
 from .codec import CTX_SHIFT, STAGE_MASK, STAGE_SHIFT, GausPcgcCodec, KMap, Level, _ptr
 
 # the 27 offsets of a 3^3 kernel at their K = 5 indices ((dz+2)*5 + (dy+2))*5 + (dx+2), as DeviceWeights places them
@@ -58,11 +61,18 @@ def conv_dgrad(dy: torch.Tensor, W125: torch.Tensor, km: KMap) -> torch.Tensor:
     return conv_v6(dy, pack_frag(W125.flip(0).transpose(1, 2).contiguous()), km)
 
 
-def conv_wgrad(x: torch.Tensor, dy: torch.Tensor, km: KMap) -> torch.Tensor:
-    """dW[k] = sum over the pairs (o, i) of offset k of x[i]^T dy[o]  ->  fp32 [125,32,32]"""
+def conv_wgrad(x: torch.Tensor, dy: torch.Tensor, km: KMap, balanced: bool = False) -> torch.Tensor:
+    """dW[k] = sum over the pairs (o, i) of offset k of x[i]^T dy[o]  ->  fp32 [125,32,32]; balanced: gpc_spconv_wgrad_v6_balanced
+    (the work split by pairs, for big levels) instead of gpc_spconv_wgrad_v6 (split by tiles)"""
     lib = _lib.load()
     n = x.shape[0]
     dW = torch.empty((125, 32, 32), dtype=torch.float32, device=x.device)
+    if balanced:
+        ws_b = int(lib.gpc_spconv_wgrad_balanced_workspace_bytes(n, km.tile_rows, km.n_pairs))
+        ws = torch.empty(max(ws_b, 256), dtype=torch.uint8, device=x.device)
+        _lib.check(lib.gpc_spconv_wgrad_v6_balanced(_ptr(x), _ptr(dy), _ptr(km.seg), _ptr(km.pairs), n, km.tile_rows, km.n_pairs, _ptr(dW),
+                                                    _ptr(ws), ws_b, _stream(x.device)), "gpc_spconv_wgrad_v6_balanced")
+        return dW
     ws_b = int(lib.gpc_spconv_wgrad_workspace_bytes(n, km.tile_rows))
     ws = torch.empty(max(ws_b, 256), dtype=torch.uint8, device=x.device)
     _lib.check(lib.gpc_spconv_wgrad_v6(_ptr(x), _ptr(dy), _ptr(km.seg), _ptr(km.pairs), n, km.tile_rows, _ptr(dW), _ptr(ws), ws_b,
@@ -70,31 +80,51 @@ def conv_wgrad(x: torch.Tensor, dy: torch.Tensor, km: KMap) -> torch.Tensor:
     return dW
 
 
+class WeightPack:
+    """One conv weight (a [125|27,32,32] parameter) prepared for the kernels: W125, its forward fragment pack, and (built on first
+    use by a backward pass) the pack of the mirrored weights W125.flip(0).transpose(1, 2).  Built once per forward pass of the
+    network, so every conv on every level reuses the same bytes the per-call packs would have been."""
+
+    def __init__(self, Wk: torch.Tensor, wgrad_balanced_min_rows: Optional[int] = None):
+        self.W125 = _to125(Wk.detach())
+        self.fwd = pack_frag(self.W125)
+        self._mirror: Optional[torch.Tensor] = None
+        self.wgrad_balanced_min_rows = wgrad_balanced_min_rows     # None: every level takes gpc_spconv_wgrad_v6
+
+    def mirror(self) -> torch.Tensor:
+        if self._mirror is None:
+            self._mirror = pack_frag(self.W125.flip(0).transpose(1, 2).contiguous())
+        return self._mirror
+
+
 class SparseConvFn(torch.autograd.Function):
     """y = conv(x, W) on the kernel map km (a KMap of the mma.sync family); W is [125,32,32] or [27,32,32] (kernel_size 3: the
-    27 matrices go to their K = 5 offsets, where the map holds the only present neighbours, and their gradient is gathered back)."""
+    27 matrices go to their K = 5 offsets, where the map holds the only present neighbours, and their gradient is gathered back).
+    pack: W's WeightPack (built from W when not given)."""
 
     @staticmethod
-    def forward(ctx, x: torch.Tensor, Wk: torch.Tensor, km: KMap):
+    def forward(ctx, x: torch.Tensor, Wk: torch.Tensor, km: KMap, pack: Optional[WeightPack] = None):
         if km.pairs is None or km.um_rows or km.sparse:
             raise _lib.GpcError("SparseConvFn runs on the mma.sync conv's kernel map (build_kmap(..., family='v6'))")
         x = x.contiguous()
-        W125 = _to125(Wk.detach())
-        ctx.km, ctx.k3 = km, Wk.shape[0] == 27
-        ctx.save_for_backward(x, W125)
-        return conv_v6(x, pack_frag(W125), km)
+        pack = pack if pack is not None else WeightPack(Wk)
+        ctx.km, ctx.k3, ctx.pack = km, Wk.shape[0] == 27, pack
+        ctx.save_for_backward(x)
+        return conv_v6(x, pack.fwd, km)
 
     @staticmethod
     def backward(ctx, dy: torch.Tensor):
-        x, W125 = ctx.saved_tensors
+        (x,) = ctx.saved_tensors
+        pack, km = ctx.pack, ctx.km
         dy = dy.contiguous()
-        dx = conv_dgrad(dy, W125, ctx.km) if ctx.needs_input_grad[0] else None
+        dx = conv_v6(dy, pack.mirror(), km) if ctx.needs_input_grad[0] else None
         dW = None
         if ctx.needs_input_grad[1]:
-            dW = conv_wgrad(x, dy, ctx.km)
+            lim = pack.wgrad_balanced_min_rows
+            dW = conv_wgrad(x, dy, km, balanced=lim is not None and x.shape[0] >= lim)
             if ctx.k3:
                 dW = dW[torch.tensor(K5_OF_K3, device=dW.device)]
-        return dx, dW, None
+        return dx, dW, None, None
 
 
 def _to125(Wk: torch.Tensor) -> torch.Tensor:
@@ -155,6 +185,12 @@ def _octant(keys: torch.Tensor) -> torch.Tensor:
     return (keys & 1) | (((keys >> 21) & 1) << 1) | (((keys >> 42) & 1) << 2)
 
 
+# Levels of at least this many rows take the balanced weight gradient (gpc_spconv_wgrad_v6_balanced): the crossover measured on
+# sparse finest levels (profiles/r07_train_batch.md), and above 150 000 in any case: a patch of at most 150 000 points has no level
+# that large, so single-patch training keeps gpc_spconv_wgrad_v6 and its bits.
+WGRAD_BALANCED_MIN_ROWS = 600_000
+
+
 class GausPcgcNet(nn.Module):
     """The GausPcgc network with the reference's state_dict layout (weights.reference_layout(32, kernel_size)).  Starts from
     `state_dict` (a checkpoint in that layout) or from make_synthetic_state_dict(seed).  fog.conv.kernel is a constant buffer."""
@@ -179,15 +215,17 @@ class GausPcgcNet(nn.Module):
             else:
                 mod.register_parameter(leaf, nn.Parameter(t))
         self._codec: Optional[GausPcgcCodec] = None
+        self.wgrad_balanced_min_rows = WGRAD_BALANCED_MIN_ROWS
+        # rows of the finest level of one union in forward_batch (plan_unions' row cap); a bigger batch runs as several unions
+        self.union_max_rows = 4_000_000
 
     def codec(self, dev: torch.device) -> GausPcgcCodec:
         if self._codec is None or self._codec.dev != dev:
             self._codec = GausPcgcCodec(_Geometry(self.kernel_size), dev, ac_threads=1)
         return self._codec
 
-    def geometry(self, xyz: torch.Tensor) -> List[Level]:
-        """the encoder's octree of a voxel cloud (GausPcgcCodec.encode): levels coarsest -> finest, each with its mma.sync kernel
-        map; levels[d + 1] are the children of levels[d] in (z, y, x) order"""
+    def _pyramid(self, xyz: torch.Tensor) -> Tuple[List[Level], Tuple[int, int]]:
+        """the encoder's octree levels (no kernel maps) and the z extent of the leaves in the key frame (after _recentre)"""
         dev = next(self.parameters()).device
         codec = self.codec(dev)
         with torch.no_grad():
@@ -200,17 +238,61 @@ class GausPcgcNet(nn.Module):
                 meta_h = meta.cpu().numpy()
             mm = meta_h[2:8].astype(np.uint32)
             levels = codec.build_pyramid(codec.sort_unique(keys, mm), mm.astype(np.int64))
+        return levels, (int(mm[2]) - (1 << 20), int(mm[5]) - (1 << 20))
+
+    def geometry(self, xyz: torch.Tensor) -> List[Level]:
+        """the encoder's octree of a voxel cloud (GausPcgcCodec.encode): levels coarsest -> finest, each with its mma.sync kernel
+        map; levels[d + 1] are the children of levels[d] in (z, y, x) order"""
+        levels, _ = self._pyramid(xyz)
+        codec = self.codec(levels[0].keys.device)
+        with torch.no_grad():
             for lv in levels:
                 lv.kmap = codec.build_kmap(lv.keys, family="v6")
         return levels
 
-    def _stack(self, x: torch.Tensor, P: Dict[str, torch.Tensor], ids: Sequence[int], km: KMap) -> torch.Tensor:
-        cw = lambda i: P[W.CONV_KEYS[i]]
-        x = torch.relu(SparseConvFn.apply(x, cw(ids[0]), km))
+    def _packs(self, P: Dict[str, torch.Tensor]) -> Dict[str, WeightPack]:
+        return {k: WeightPack(P[k], self.wgrad_balanced_min_rows) for k in W.CONV_KEYS}
+
+    def _stack(self, x: torch.Tensor, P: Dict[str, torch.Tensor], packs: Dict[str, WeightPack], ids: Sequence[int],
+               km: KMap) -> torch.Tensor:
+        conv = lambda t, i: SparseConvFn.apply(t, P[W.CONV_KEYS[i]], km, packs[W.CONV_KEYS[i]])
+        x = torch.relu(conv(x, ids[0]))
         for a, b in ((ids[1], ids[2]), (ids[3], ids[4])):
-            t = torch.relu(SparseConvFn.apply(x, cw(a), km))
-            x = torch.relu(SparseConvFn.apply(t, cw(b), km) + x)
+            t = torch.relu(conv(x, a))
+            x = torch.relu(conv(t, b) + x)
         return x
+
+    def _level_bits(self, parent: Level, gt: Level, P: Dict[str, torch.Tensor], packs: Dict[str, WeightPack], bits: torch.Tensor,
+                    probs: Optional[List[torch.Tensor]]) -> torch.Tensor:
+        """bits + the code length of gt's four stages given its parent level (each with its mma.sync kernel map); the stages'
+        probability rows are appended to probs when it is a list"""
+        codec = self.codec(gt.keys.device)
+        dev = gt.keys.device
+        with torch.no_grad():
+            _, cp = codec.expand(parent, gt.n)                         # children == gt.keys row for row
+            cp = cp.to(torch.int64)
+            occ = gt.occ.to(torch.int64)
+        f = EmbedFn.apply(P["prior_embedding.weight"], parent.occ.to(torch.int64))
+        f = self._stack(f, P, packs, W.PRIOR_CONVS, parent.kmap)
+        u = ChildGatherFn.apply(f, cp, _octant(gt.keys)) + EmbedFn.apply(P["target_embedding.target_res_embedding.weight"], _octant(gt.keys))
+        u = self._stack(u, P, packs, W.TARGET_CONVS, gt.kmap)
+        for i in range(4):
+            f = u if i == 0 else u + EmbedFn.apply(P[f"pred_head_s{i}_emb.weight"], occ >> CTX_SHIFT[i])
+            c0, c1 = W.stage_convs(i)
+            t = torch.relu(SparseConvFn.apply(f, P[W.CONV_KEYS[c0]], gt.kmap, packs[W.CONV_KEYS[c0]]))
+            t = SparseConvFn.apply(t, P[W.CONV_KEYS[c1]], gt.kmap, packs[W.CONV_KEYS[c1]])
+            h = torch.relu(nn.functional.linear(t, P[f"pred_head_s{i}.0.weight"], P[f"pred_head_s{i}.0.bias"]))
+            logits = nn.functional.linear(h, P[f"pred_head_s{i}.2.weight"], P[f"pred_head_s{i}.2.bias"])
+            p = torch.softmax(logits, dim=1)
+            A = W.STAGE_ALPHABETS[i]
+            sym = (occ >> STAGE_SHIFT[i]) & STAGE_MASK[i]
+            hot = sym[:, None] == torch.arange(A, device=dev)[None, :]
+            # the coder's probability of the symbol: q[k] = round(cdf[k] * (65536 - A)) + k (kit/op.py) gives it
+            # (p * (65536 - A) + 1) / 65536 up to rounding, so a symbol never costs more than 16 bits
+            bits = bits - torch.log2(((p * hot).sum(1) * (65536 - A) + 1) / 65536).sum()
+            if probs is not None:
+                probs.append(p.detach())
+        return bits
 
     def forward(self, xyz: torch.Tensor, collect: bool = False) -> Dict[str, object]:
         """xyz int [N,3] voxel coordinates -> {"bits": code length of the occupancy streams, sum of -log2 of the coder's
@@ -219,38 +301,69 @@ class GausPcgcNet(nn.Module):
         in the codec's stream order (encode(..., collect=True)'s aux["probs"])."""
         levels = self.geometry(xyz)
         P = dict(self.named_parameters())
-        dev = levels[0].keys.device
-        bits = torch.zeros((), dtype=torch.float32, device=dev)
+        packs = self._packs(P)
+        bits = torch.zeros((), dtype=torch.float32, device=levels[0].keys.device)
         probs: List[torch.Tensor] = []
-        codec = self.codec(dev)
         for d in range(len(levels) - 1):
-            parent, gt = levels[d], levels[d + 1]
-            with torch.no_grad():
-                _, cp = codec.expand(parent, gt.n)                     # children == gt.keys row for row
-                cp = cp.to(torch.int64)
-                occ = gt.occ.to(torch.int64)
-            f = EmbedFn.apply(P["prior_embedding.weight"], parent.occ.to(torch.int64))
-            f = self._stack(f, P, W.PRIOR_CONVS, parent.kmap)
-            u = ChildGatherFn.apply(f, cp, _octant(gt.keys)) + EmbedFn.apply(P["target_embedding.target_res_embedding.weight"], _octant(gt.keys))
-            u = self._stack(u, P, W.TARGET_CONVS, gt.kmap)
-            for i in range(4):
-                f = u if i == 0 else u + EmbedFn.apply(P[f"pred_head_s{i}_emb.weight"], occ >> CTX_SHIFT[i])
-                c0, c1 = W.stage_convs(i)
-                t = torch.relu(SparseConvFn.apply(f, P[W.CONV_KEYS[c0]], gt.kmap))
-                t = SparseConvFn.apply(t, P[W.CONV_KEYS[c1]], gt.kmap)
-                h = torch.relu(nn.functional.linear(t, P[f"pred_head_s{i}.0.weight"], P[f"pred_head_s{i}.0.bias"]))
-                logits = nn.functional.linear(h, P[f"pred_head_s{i}.2.weight"], P[f"pred_head_s{i}.2.bias"])
-                p = torch.softmax(logits, dim=1)
-                A = W.STAGE_ALPHABETS[i]
-                sym = (occ >> STAGE_SHIFT[i]) & STAGE_MASK[i]
-                hot = sym[:, None] == torch.arange(A, device=dev)[None, :]
-                # the coder's probability of the symbol: q[k] = round(cdf[k] * (65536 - A)) + k (kit/op.py) gives it
-                # (p * (65536 - A) + 1) / 65536 up to rounding, so a symbol never costs more than 16 bits
-                bits = bits - torch.log2(((p * hot).sum(1) * (65536 - A) + 1) / 65536).sum()
-                if collect:
-                    probs.append(p.detach())
+            bits = self._level_bits(levels[d], levels[d + 1], P, packs, bits, probs if collect else None)
         n = int(xyz.shape[0])
         out = {"bits": bits, "bpp": bits / max(n, 1), "points": n, "levels": len(levels) - 1}
+        if collect:
+            out["probs"] = probs
+        return out
+
+    def forward_batch(self, patches: Sequence[torch.Tensor], collect: bool = False) -> Dict[str, object]:
+        """The code length of many voxel clouds (int [N,3] each), run as union octrees (batch.py): each patch's pyramid is built as
+        geometry() builds it, plan_unions stacks them along z with at most union_max_rows rows in a union's finest level, and every
+        union runs the network once per union level, so one launch per conv serves all its patches.  No 5^3 neighbourhood and no
+        parent spans two patches, so every patch's rows see exactly what they see alone; only the conv tilings (which depend on the
+        level's size) and the summation order of the bits differ.  A parent runs on its whole union level, a child on the level's
+        first M rows (the patches with parents at that scale).  Patches that fit no union run alone.
+        Returns {"bits": summed over the patches (fp32 scalar, differentiable), "bpp": bits / total points, "points", "patches",
+        "unions"}; collect=True adds "probs": per patch, its rows of every (level, stage) in the order forward(xyz, collect=True)
+        gives them."""
+        if not patches:
+            raise ValueError("forward_batch needs at least one patch")
+        P = dict(self.named_parameters())
+        packs = self._packs(P)
+        dev = next(self.parameters()).device
+        codec = self.codec(dev)
+        geo = [self._pyramid(xyz) for xyz in patches]
+        bits = torch.zeros((), dtype=torch.float32, device=dev)
+        probs: List[List[torch.Tensor]] = [[] for _ in patches]
+        multi = [s for s, (lv, _) in enumerate(geo) if len(lv) >= 2]
+        unions, singles = plan_unions([geo[s][1][0] for s in multi], [geo[s][1][1] for s in multi], [len(geo[s][0]) for s in multi],
+                                      [geo[s][0][-1].n for s in multi], self.union_max_rows)
+        for j in singles:
+            s = multi[j]
+            levels = geo[s][0]
+            with torch.no_grad():
+                for lv in levels:
+                    lv.kmap = codec.build_kmap(lv.keys, family="v6")
+            for d in range(len(levels) - 1):
+                bits = self._level_bits(levels[d], levels[d + 1], P, packs, bits, probs[s] if collect else None)
+        for up in unions:
+            members = [multi[j] for j in up.scenes]
+            U, K, M = union_levels([geo[s][0] for s in members], up.tz)
+            D = max(len(geo[s][0]) for s in members)
+            maps: Dict[Tuple[int, int], KMap] = {}
+
+            def level(sg: int, rows: int) -> Level:
+                ul = U[sg]
+                if (sg, rows) not in maps:
+                    with torch.no_grad():
+                        maps[sg, rows] = codec.build_kmap(ul.keys[:rows], family="v6")
+                return Level(ul.keys[:rows], ul.occ[:rows], rows, maps[sg, rows])
+
+            for sg in range(D - 1, 0, -1):                     # coarsest first, as forward() runs a patch's levels
+                got: Optional[List[torch.Tensor]] = [] if collect else None
+                bits = self._level_bits(level(sg + 1, U[sg + 1].n), level(sg, M[sg]), P, packs, bits, got)
+                if collect:
+                    for j in range(K[sg]):
+                        r0, r1 = U[sg].ranges[j]
+                        probs[members[U[sg].members[j]]] += [q[r0:r1] for q in got]
+        n = sum(int(xyz.shape[0]) for xyz in patches)
+        out = {"bits": bits, "bpp": bits / max(n, 1), "points": n, "patches": len(patches), "unions": len(unions)}
         if collect:
             out["probs"] = probs
         return out
@@ -291,14 +404,38 @@ def _load_init(init) -> Optional[Dict[str, torch.Tensor]]:
     return torch.load(init, map_location="cpu")
 
 
+def batches(n_patches: int, batch_size: int, seed: int) -> Iterator[List[int]]:
+    """The patch indices of every step: consecutive batch_size entries of one stream of permutations of range(n_patches), a new
+    permutation drawn from `seed` whenever the last one is used up (so every patch is seen once per pass, and a batch may straddle
+    two passes).  batch_size 1 gives the order single-patch training has always used."""
+    if batch_size < 1:
+        raise ValueError(f"batch_size must be >= 1, got {batch_size}")
+    if batch_size > n_patches:
+        raise ValueError(f"batch_size {batch_size} exceeds the {n_patches} patches to train on")
+
+    def stream() -> Iterator[List[int]]:
+        gen = torch.Generator().manual_seed(int(seed))
+        order: List[int] = []
+        while True:
+            batch = []
+            while len(batch) < batch_size:
+                if not order:
+                    order = torch.randperm(n_patches, generator=gen).tolist()
+                batch.append(order.pop(0))
+            yield batch
+    return stream()
+
+
 def train(clouds: Sequence[torch.Tensor], ckpt_out: Optional[str] = None, init: Union[None, str, Dict[str, torch.Tensor]] = None,
           steps: int = 1000, lr: float = 5e-4, seed: int = 0, kernel_size: int = 5, max_points: int = 150_000, save_every: int = 0,
-          synthetic_seed: int = 5, log: Optional[Callable[[Dict[str, float]], None]] = None):
+          synthetic_seed: int = 5, log: Optional[Callable[[Dict[str, float]], None]] = None, batch_size: int = 1):
     """Train on voxel clouds (int [N,3] each): the clouds are cut into kd-tree patches of at most max_points points, and every
-    step codes one patch (the order a permutation per pass, drawn from `seed`) and takes one Adam step (lr 5e-4 as the reference)
-    on its bits per point.  Starts from `init` (checkpoint path or state_dict) or make_synthetic_state_dict(synthetic_seed).
+    step codes batch_size patches (batches(): the order a permutation per pass, drawn from `seed`) and takes one Adam step (lr 5e-4
+    as the reference) on their bits per point.  batch_size 1 runs GausPcgcNet.forward on the patch; larger batches run
+    forward_batch (union octrees).  Starts from `init` (checkpoint path or state_dict) or make_synthetic_state_dict(synthetic_seed).
     Saves torch.save(state_dict) in the reference layout to ckpt_out every save_every steps (0: never) and at the end.
-    Returns (state_dict, rows) with one row {"step", "points", "bpp", "time"} per step; `log` is called with each row."""
+    Returns (state_dict, rows) with one row {"step", "points" (of the step's patches), "bpp", "time"} per step; `log` is called
+    with each row."""
     if not torch.cuda.is_available():
         raise _lib.GpcError("training needs a CUDA device (B200, sm_100a); there is no CPU fallback")
     dev = torch.device("cuda", torch.cuda.current_device())
@@ -308,22 +445,19 @@ def train(clouds: Sequence[torch.Tensor], ckpt_out: Optional[str] = None, init: 
         patches += [xyz[i].contiguous() for i in partition(xyz, max_points)]
     if not patches:
         raise ValueError("no points to train on")
+    order = batches(len(patches), batch_size, seed)
     net = GausPcgcNet(kernel_size, _load_init(init), synthetic_seed).to(dev)
     opt = torch.optim.Adam(net.parameters(), lr=lr)
-    gen = torch.Generator().manual_seed(int(seed))
-    order: List[int] = []
     rows: List[Dict[str, float]] = []
     t0 = time.time()
     for step in range(1, steps + 1):
-        if not order:
-            order = torch.randperm(len(patches), generator=gen).tolist()
-        xyz = patches[order.pop(0)]
+        batch = [patches[i] for i in next(order)]
         opt.zero_grad(set_to_none=True)
-        out = net(xyz)
+        out = net(batch[0]) if batch_size == 1 else net.forward_batch(batch)
         if out["bpp"].requires_grad:
             out["bpp"].backward()
             opt.step()
-        row = {"step": step, "points": int(xyz.shape[0]), "bpp": float(out["bpp"].detach()), "time": time.time() - t0}
+        row = {"step": step, "points": int(out["points"]), "bpp": float(out["bpp"].detach()), "time": time.time() - t0}
         rows.append(row)
         if log is not None:
             log(row)

@@ -177,6 +177,14 @@ int gpc_spconv_fwd_v6_range(const float *x, const void *Wa, const uint32_t *seg,
 size_t gpc_spconv_wgrad_workspace_bytes(int64_t n, int tile_rows);
 int gpc_spconv_wgrad_v6(const float *x, const float *dy, const uint32_t *seg, const uint64_t *pairs, int64_t n, int tile_rows,
                         float *dW, void *ws, size_t ws_bytes, void *stream);
+/* The same dW over the same stream, with the work balanced by pairs rather than by tiles: every offset's 8-entry units are cut into
+ * chunks of a compile-time number of units, one warp per chunk, and each offset's chunk partials are added in chunk order by a fixed
+ * tree.  Same arithmetic and contract as gpc_spconv_wgrad_v6 (no atomics; the summation order depends on the map, tile_rows and the
+ * chunk size only).  n_entries = the stream's entry count (KMap.n_pairs); the grid is sized from it, nothing is read back.
+ * ws: gpc_spconv_wgrad_balanced_workspace_bytes(n, tile_rows, n_entries) bytes. */
+size_t gpc_spconv_wgrad_balanced_workspace_bytes(int64_t n, int tile_rows, int64_t n_entries);
+int gpc_spconv_wgrad_v6_balanced(const float *x, const float *dy, const uint32_t *seg, const uint64_t *pairs, int64_t n, int tile_rows,
+                                 int64_t n_entries, float *dW, void *ws, size_t ws_bytes, void *stream);
 
 /* ---- the conv of the SPARSE big levels (spconv_sparse.cu): dense centre product + offset-sorted "stragglers" ----
  * For levels with ~1-4 neighbours per row (the finest octree levels).  Sparse map: seg u32[gpc_kmap_sparse_segments(n) + 1]
