@@ -61,6 +61,10 @@ SIGNATURES = {
     "gpc_spconv_wgrad_v6": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_vp, c_vp, c_sz, c_vp]),
     "gpc_spconv_wgrad_balanced_workspace_bytes": (c_sz, [c_i64, c_int, c_i64]),
     "gpc_spconv_wgrad_v6_balanced": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_i64, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_spconv_wgrad_um_workspace_bytes": (c_sz, [c_i64, c_int, c_i64]),
+    "gpc_spconv_wgrad_um": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_i64, c_vp, c_vp, c_sz, c_vp]),
+    "gpc_spconv_wgrad_sparse_workspace_bytes": (c_sz, [c_i64, c_i64]),
+    "gpc_spconv_wgrad_sparse": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_sz, c_vp]),
     "gpc_kmap_sparse_segments": (c_i64, [c_i64]),
     "gpc_kmap_sparse_workspace_bytes": (c_sz, [c_i64]),
     "gpc_kmap_sparse_count": (c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),

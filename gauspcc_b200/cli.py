@@ -5,7 +5,7 @@
     python -m gauspcc_b200.cli decompress --input_glob OUT --output_folder DEC --ckpt CKPT [--is_data_pre_quantized]
     python -m gauspcc_b200.cli train      --input_glob DIR --ckpt_out CKPT [--init CKPT] [--steps N] [--lr 5e-4] [--seed S]
                                           [--kernel_size 3|5] [--posQ 16] [--is_data_pre_quantized] [--max_points 150000]
-                                          [--batch_size 1] [--resultdir R]
+                                          [--batch_size 1] [--conv_families v6|codec] [--resultdir R]
 
 Same argument names, file discovery (recursive, sorted, h5 / ply / bin / npy; compress_ue_4stage_conv.py:57-63), coordinate
 mapping (`x / 0.001 + 131072` unless pre-quantised, then `round(x / posQ)`, :90-95; inverse `(c * posQ - 131072) * 0.001`,
@@ -21,7 +21,9 @@ to voxels there with the same float64 operations as `quantise`; decoded clouds a
 `train` (not in the reference scripts, whose trainer runs on torchsparse): reads and quantises files exactly as `compress` does, cuts
 them into kd-tree patches of at most --max_points points and trains a checkpoint on the GPU (gauspcc_b200/train.py), written in the
 reference layout to --ckpt_out; `compress` / `decompress` load it with the same --kernel_size.  `--batch_size B` (default 1) codes B
-patches per step as one union octree and takes one Adam step on their bits per point.  The CSV log (`<prefix>_train_data<N>.csv`:
+patches per step as one union octree and takes one Adam step on their bits per point.  `--conv_families codec` runs every level
+on the conv family the codec codes it with (the sparse or tcgen05 conv on levels of 150 K rows and more) instead of the mma.sync
+conv everywhere (`v6`, the default).  The CSV log (`<prefix>_train_data<N>.csv`:
 step, points of the step's patches, bpp, elapsed seconds) goes to --resultdir beside the other reports.
 
 `--batch N` (default 1): with N > 1, consecutive groups of N files are coded in one call each (pcc_utils.compress_point_clouds /
@@ -201,6 +203,9 @@ def build_parser() -> argparse.ArgumentParser:
     tp.add_argument("--save_every", type=int, default=0)
     tp.add_argument("--batch_size", type=_positive, default=1,
                     help="patches per step, run as one union octree (batch 1 is single-patch training)")
+    tp.add_argument("--conv_families", default="v6", choices=("v6", "codec"),
+                    help="conv kernels of the levels: v6 = the mma.sync conv everywhere, codec = the family the codec codes each "
+                         "level with (the sparse or tcgen05 conv on big levels)")
     tp.add_argument("--resultdir", default=None, help="folder for the CSV training log")
     tp.add_argument("--prefix", default="ue_4stage_conv")
     return ap
@@ -209,7 +214,7 @@ def build_parser() -> argparse.ArgumentParser:
 def train_files(input_glob: str, ckpt_out: str, init: Optional[str] = None, steps: int = 1000, lr: float = 5e-4, seed: int = 0,
                 kernel_size: int = 3, posQ: int = 16, is_data_pre_quantized: bool = False, max_points: int = 150_000,
                 save_every: int = 0, resultdir: Optional[str] = None, prefix: str = "ue_4stage_conv",
-                init_seed: int = 5, batch_size: int = 1) -> List[Dict[str, object]]:
+                init_seed: int = 5, batch_size: int = 1, conv_families: str = "v6") -> List[Dict[str, object]]:
     """Train a checkpoint (gauspcc_b200/train.py) on the files under input_glob, read and quantised exactly as `compress` reads them,
     so that the checkpoint learns the voxels it will code.  Writes `<prefix>_train_data<N>.csv` (one row per step) to resultdir."""
     from . import train as T
@@ -221,7 +226,7 @@ def train_files(input_glob: str, ckpt_out: str, init: Optional[str] = None, step
     d = os.path.dirname(os.path.abspath(ckpt_out))
     os.makedirs(d, exist_ok=True)
     _, rows = T.train(clouds, ckpt_out, init=init, steps=steps, lr=lr, seed=seed, kernel_size=kernel_size, max_points=max_points,
-                      save_every=save_every, synthetic_seed=init_seed, batch_size=batch_size)
+                      save_every=save_every, synthetic_seed=init_seed, batch_size=batch_size, conv_families=conv_families)
     if resultdir:
         os.makedirs(resultdir, exist_ok=True)
         with open(os.path.join(resultdir, f"{prefix}_train_data{len(paths)}.csv"), "w", newline="") as f:
@@ -236,7 +241,7 @@ def main(argv: Optional[List[str]] = None) -> int:
     t0 = time.time()
     if a.cmd == "train":
         rows = train_files(a.input_glob, a.ckpt_out, a.init, a.steps, a.lr, a.seed, a.kernel_size, a.posQ, a.is_data_pre_quantized,
-                           a.max_points, a.save_every, a.resultdir, a.prefix, a.init_seed, a.batch_size)
+                           a.max_points, a.save_every, a.resultdir, a.prefix, a.init_seed, a.batch_size, a.conv_families)
         tail = rows[-min(20, len(rows)):]
         print("Steps: {:d} | bpp first {:.3f} last {:.3f} (mean of up to 20 steps) | Max GPU memory:{:.2f}MB".format(
             len(rows), float(np.mean([r["bpp"] for r in rows[:20]])), float(np.mean([r["bpp"] for r in tail])),

@@ -1,10 +1,14 @@
 """Training of GausPcgc checkpoints on the GPU, on the codec's own geometry and conv kernels.
 
-    SparseConvFn   autograd of one 5^3 sparse conv on the mma.sync family: forward gpc_spconv_fwd_v6, input gradient the same kernel
-                   with the mirrored, transposed weights W'[k] = W[124 - k]^T (a submanifold map is symmetric: nbr_k(o) = i exactly
-                   when nbr_{124-k}(i) = o), weight gradient gpc_spconv_wgrad_v6, or gpc_spconv_wgrad_v6_balanced on levels of at
-                   least GausPcgcNet.wgrad_balanced_min_rows rows (csrc/spconv_grad.cu)
-    WeightPack     one conv weight's fragment packs, built once per forward pass and shared by every conv on every level
+    SparseConvFn   autograd of one 5^3 sparse conv on any of the codec's three conv families (the KMap's): forward the family's
+                   kernel, input gradient the same kernel with the mirrored, transposed weights W'[k] = W[124 - k]^T (a submanifold
+                   map is symmetric: nbr_k(o) = i exactly when nbr_{124-k}(i) = o), weight gradient the family's (csrc/spconv_grad.cu):
+                     mma.sync  gpc_spconv_fwd_v6, gpc_spconv_wgrad_v6 (or gpc_spconv_wgrad_v6_balanced on levels of at least
+                               GausPcgcNet.wgrad_balanced_min_rows rows)
+                     sparse    gpc_spconv_sparse_fwd, gpc_spconv_wgrad_sparse
+                     tcgen05   gpc_spconv_fwd_um on split rows (gpc_rows_split), gpc_spconv_wgrad_um
+    WeightPack     one conv weight's packs (mma.sync fragments, tcgen05 operand, and their mirrors), built once per forward pass
+                   and shared by every conv on every level
     GausPcgcNet    the model of SURVEY.md Appendix A as an nn.Module whose state_dict() is the reference layout
                    (weights.reference_layout); forward(xyz) returns the code length of the file's occupancy streams under the
                    coder's probabilities; forward_batch(patches) the same for many patches, run as union octrees (batch.py)
@@ -13,7 +17,9 @@
 
 The geometry (pyramid, children, kernel maps) comes from GausPcgcCodec exactly as the encoder builds it, so a checkpoint trained here
 is trained on the voxels, row orders and conv offsets it is later coded with: it loads with pcc_utils.compress_point_cloud unchanged.
-Every level runs the mma.sync conv family (the codec's family for levels below 150 K rows; patches are at most 150 K points).
+GausPcgcNet.conv_families picks the conv kernels: "v6" (the default) runs every level on the mma.sync family, "codec" runs every
+level on the family the codec codes it with (GausPcgcCodec.build_kmap's rule: mma.sync below 150 K rows, the sparse conv or the
+tcgen05 conv above), so a network trains on the very kernels and summation orders that will code its levels.
 
 Determinism: the same seed, inputs and initial weights give a bit-identical checkpoint.  The convs sum in an order fixed by the map,
 and the torch backward steps that would accumulate with atomics (embedding rows, the children -> parent gather) are written as
@@ -56,17 +62,68 @@ def conv_v6(x: torch.Tensor, Wa: torch.Tensor, km: KMap) -> torch.Tensor:
     return y
 
 
+def pack_um(W125: torch.Tensor) -> torch.Tensor:
+    """W [125,32,32] fp32 -> the tcgen05 conv's A operand of W^T (gpc_spconv_pack_weights_um, 512 000 bytes)"""
+    Wp = torch.empty_like(W125)
+    _lib.check(_lib.load().gpc_spconv_pack_weights_um(_ptr(W125), 1, _ptr(Wp), _stream(W125.device)), "gpc_spconv_pack_weights_um")
+    return Wp
+
+
+def conv_sparse(x: torch.Tensor, Wa: torch.Tensor, km: KMap) -> torch.Tensor:
+    """the same conv on a sparse level's map (gpc_spconv_sparse_fwd).  The stragglers' products go through km.contrib, the one
+    scratch every conv on the level shares, forward and backward alike: that is safe only because they all run in order on one
+    stream (the current one), each rewriting contrib completely before it reads it back."""
+    y = torch.empty_like(x)
+    _lib.check(_lib.load().gpc_spconv_sparse_fwd(_ptr(x), _ptr(Wa), _ptr(km.seg), _ptr(km.pairs), _ptr(km.rowptr), x.shape[0], km.n_pairs,
+                                                 _ptr(km.contrib), None, 0, _ptr(y), _stream(x.device)), "gpc_spconv_sparse_fwd")
+    return y
+
+
+def conv_um(x: torch.Tensor, Wp: torch.Tensor, km: KMap) -> torch.Tensor:
+    """the same conv on a tcgen05 level's map (gpc_spconv_fwd_um): x fp32 is split into bf16 hi / lo rows first, y is fp32"""
+    lib, st, n = _lib.load(), _stream(x.device), x.shape[0]
+    xs = torch.empty((n, 32), dtype=torch.int32, device=x.device)
+    _lib.check(lib.gpc_rows_split(_ptr(x), n, _ptr(xs), st), "gpc_rows_split")
+    y = torch.empty_like(x)
+    _lib.check(lib.gpc_spconv_fwd_um(_ptr(xs), _ptr(Wp), _ptr(km.seg), _ptr(km.pair_nbr), _ptr(km.pair_off), n, km.um_rows,
+                                     _ptr(km.tile_order), None, 0, _ptr(y), None, 0, 0, st), "gpc_spconv_fwd_um")
+    return y
+
+
+def kmap_family(km: KMap) -> str:
+    """"v6" (mma.sync), "sparse" or "um" (tcgen05): the conv family a kernel map was built for"""
+    return "um" if km.um_rows else ("sparse" if km.sparse else "v6")
+
+
 def conv_dgrad(dy: torch.Tensor, W125: torch.Tensor, km: KMap) -> torch.Tensor:
-    """dx = sum_k dy[nbr_{124-k}(i)] . W[124-k]^T: the forward conv with W'[k] = W[124 - k]^T"""
-    return conv_v6(dy, pack_frag(W125.flip(0).transpose(1, 2).contiguous()), km)
+    """dx = sum_k dy[nbr_{124-k}(i)] . W[124-k]^T: the family's forward conv with W'[k] = W[124 - k]^T"""
+    Wm = W125.flip(0).transpose(1, 2).contiguous()
+    if km.um_rows:
+        return conv_um(dy, pack_um(Wm), km)
+    if km.sparse:
+        return conv_sparse(dy, pack_frag(Wm), km)
+    return conv_v6(dy, pack_frag(Wm), km)
 
 
 def conv_wgrad(x: torch.Tensor, dy: torch.Tensor, km: KMap, balanced: bool = False) -> torch.Tensor:
-    """dW[k] = sum over the pairs (o, i) of offset k of x[i]^T dy[o]  ->  fp32 [125,32,32]; balanced: gpc_spconv_wgrad_v6_balanced
-    (the work split by pairs, for big levels) instead of gpc_spconv_wgrad_v6 (split by tiles)"""
+    """dW[k] = sum over the pairs (o, i) of offset k of x[i]^T dy[o]  ->  fp32 [125,32,32], by the map's family: gpc_spconv_wgrad_um
+    and gpc_spconv_wgrad_sparse on tcgen05 and sparse maps; on mma.sync maps gpc_spconv_wgrad_v6 (split by tiles), or with
+    balanced gpc_spconv_wgrad_v6_balanced (the work split by pairs, for big levels)"""
     lib = _lib.load()
     n = x.shape[0]
     dW = torch.empty((125, 32, 32), dtype=torch.float32, device=x.device)
+    if km.um_rows:
+        ws_b = int(lib.gpc_spconv_wgrad_um_workspace_bytes(n, km.um_rows, km.n_pairs))
+        ws = torch.empty(max(ws_b, 256), dtype=torch.uint8, device=x.device)
+        _lib.check(lib.gpc_spconv_wgrad_um(_ptr(x), _ptr(dy), _ptr(km.seg), _ptr(km.pair_nbr), _ptr(km.pair_off), n, km.um_rows,
+                                           km.n_pairs, _ptr(dW), _ptr(ws), ws_b, _stream(x.device)), "gpc_spconv_wgrad_um")
+        return dW
+    if km.sparse:
+        ws_b = int(lib.gpc_spconv_wgrad_sparse_workspace_bytes(n, km.n_pairs))
+        ws = torch.empty(max(ws_b, 256), dtype=torch.uint8, device=x.device)
+        _lib.check(lib.gpc_spconv_wgrad_sparse(_ptr(x), _ptr(dy), _ptr(km.seg), _ptr(km.pairs), _ptr(km.rowptr), n, km.n_pairs,
+                                               _ptr(dW), _ptr(ws), ws_b, _stream(x.device)), "gpc_spconv_wgrad_sparse")
+        return dW
     if balanced:
         ws_b = int(lib.gpc_spconv_wgrad_balanced_workspace_bytes(n, km.tile_rows, km.n_pairs))
         ws = torch.empty(max(ws_b, 256), dtype=torch.uint8, device=x.device)
@@ -81,14 +138,17 @@ def conv_wgrad(x: torch.Tensor, dy: torch.Tensor, km: KMap, balanced: bool = Fal
 
 
 class WeightPack:
-    """One conv weight (a [125|27,32,32] parameter) prepared for the kernels: W125, its forward fragment pack, and (built on first
-    use by a backward pass) the pack of the mirrored weights W125.flip(0).transpose(1, 2).  Built once per forward pass of the
-    network, so every conv on every level reuses the same bytes the per-call packs would have been."""
+    """One conv weight (a [125|27,32,32] parameter) prepared for the kernels: W125, its forward fragment pack (mma.sync and sparse
+    convs), and, each built on first use, the tcgen05 operand pack and the packs of the mirrored weights W125.flip(0).transpose(1, 2)
+    that the backward passes use.  Built once per forward pass of the network, so every conv on every level reuses the same bytes
+    the per-call packs would have been."""
 
     def __init__(self, Wk: torch.Tensor, wgrad_balanced_min_rows: Optional[int] = None):
         self.W125 = _to125(Wk.detach())
         self.fwd = pack_frag(self.W125)
         self._mirror: Optional[torch.Tensor] = None
+        self._um: Optional[torch.Tensor] = None
+        self._mirror_um: Optional[torch.Tensor] = None
         self.wgrad_balanced_min_rows = wgrad_balanced_min_rows     # None: every level takes gpc_spconv_wgrad_v6
 
     def mirror(self) -> torch.Tensor:
@@ -96,32 +156,49 @@ class WeightPack:
             self._mirror = pack_frag(self.W125.flip(0).transpose(1, 2).contiguous())
         return self._mirror
 
+    def um(self) -> torch.Tensor:
+        if self._um is None:
+            self._um = pack_um(self.W125)
+        return self._um
+
+    def mirror_um(self) -> torch.Tensor:
+        if self._mirror_um is None:
+            self._mirror_um = pack_um(self.W125.flip(0).transpose(1, 2).contiguous())
+        return self._mirror_um
+
+    def conv(self, x: torch.Tensor, km: KMap, mirrored: bool = False) -> torch.Tensor:
+        """x through the conv of km's family with these weights (mirrored: with W'[k] = W[124 - k]^T, the input gradient)"""
+        if km.um_rows:
+            return conv_um(x, self.mirror_um() if mirrored else self.um(), km)
+        Wa = self.mirror() if mirrored else self.fwd
+        return conv_sparse(x, Wa, km) if km.sparse else conv_v6(x, Wa, km)
+
 
 class SparseConvFn(torch.autograd.Function):
-    """y = conv(x, W) on the kernel map km (a KMap of the mma.sync family); W is [125,32,32] or [27,32,32] (kernel_size 3: the
-    27 matrices go to their K = 5 offsets, where the map holds the only present neighbours, and their gradient is gathered back).
-    pack: W's WeightPack (built from W when not given)."""
+    """y = conv(x, W) on the kernel map km (a KMap of any family: mma.sync, sparse or tcgen05, fp32 rows in and out); W is
+    [125,32,32] or [27,32,32] (kernel_size 3: the 27 matrices go to their K = 5 offsets, where the map holds the only present
+    neighbours, and their gradient is gathered back).  pack: W's WeightPack (built from W when not given)."""
 
     @staticmethod
     def forward(ctx, x: torch.Tensor, Wk: torch.Tensor, km: KMap, pack: Optional[WeightPack] = None):
-        if km.pairs is None or km.um_rows or km.sparse:
-            raise _lib.GpcError("SparseConvFn runs on the mma.sync conv's kernel map (build_kmap(..., family='v6'))")
+        if (km.pairs is None) == (km.um_rows == 0):
+            raise _lib.GpcError("SparseConvFn needs a kernel map from GausPcgcCodec.build_kmap")
         x = x.contiguous()
         pack = pack if pack is not None else WeightPack(Wk)
         ctx.km, ctx.k3, ctx.pack = km, Wk.shape[0] == 27, pack
         ctx.save_for_backward(x)
-        return conv_v6(x, pack.fwd, km)
+        return pack.conv(x, km)
 
     @staticmethod
     def backward(ctx, dy: torch.Tensor):
         (x,) = ctx.saved_tensors
         pack, km = ctx.pack, ctx.km
         dy = dy.contiguous()
-        dx = conv_v6(dy, pack.mirror(), km) if ctx.needs_input_grad[0] else None
+        dx = pack.conv(dy, km, mirrored=True) if ctx.needs_input_grad[0] else None
         dW = None
         if ctx.needs_input_grad[1]:
             lim = pack.wgrad_balanced_min_rows
-            dW = conv_wgrad(x, dy, km, balanced=lim is not None and x.shape[0] >= lim)
+            dW = conv_wgrad(x, dy, km, balanced=lim is not None and x.shape[0] >= lim)      # (balanced: mma.sync maps only)
             if ctx.k3:
                 dW = dW[torch.tensor(K5_OF_K3, device=dW.device)]
         return dx, dW, None, None
@@ -190,15 +267,28 @@ def _octant(keys: torch.Tensor) -> torch.Tensor:
 # that large, so single-patch training keeps gpc_spconv_wgrad_v6 and its bits.
 WGRAD_BALANCED_MIN_ROWS = 600_000
 
+# GausPcgcNet.conv_families: "v6" every level on the mma.sync conv; "codec" every level on the family the codec codes it with
+CONV_FAMILIES = ("v6", "codec")
+
+
+def check_conv_families(conv_families: str) -> str:
+    if conv_families not in CONV_FAMILIES:
+        raise ValueError(f"conv_families must be one of {CONV_FAMILIES}, got {conv_families!r}")
+    return conv_families
+
 
 class GausPcgcNet(nn.Module):
     """The GausPcgc network with the reference's state_dict layout (weights.reference_layout(32, kernel_size)).  Starts from
-    `state_dict` (a checkpoint in that layout) or from make_synthetic_state_dict(seed).  fog.conv.kernel is a constant buffer."""
+    `state_dict` (a checkpoint in that layout) or from make_synthetic_state_dict(seed).  fog.conv.kernel is a constant buffer.
+    conv_families: "v6" runs every level on the mma.sync conv; "codec" runs every level on the conv family the codec picks for it
+    (GausPcgcCodec.build_kmap with its own thresholds; in forward_batch the rule sees each union level as a whole)."""
 
-    def __init__(self, kernel_size: int = 5, state_dict: Optional[Dict[str, torch.Tensor]] = None, seed: int = 5):
+    def __init__(self, kernel_size: int = 5, state_dict: Optional[Dict[str, torch.Tensor]] = None, seed: int = 5,
+                 conv_families: str = "v6"):
         super().__init__()
         if kernel_size not in (3, 5):
             raise ValueError("kernel_size must be 3 or 5")
+        self.conv_families = check_conv_families(conv_families)
         self.kernel_size = kernel_size
         sd = state_dict if state_dict is not None else W.make_synthetic_state_dict(seed, 32, kernel_size)
         W.validate_state_dict(sd, 32, kernel_size)
@@ -240,14 +330,19 @@ class GausPcgcNet(nn.Module):
             levels = codec.build_pyramid(codec.sort_unique(keys, mm), mm.astype(np.int64))
         return levels, (int(mm[2]) - (1 << 20), int(mm[5]) - (1 << 20))
 
-    def geometry(self, xyz: torch.Tensor) -> List[Level]:
-        """the encoder's octree of a voxel cloud (GausPcgcCodec.encode): levels coarsest -> finest, each with its mma.sync kernel
-        map; levels[d + 1] are the children of levels[d] in (z, y, x) order"""
-        levels, _ = self._pyramid(xyz)
-        codec = self.codec(levels[0].keys.device)
+    def kmap(self, keys: torch.Tensor) -> KMap:
+        """the kernel map a level of these keys runs on: the mma.sync family ("v6"), or the codec's own choice ("codec")"""
+        family = "v6" if check_conv_families(self.conv_families) == "v6" else None
+        codec = self.codec(keys.device)
         with torch.no_grad():
-            for lv in levels:
-                lv.kmap = codec.build_kmap(lv.keys, family="v6")
+            return codec.build_kmap(keys, family=family)
+
+    def geometry(self, xyz: torch.Tensor) -> List[Level]:
+        """the encoder's octree of a voxel cloud (GausPcgcCodec.encode): levels coarsest -> finest, each with its kernel map
+        (self.kmap); levels[d + 1] are the children of levels[d] in (z, y, x) order"""
+        levels, _ = self._pyramid(xyz)
+        for lv in levels:
+            lv.kmap = self.kmap(lv.keys)
         return levels
 
     def _packs(self, P: Dict[str, torch.Tensor]) -> Dict[str, WeightPack]:
@@ -264,7 +359,7 @@ class GausPcgcNet(nn.Module):
 
     def _level_bits(self, parent: Level, gt: Level, P: Dict[str, torch.Tensor], packs: Dict[str, WeightPack], bits: torch.Tensor,
                     probs: Optional[List[torch.Tensor]]) -> torch.Tensor:
-        """bits + the code length of gt's four stages given its parent level (each with its mma.sync kernel map); the stages'
+        """bits + the code length of gt's four stages given its parent level (each with its kernel map); the stages'
         probability rows are appended to probs when it is a list"""
         codec = self.codec(gt.keys.device)
         dev = gt.keys.device
@@ -297,8 +392,9 @@ class GausPcgcNet(nn.Module):
     def forward(self, xyz: torch.Tensor, collect: bool = False) -> Dict[str, object]:
         """xyz int [N,3] voxel coordinates -> {"bits": code length of the occupancy streams, sum of -log2 of the coder's
         probability of every true symbol, (p * (65536 - A) + 1) / 65536 (fp32 scalar, differentiable),
-        "bpp": bits / N, "points": N, "levels": coded levels}; collect=True adds "probs": the softmax rows of every (level, stage)
-        in the codec's stream order (encode(..., collect=True)'s aux["probs"])."""
+        "bpp": bits / N, "points": N, "levels": coded levels, "families": {"v6" | "sparse" | "um": levels whose kernel map is of
+        that conv family}}; collect=True adds "probs": the softmax rows of every (level, stage) in the codec's stream order
+        (encode(..., collect=True)'s aux["probs"])."""
         levels = self.geometry(xyz)
         P = dict(self.named_parameters())
         packs = self._packs(P)
@@ -307,7 +403,8 @@ class GausPcgcNet(nn.Module):
         for d in range(len(levels) - 1):
             bits = self._level_bits(levels[d], levels[d + 1], P, packs, bits, probs if collect else None)
         n = int(xyz.shape[0])
-        out = {"bits": bits, "bpp": bits / max(n, 1), "points": n, "levels": len(levels) - 1}
+        out = {"bits": bits, "bpp": bits / max(n, 1), "points": n, "levels": len(levels) - 1,
+               "families": _family_counts(lv.kmap for lv in levels)}
         if collect:
             out["probs"] = probs
         return out
@@ -320,26 +417,27 @@ class GausPcgcNet(nn.Module):
         level's size) and the summation order of the bits differ.  A parent runs on its whole union level, a child on the level's
         first M rows (the patches with parents at that scale).  Patches that fit no union run alone.
         Returns {"bits": summed over the patches (fp32 scalar, differentiable), "bpp": bits / total points, "points", "patches",
-        "unions"}; collect=True adds "probs": per patch, its rows of every (level, stage) in the order forward(xyz, collect=True)
-        gives them."""
+        "unions", "families": {"v6" | "sparse" | "um": kernel maps of that conv family the step ran (one per union level and row
+        count, one per level of a patch run alone)}}; collect=True adds "probs": per patch, its rows of every (level, stage) in the
+        order forward(xyz, collect=True) gives them."""
         if not patches:
             raise ValueError("forward_batch needs at least one patch")
         P = dict(self.named_parameters())
         packs = self._packs(P)
         dev = next(self.parameters()).device
-        codec = self.codec(dev)
         geo = [self._pyramid(xyz) for xyz in patches]
         bits = torch.zeros((), dtype=torch.float32, device=dev)
         probs: List[List[torch.Tensor]] = [[] for _ in patches]
+        ran: List[KMap] = []
         multi = [s for s, (lv, _) in enumerate(geo) if len(lv) >= 2]
         unions, singles = plan_unions([geo[s][1][0] for s in multi], [geo[s][1][1] for s in multi], [len(geo[s][0]) for s in multi],
                                       [geo[s][0][-1].n for s in multi], self.union_max_rows)
         for j in singles:
             s = multi[j]
             levels = geo[s][0]
-            with torch.no_grad():
-                for lv in levels:
-                    lv.kmap = codec.build_kmap(lv.keys, family="v6")
+            for lv in levels:
+                lv.kmap = self.kmap(lv.keys)
+                ran.append(lv.kmap)
             for d in range(len(levels) - 1):
                 bits = self._level_bits(levels[d], levels[d + 1], P, packs, bits, probs[s] if collect else None)
         for up in unions:
@@ -351,8 +449,8 @@ class GausPcgcNet(nn.Module):
             def level(sg: int, rows: int) -> Level:
                 ul = U[sg]
                 if (sg, rows) not in maps:
-                    with torch.no_grad():
-                        maps[sg, rows] = codec.build_kmap(ul.keys[:rows], family="v6")
+                    maps[sg, rows] = self.kmap(ul.keys[:rows])
+                    ran.append(maps[sg, rows])
                 return Level(ul.keys[:rows], ul.occ[:rows], rows, maps[sg, rows])
 
             for sg in range(D - 1, 0, -1):                     # coarsest first, as forward() runs a patch's levels
@@ -363,7 +461,8 @@ class GausPcgcNet(nn.Module):
                         r0, r1 = U[sg].ranges[j]
                         probs[members[U[sg].members[j]]] += [q[r0:r1] for q in got]
         n = sum(int(xyz.shape[0]) for xyz in patches)
-        out = {"bits": bits, "bpp": bits / max(n, 1), "points": n, "patches": len(patches), "unions": len(unions)}
+        out = {"bits": bits, "bpp": bits / max(n, 1), "points": n, "patches": len(patches), "unions": len(unions),
+               "families": _family_counts(ran)}
         if collect:
             out["probs"] = probs
         return out
@@ -371,6 +470,13 @@ class GausPcgcNet(nn.Module):
     def checkpoint(self) -> Dict[str, torch.Tensor]:
         """state_dict in the reference layout, on the CPU (what torch.save writes and compress_point_cloud loads)"""
         return {k: v.detach().to("cpu").clone() for k, v in self.state_dict().items()}
+
+
+def _family_counts(kmaps) -> Dict[str, int]:
+    counts = {"v6": 0, "sparse": 0, "um": 0}
+    for km in kmaps:
+        counts[kmap_family(km)] += 1
+    return counts
 
 
 def partition(xyz: torch.Tensor, max_points: int = 150_000) -> List[torch.Tensor]:
@@ -428,14 +534,17 @@ def batches(n_patches: int, batch_size: int, seed: int) -> Iterator[List[int]]:
 
 def train(clouds: Sequence[torch.Tensor], ckpt_out: Optional[str] = None, init: Union[None, str, Dict[str, torch.Tensor]] = None,
           steps: int = 1000, lr: float = 5e-4, seed: int = 0, kernel_size: int = 5, max_points: int = 150_000, save_every: int = 0,
-          synthetic_seed: int = 5, log: Optional[Callable[[Dict[str, float]], None]] = None, batch_size: int = 1):
+          synthetic_seed: int = 5, log: Optional[Callable[[Dict[str, float]], None]] = None, batch_size: int = 1,
+          conv_families: str = "v6"):
     """Train on voxel clouds (int [N,3] each): the clouds are cut into kd-tree patches of at most max_points points, and every
     step codes batch_size patches (batches(): the order a permutation per pass, drawn from `seed`) and takes one Adam step (lr 5e-4
     as the reference) on their bits per point.  batch_size 1 runs GausPcgcNet.forward on the patch; larger batches run
-    forward_batch (union octrees).  Starts from `init` (checkpoint path or state_dict) or make_synthetic_state_dict(synthetic_seed).
+    forward_batch (union octrees).  conv_families: "v6" (every level on the mma.sync conv) or "codec" (every level on the conv
+    family the codec codes it with; GausPcgcNet).  Starts from `init` (checkpoint path or state_dict) or make_synthetic_state_dict(synthetic_seed).
     Saves torch.save(state_dict) in the reference layout to ckpt_out every save_every steps (0: never) and at the end.
     Returns (state_dict, rows) with one row {"step", "points" (of the step's patches), "bpp", "time"} per step; `log` is called
     with each row."""
+    check_conv_families(conv_families)
     if not torch.cuda.is_available():
         raise _lib.GpcError("training needs a CUDA device (B200, sm_100a); there is no CPU fallback")
     dev = torch.device("cuda", torch.cuda.current_device())
@@ -446,7 +555,7 @@ def train(clouds: Sequence[torch.Tensor], ckpt_out: Optional[str] = None, init: 
     if not patches:
         raise ValueError("no points to train on")
     order = batches(len(patches), batch_size, seed)
-    net = GausPcgcNet(kernel_size, _load_init(init), synthetic_seed).to(dev)
+    net = GausPcgcNet(kernel_size, _load_init(init), synthetic_seed, conv_families=conv_families).to(dev)
     opt = torch.optim.Adam(net.parameters(), lr=lr)
     rows: List[Dict[str, float]] = []
     t0 = time.time()

@@ -185,6 +185,21 @@ int gpc_spconv_wgrad_v6(const float *x, const float *dy, const uint32_t *seg, co
 size_t gpc_spconv_wgrad_balanced_workspace_bytes(int64_t n, int tile_rows, int64_t n_entries);
 int gpc_spconv_wgrad_v6_balanced(const float *x, const float *dy, const uint32_t *seg, const uint64_t *pairs, int64_t n, int tile_rows,
                                  int64_t n_entries, float *dW, void *ws, size_t ws_bytes, void *stream);
+/* The same dW, balanced the same way, over the pair stream of gpc_spconv_fwd_um (seg, pair_nbr, pair_off of gpc_kmap_um_fill with
+ * tile_rows = 512; n_entries = the stream's entry count, a multiple of 16).  An entry's output row is tile * 512 + pair_off / 128;
+ * padding entries (0xFFFFFFFF) add nothing.  ws: gpc_spconv_wgrad_um_workspace_bytes(n, tile_rows, n_entries) bytes.
+ * The input gradient is gpc_spconv_fwd_um with the gpc_spconv_pack_weights_um pack of W'[k] = W[124 - k]^T. */
+size_t gpc_spconv_wgrad_um_workspace_bytes(int64_t n, int tile_rows, int64_t n_entries);
+int gpc_spconv_wgrad_um(const float *x, const float *dy, const uint32_t *seg, const uint32_t *pair_nbr, const uint32_t *pair_off,
+                        int64_t n, int tile_rows, int64_t n_entries, float *dW, void *ws, size_t ws_bytes, void *stream);
+/* The same dW over the sparse map of gpc_spconv_sparse_fwd (seg, pairs, rowptr of gpc_kmap_sparse_fill; n_entries = its entry count,
+ * a multiple of 8).  The centre offset is x^T dy over all rows in 8-row units without a gather; the straggler segments are walked
+ * like any other stream, each entry's output row read from a slot -> row array the call builds from rowptr in the workspace.
+ * ws: gpc_spconv_wgrad_sparse_workspace_bytes(n, n_entries) bytes.  The input gradient is gpc_spconv_sparse_fwd with the
+ * gpc_spconv_pack_weights_frag pack of W'[k] = W[124 - k]^T. */
+size_t gpc_spconv_wgrad_sparse_workspace_bytes(int64_t n, int64_t n_entries);
+int gpc_spconv_wgrad_sparse(const float *x, const float *dy, const uint32_t *seg, const uint64_t *pairs, const uint32_t *rowptr,
+                            int64_t n, int64_t n_entries, float *dW, void *ws, size_t ws_bytes, void *stream);
 
 /* ---- the conv of the SPARSE big levels (spconv_sparse.cu): dense centre product + offset-sorted "stragglers" ----
  * For levels with ~1-4 neighbours per row (the finest octree levels).  Sparse map: seg u32[gpc_kmap_sparse_segments(n) + 1]
