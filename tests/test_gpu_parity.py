@@ -425,13 +425,16 @@ def test_codec_vs_oracle(env, n, seed, ext):
     _check_codec_vs_oracle(env["codec"], env["w"], n, seed, ext)
 
 
-def _check_codec_vs_oracle(codec, w, n, seed, ext, K=5):
+def _check_codec_vs_oracle(codec, w, n, seed, ext, K=5, oracle=None, prob_tol=PROB_TOL):
+    """oracle: (file, collected levels, decoded rows) of the oracle on this cloud and these weights, when already computed (they do
+    not depend on the codec's conv families).  Returns dict(aux=the encoder's collected aux, oracle=that triple, worst=the worst
+    probability gap, bytes=(file bytes, oracle file bytes))."""
     from gauspcc_b200.synth import hac_like_cloud
     from oracle import oracle as O
     xyz = hac_like_cloud(n, seed, extent_log2=ext)
     x = torch.tensor(xyz, dtype=torch.float32, device=codec.dev)
     blob, (bx, bo, streams), aux = _encode_file(codec, x)
-    ref_blob, ref = O.encode(xyz, w, K=K, collect=True)
+    ref_blob, ref, ref_dec = oracle if oracle is not None else (*O.encode(xyz, w, K=K, collect=True), None)
     # pyramid / base / stream structure bit-exact
     assert np.array_equal(bx, ref["levels"][0][0]) and np.array_equal(bo, ref["levels"][0][1])
     assert len(streams) == 4 * len(ref["aux"])
@@ -444,14 +447,17 @@ def _check_codec_vs_oracle(codec, w, n, seed, ext, K=5):
         for p in lv["probs"]:
             worst = max(worst, float(np.abs(aux["probs"][k].cpu().numpy() - p).max()))
             k += 1
-    assert worst <= PROB_TOL, worst
+    assert worst <= prob_tol, worst
     # bitstream size
     assert abs(len(blob) - len(ref_blob)) <= max(4, SIZE_TOL * len(ref_blob)), (len(blob), len(ref_blob))
     # lossless round trip, decoded rows in the reference's order (oracle decode of its own file)
     dec = codec.decode(bx, bo, streams).cpu().numpy()
     assert dec.dtype == np.float32
     assert np.array_equal(np.unique(dec.astype(np.int32), axis=0), np.unique(xyz, axis=0))
-    assert np.array_equal(dec, O.decode(ref_blob, w, K=K))
+    if ref_dec is None:
+        ref_dec = O.decode(ref_blob, w, K=K)
+    assert np.array_equal(dec, ref_dec)
+    return dict(aux=aux, oracle=(ref_blob, ref, ref_dec), worst=worst, bytes=(len(blob), len(ref_blob)))
 
 
 @pytest.mark.parametrize("n,seed,ext", [(20000, 1, 16), (2500, 5, 12)])

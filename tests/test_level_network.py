@@ -835,26 +835,30 @@ def run_chain(codec, xyz, w, K=5):
     return rec
 
 
-def _codec(gpu, kind):
-    from gauspcc_b200.codec import DeviceWeights, GausPcgcCodec
-    from gauspcc_b200.weights import make_synthetic_state_dict, state_dict_to_numpy
-    base = gpu["codec"]
-    w, K = gpu["w"], 5
-    if kind == "k3":
-        sd = make_synthetic_state_dict(kernel_size=3)
-        codec = GausPcgcCodec(DeviceWeights(sd, gpu["dev"], kernel_size=3), gpu["dev"])
-        w, K = state_dict_to_numpy(sd), 3
-    elif kind == "v6d":
-        codec = GausPcgcCodec(base.w, gpu["dev"], tile_rows=128)
+def family_codec(weights, dev, kind):
+    """a codec on these DeviceWeights whose levels all run one conv family: "v6d" (v6d<128>), "sparse", "um" (tcgen05), or
+    "default" (the codec's own thresholds)"""
+    from gauspcc_b200.codec import GausPcgcCodec
+    if kind == "v6d":
+        codec = GausPcgcCodec(weights, dev, tile_rows=128)
         codec.v6_variant = 48
         codec.um_min_rows = codec.sparse_min_rows = 1 << 40
-    else:
-        codec = GausPcgcCodec(base.w, gpu["dev"])
+        return codec
+    codec = GausPcgcCodec(weights, dev)
     if kind == "sparse":
         codec.um_min_rows, codec.sparse_min_rows, codec.sparse_max_density = 1, 1, 1e9
-    if kind in ("um", "k3"):
+    elif kind == "um":
         codec.um_min_rows, codec.sparse_max_density = 1, 0.0
-    return codec, w, K
+    return codec
+
+
+def _codec(gpu, kind):
+    from gauspcc_b200.codec import DeviceWeights
+    from gauspcc_b200.weights import make_synthetic_state_dict, state_dict_to_numpy
+    if kind == "k3":
+        sd = make_synthetic_state_dict(kernel_size=3)
+        return family_codec(DeviceWeights(sd, gpu["dev"], kernel_size=3), gpu["dev"], "um"), state_dict_to_numpy(sd), 3
+    return family_codec(gpu["codec"].w, gpu["dev"], kind), gpu["w"], 5
 
 
 @pytest.mark.gpu

@@ -269,7 +269,12 @@ def test_whole_network_gradients_against_fp64(env, k, monkeypatch):
     from gauspcc_b200.synth import hac_like_cloud
     T, dev = env["T"], env["dev"]
     net = T.GausPcgcNet(k, seed=5).to(dev)
-    xyz = torch.tensor(hac_like_cloud(5_000, seed=21, extent_log2=11), device=dev)
+    check_network_gradients(net, torch.tensor(hac_like_cloud(5_000, seed=21, extent_log2=11), device=dev), monkeypatch)
+
+
+def check_network_gradients(net, xyz, monkeypatch, tag=""):
+    """the network's bits and every parameter's gradient on the voxel cloud xyz against reference_bits in fp64"""
+    k, dev = net.kernel_size, xyz.device
     relu_inputs, relu = [], torch.relu
     monkeypatch.setattr(torch, "relu", lambda t: (relu_inputs.append(t.detach().double()), relu(t))[1])
     out = net(xyz)
@@ -288,7 +293,7 @@ def test_whole_network_gradients_against_fp64(env, k, monkeypatch):
         rel = float((p.grad.double() - g64).norm() / g64.norm())
         worst = max(worst, rel)
         assert rel <= 1e-3, (n, rel)
-    print(f"\nK={k}: {out['levels']} levels, bits {float(out['bits']):.1f}; worst per-parameter relative L2 error {worst:.2e}; "
+    print(f"\n{tag}K={k}: {out['levels']} levels, bits {float(out['bits']):.1f}; worst per-parameter relative L2 error {worst:.2e}; "
           f"{flips} of {units} ReLU units on the other side of zero in fp64 (at most {flip_mag:.1e} of their tensor's largest value)")
 
 
